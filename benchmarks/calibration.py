@@ -36,6 +36,8 @@ def parse(argv=None):
                     help="NHWC weights / activations (cuDNN's native layout on sm_100); observers and the BN moments "
                          "pass walk that memory in place")
     ap.add_argument("--cudnn-benchmark", action="store_true", help="autotuned (non-reproducible) cuDNN algorithms")
+    ap.add_argument("--observer", default="MinMaxObserver",
+                    help="weight observer by registry name, e.g. MSEObserver (clipping-range search at the weight width)")
     return ap.parse_args(argv)
 
 
@@ -67,7 +69,8 @@ def run(args) -> dict:
 
     torch.manual_seed(0)
     model = getattr(yolov8, f"yolo_v8_{args.model}")(num_classes=20).to(dev)
-    cfg = create_fuse_config_manager(FuseConfig(is_fuse_bn=False, bits_w=8, bits_a=8))  # BN kept: needed for re-estimation
+    cfg = create_fuse_config_manager(FuseConfig(is_fuse_bn=False, bits_w=8, bits_a=8,  # BN kept: needed for re-estimation
+                                                observer_w_name=args.observer))
     model = fuse_modules_unified(model, [["conv", "bn", "relu"]], config_manager=cfg)
     if args.channels_last:
         model.to(memory_format=torch.channels_last)
@@ -144,7 +147,7 @@ def run(args) -> dict:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
     t_cal, t_bn, sync_ms, t_fwd = (float(v) for v in t.tolist())
     n_img = args.batches * args.batch
-    return {"model": f"yolov8{args.model}", "n_gpus": world, "global_batches": args.batches, "batch": args.batch,
+    return {"model": f"yolov8{args.model}", "weight_observer": args.observer, "n_gpus": world, "global_batches": args.batches, "batch": args.batch,
             "imgsz": args.imgsz, "channels_last": args.channels_last, "observer_rows_synced": rows,
             "calibration_s": t_cal, "images_per_s": n_img / t_cal, "calibration_images_per_s": n_img / t_cal,
             "calibration_forward_s": t_fwd, "sync_ms": sync_ms,

@@ -195,6 +195,28 @@ int vsiq_qparams_from_minmax(double *state, int64_t n, const int32_t *bits, cons
 int vsiq_lsq_init_scale(const double *state, int64_t channels, int bits, void *scale_out, int scale_dtype,
                         vsiq_stream_t stream);
 
+/* ---- MSE observer: clipping-range search --------------------------------------------------------------------------
+ * One calibration call of observers/mse.py's MSEObserver after vsiq_observe / vsiq_ci_observe has produced this call's
+ * per-channel stats (state NULL).  For k = 1..K, alpha_k = k / K (fp64), candidate k clips the running range to
+ * (alpha_k * run_min, alpha_k * run_max) and takes (s_k, z_k) from the vsiq_qparams_from_minmax formula at `bits` /
+ * `symmetric`; its error is
+ *     E[c,k] = sum_i ((double)fq(x_i; s_k, z_k) - (double)x_i)^2      (fq: the fake-quant forward with s_k rounded to fp32,
+ *                                                                      integer range of a `bits`-bit quantiser)
+ * summed in fp64.  k* = argmin_k E[c,k], ties to the larger alpha; a channel whose range or any E is not finite takes
+ * alpha = 1.  The state is [channels][VSIQ_MSE_STATE_WIDTH]: columns 0..7 follow vsiq_observe's rule exactly (running
+ * range, call statistics), columns 8, 9 are running means m += (alpha* x run_min - m) / n_calls (and run_max), and columns
+ * 2, 3 become scale / zero-point of the mean clipped range.
+ * layout: [outer, channels, inner] as everywhere (per tensor, ch_axis 0, NCHW ch_axis 1), or a channels_last [rows, C]
+ * tensor as {rows, C, 1} (read in place, four channels per 16-byte load when C % 4 == 0 and x is 16-byte aligned).
+ * x is read once; all K candidates are scored from shared memory.  n_candidates: 1..256.
+ * err (optional): [channels][n_candidates] fp64, E of this call.  alpha (optional): [channels] fp64, the chosen alpha.
+ * Deterministic (fixed-order fp64 combination).  Two launches (search + finalize). */
+#define VSIQ_MSE_STATE_WIDTH 10 /* VSIQ_STATE_WIDTH columns, mean clipped min, mean clipped max */
+size_t vsiq_mse_search_workspace_bytes(const vsiq_layout *layout, int n_candidates);
+int vsiq_mse_search(const float *x, const vsiq_layout *layout, const double *stats, double *state, int bits,
+                    int symmetric, double eps, int n_candidates, double *err, double *alpha, void *workspace,
+                    size_t workspace_bytes, vsiq_stream_t stream);
+
 /* ---- BN re-estimation under data parallelism: the per-layer exchange as ONE kernel over NVLink peer memory -------
  * reestimate_BN_stats (utils/estimate_bn.py:56-99) with the batch sharded over ranks needs sum x / sum x^2 of every rank
  * before a layer's output can be normalised (SURVEY.md 8e).  Instead of combine kernel -> ncclAllReduce -> moments kernel,

@@ -16,6 +16,7 @@ F32, F64 = 0, 1
 MASK_ROUNDED, MASK_FUNLSQ = 0, 1
 PRE_NONE, PRE_RELU, PRE_SILU = 0, 1, 2
 STATS_WIDTH, STATE_WIDTH = 5, 8
+MSE_STATE_WIDTH = 10
 
 c_void_p, c_int, c_int64, c_float, c_double, c_size_t = (
     ctypes.c_void_p, ctypes.c_int, ctypes.c_int64, ctypes.c_float, ctypes.c_double, ctypes.c_size_t)
@@ -99,6 +100,9 @@ _SIGNATURES = {
                                 c_void_p]),
     "vsiq_ci_epilogue_observe": (c_int, [c_void_p] * 6 + [c_float, c_int, c_void_p, c_int64, c_int64, c_void_p, c_void_p,
                                          c_int, c_int, c_double, c_void_p, c_size_t, c_void_p]),
+    "vsiq_mse_search_workspace_bytes": (c_size_t, [ctypes.POINTER(Layout), c_int]),
+    "vsiq_mse_search": (c_int, [c_void_p, ctypes.POINTER(Layout), c_void_p, c_void_p, c_int, c_int, c_double, c_int, c_void_p,
+                                c_void_p, c_void_p, c_size_t, c_void_p]),
     "vsiq_peer_buffer_bytes": (c_size_t, []),
     "vsiq_peer_max_world": (c_int, []),
     "vsiq_peer_max_channels": (c_int, []),

@@ -258,6 +258,42 @@ struct OpBase {
     __device__ __forceinline__ void vec_done() {}
 };
 
+// observers/minmax.py:67-74 in IEEE doubles
+__device__ __forceinline__ void qparams_from_minmax(double mn, double mx, int bits, int symmetric, double eps,
+                                                    double* scale, double* zp) {
+    if (symmetric) {
+        const double a = fabs(mn), b = fabs(mx);
+        const double max_abs = (b > a) ? b : a;  // Python max(a, b)
+        *scale = max_abs / ((double)((1 << (bits - 1)) - 1) + eps);
+        *zp = 0.0;
+    } else {
+        const double s = (mx - mn) / ((double)((1 << bits) - 1) + eps);
+        *scale = s;
+        *zp = rint(-mn / (s + eps));
+    }
+}
+
+// The running-state rule of every min/max observer (observers/minmax.py:44-47, quantization_manager.py:66-68): one call's
+// extrema and sums (count elements per channel) folded into st[0..7], scale / zero-point from the running extrema.
+__device__ __forceinline__ void observer_state_update(double* st, float mn, float mx, double sa, double s1, double s2,
+                                                      double count, int bits, int symmetric, double eps) {
+    double run_min = st[0], run_max = st[1];
+    if ((double)mn < run_min) run_min = (double)mn;  // NaN compares false: never updates (minmax.py:44-47)
+    if ((double)mx > run_max) run_max = (double)mx;
+    double sc, zp;
+    qparams_from_minmax(run_min, run_max, bits, symmetric, eps, &sc, &zp);
+    const double mean = s1 / count;
+    const double var = (s2 - count * mean * mean) / (count - 1.0);  // torch.std: unbiased
+    st[0] = run_min;
+    st[1] = run_max;
+    st[2] = sc;
+    st[3] = zp;
+    st[4] += 1.0;
+    st[5] += sa / count;
+    st[6] += mean;
+    st[7] += sqrt(var > 0.0 ? var : 0.0);
+}
+
 // ---------------------------------------------------------------------------------------------
 // Tile schedule
 // ---------------------------------------------------------------------------------------------

@@ -91,21 +91,6 @@ __device__ __forceinline__ void stats_group_reduce(StatsOp& op, double (&out)[kP
     }
 }
 
-// observers/minmax.py:67-74 in IEEE doubles
-__device__ __forceinline__ void qparams_from_minmax(double mn, double mx, int bits, int symmetric, double eps,
-                                                    double* scale, double* zp) {
-    if (symmetric) {
-        const double a = fabs(mn), b = fabs(mx);
-        const double max_abs = (b > a) ? b : a;  // Python max(a, b)
-        *scale = max_abs / ((double)((1 << (bits - 1)) - 1) + eps);
-        *zp = 0.0;
-    } else {
-        const double s = (mx - mn) / ((double)((1 << bits) - 1) + eps);
-        *scale = s;
-        *zp = rint(-mn / (s + eps));
-    }
-}
-
 // What the combine step produces / updates for one channel.
 struct ObserveOut {
     double* stats;  // [C][VSIQ_STATS_WIDTH] or null
@@ -126,24 +111,7 @@ __device__ __forceinline__ void observe_store_channel(const ObserveOut& o, int64
         d[3] = s1;
         d[4] = s2;
     }
-    if (o.state) {
-        double* st = o.state + c * VSIQ_STATE_WIDTH;
-        double run_min = st[0], run_max = st[1];
-        if ((double)mn < run_min) run_min = (double)mn;  // NaN compares false: never updates (minmax.py:44-47)
-        if ((double)mx > run_max) run_max = (double)mx;
-        double sc, zp;
-        qparams_from_minmax(run_min, run_max, o.bits, o.symmetric, o.eps, &sc, &zp);
-        const double mean = s1 / o.count;
-        const double var = (s2 - o.count * mean * mean) / (o.count - 1.0);  // torch.std: unbiased
-        st[0] = run_min;
-        st[1] = run_max;
-        st[2] = sc;
-        st[3] = zp;
-        st[4] += 1.0;
-        st[5] += sa / o.count;
-        st[6] += mean;
-        st[7] += sqrt(var > 0.0 ? var : 0.0);
-    }
+    if (o.state) observer_state_update(o.state + c * VSIQ_STATE_WIDTH, mn, mx, sa, s1, s2, o.count, o.bits, o.symmetric, o.eps);
 }
 
 // Combine the records of channel c: STRIDE threads cooperate (32 = one warp, kThreads = the whole CTA).

@@ -565,6 +565,48 @@ def ci_epilogue_observe(x: torch.Tensor, state: torch.Tensor, bits: int = 8, sym
     return y, stats
 
 
+def new_mse_state(channels: int = 1, device=None) -> torch.Tensor:
+    """[channels, 10] fp64 MSE observer state: new_observer_state's eight columns, then the running means of the chosen
+    clipped min / max."""
+    st = torch.zeros(channels, _lib.MSE_STATE_WIDTH, dtype=torch.float64, device=device)
+    st[:, 2] = 1.0
+    return st
+
+
+def mse_search(x: torch.Tensor, ch_axis: Optional[int], state: torch.Tensor, bits: int, symmetric: bool = True,
+               eps: float = 1e-8, n_candidates: int = 100, want_err: bool = False):
+    """One calibration call of the MSE observer (vsiq_mse_search): the min/max pass for this call's statistics, then the
+    search over n_candidates clipped ranges and the state update, all on the device (no host sync).  channels_last
+    activations quantised along dim 1 are searched in place (no layout conversion).
+    Returns (stats [C, 5], err [C, K] or None, alpha [C] or None)."""
+    ci = ch_axis == 1 and ci_supported(x)
+    if not ci:
+        x = _dense_for(x, "x", ch_axis)
+    if ci:
+        N, C, H, W = x.shape
+        outer, inner = N * H * W, 1
+    else:
+        outer, C, inner = layout_of(x.shape, ch_axis)
+    lay = Layout(outer, C, inner)
+    K = int(n_candidates)
+    if state.dtype != torch.float64 or not state.is_cuda or tuple(state.shape) != (C, _lib.MSE_STATE_WIDTH) \
+            or not state.is_contiguous() or state.device != x.device:
+        raise ValueError(f"MSE observer state must be a contiguous float64 tensor [{C}, {_lib.MSE_STATE_WIDTH}] on {x.device}")
+    if not 1 <= K <= 256:
+        raise ValueError("n_candidates must be in 1..256")
+    stats = _ci_observe(x, None, bits, symmetric, eps, True) if ci else observe(x, ch_axis, None, bits, symmetric, eps)
+    with torch.cuda.device(x.device):
+        err = torch.empty(C, K, dtype=torch.float64, device=x.device) if want_err else None
+        alpha = torch.empty(C, dtype=torch.float64, device=x.device) if want_err else None
+        ws = _workspace(lib.vsiq_mse_search_workspace_bytes(ctypes.byref(lay), K), x.device)
+        check(lib.vsiq_mse_search(x.data_ptr(), ctypes.byref(lay), stats.data_ptr(), state.data_ptr(), int(bits),
+                                  int(bool(symmetric)), float(eps), K, err.data_ptr() if want_err else None,
+                                  alpha.data_ptr() if want_err else None, ws.data_ptr(), ws.numel(), _stream_ptr()),
+              "vsiq_mse_search")
+        _count_launch(2)
+    return stats, err, alpha
+
+
 def qparams_from_minmax(states: torch.Tensor, bits: torch.Tensor, symmetric: torch.Tensor, eps: float = 1e-8) -> None:
     """Recompute scale / zero-point of n observers in place from their running extrema [minmax.py:67-74]."""
     n = states.numel() // _lib.STATE_WIDTH

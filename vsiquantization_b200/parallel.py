@@ -21,6 +21,7 @@ import torch
 import torch.distributed as dist
 
 STATE_WIDTH = 8  # run_min, run_max, scale, zero_point, n_calls, sum mean|x|, sum mean x, sum std
+MSE_STATE_WIDTH = 10  # STATE_WIDTH columns, then the running means of the chosen clipped min / max (observers/mse.py)
 
 
 def _world(group=None) -> int:
@@ -55,6 +56,34 @@ def reduce_observer_states(states: torch.Tensor, group=None) -> torch.Tensor:
     return states
 
 
+def reduce_mse_states(states: torch.Tensor, group=None) -> torch.Tensor:
+    """All-reduce a packed [rows, 10] fp64 MSE observer-state block in place: columns 0..7 as reduce_observer_states, the
+    clipped means (columns 8, 9) combined as sum_r n_r * m_r / sum_r n_r with n_r the rank's call count, added in rank
+    order on every rank (all_gather, then a local sum), so every rank ends with the same bits.  Device-agnostic."""
+    if states.dtype != torch.float64 or states.dim() != 2 or states.shape[1] != MSE_STATE_WIDTH:
+        raise ValueError("states must be [rows, 10] float64")
+    w = _world(group)
+    if w == 1:
+        return states
+    mine = torch.stack([states[:, 4], states[:, 8], states[:, 9]], dim=1).contiguous()
+    everyone = [torch.empty_like(mine) for _ in range(w)]
+    dist.all_gather(everyone, mine, group=group)
+    n = torch.zeros_like(mine[:, 0])
+    lo = torch.zeros_like(n)
+    hi = torch.zeros_like(n)
+    for r in range(w):  # rank order
+        n = n + everyone[r][:, 0]
+        lo = lo + everyone[r][:, 0] * everyone[r][:, 1]
+        hi = hi + everyone[r][:, 0] * everyone[r][:, 2]
+    has = n > 0
+    base = states[:, :STATE_WIDTH].contiguous()
+    reduce_observer_states(base, group)
+    states[:, :STATE_WIDTH] = base
+    states[:, 8] = torch.where(has, lo / torch.where(has, n, torch.ones_like(n)), states[:, 8])
+    states[:, 9] = torch.where(has, hi / torch.where(has, n, torch.ones_like(n)), states[:, 9])
+    return states
+
+
 def sync_observers(model, group=None) -> int:
     """Make every rank's observers agree after sharded calibration; returns the number of observer rows synchronised.
     Scales / zero-points are recomputed from the reduced extrema exactly as observers/minmax.py:67-74 would."""
@@ -63,8 +92,30 @@ def sync_observers(model, group=None) -> int:
     # moving-average observers (observers/moving_average.py) hold averages, not extrema: their running min / max are
     # AVERAGED over the ranks and their qparams recomputed with torch's formula; the call statistics are summed
     ema = [(m, o) for m, o in every if hasattr(o, "averaging_constant")]
-    entries = [(m, o) for m, o in every if not hasattr(o, "averaging_constant")]
-    rows_ema = 0
+    # MSE observers (observers/mse.py): range and statistics like min/max observers, clipped means weighted by call counts;
+    # scale / zero-point then come from the combined means
+    mse = [(m, o) for m, o in every if o.state.shape[1] == MSE_STATE_WIDTH]
+    entries = [(m, o) for m, o in every if not hasattr(o, "averaging_constant") and o.state.shape[1] == STATE_WIDTH]
+    rows_mse = 0
+    if mse:
+        arena = torch.cat([o.state for _, o in mse]).contiguous()
+        reduce_mse_states(arena, group)
+        means = arena[:, :STATE_WIDTH].clone()
+        means[:, 0:2] = arena[:, 8:10]
+        bits = torch.cat([torch.full((o.state.shape[0],), int(o.num_bits), dtype=torch.int32) for _, o in mse])
+        sym = torch.cat([torch.full((o.state.shape[0],), int(bool(o.symmetric)), dtype=torch.int32) for _, o in mse])
+        eps = {float(o.eps) for _, o in mse}
+        if len(eps) != 1:
+            raise ValueError("observers with different eps cannot be recomputed in one launch")
+        ops.qparams_from_minmax(means, bits, sym, eps.pop())
+        arena[:, 2:4] = means[:, 2:4]
+        for m, o in mse:
+            k = o.state.shape[0]
+            o.state.copy_(arena[rows_mse:rows_mse + k])
+            o._host = None
+            m._invalidate()
+            rows_mse += k
+    rows_ema = rows_mse
     if ema:
         from .observers.moving_average import torch_qparams
         arena = torch.cat([o.state for _, o in ema]).contiguous()
@@ -88,7 +139,7 @@ def sync_observers(model, group=None) -> int:
             o._host = None
             m._invalidate()
             row += k
-        rows_ema = row
+        rows_ema += row
     if not entries:
         return rows_ema
     arena = torch.cat([o.state for _, o in entries]).contiguous()

@@ -34,6 +34,7 @@ import torch.nn as nn
 
 from ..observers.minmax import MinMaxObserver  # noqa: F401  (registers the plugin classes)
 from ..observers.moving_average import MovingAverageMinMaxObserver  # noqa: F401
+from ..observers.mse import MSEObserver  # noqa: F401
 from ..quantizers.uniform import UniformQuantizer  # noqa: F401
 from ..utils.registry import CLASS_REGISTRY
 
@@ -46,6 +47,8 @@ class QuantizationManager(nn.Module):
                  param_dtype: torch.dtype = torch.float64) -> None:
         super().__init__()
         self.quantizer = CLASS_REGISTRY[quantizer_name](bits_width, is_symmetric)
+        if observer_bits is None and getattr(CLASS_REGISTRY[observer_name], "needs_quantizer_bits", False):
+            observer_bits = bits_width  # an observer whose result depends on the quantiser's width (MSEObserver)
         if observer_bits is None:
             self.observer = CLASS_REGISTRY[observer_name](is_symmetric)  # num_bits stays 8, like the reference
         else:
@@ -113,6 +116,8 @@ class QuantizationManager(nn.Module):
     #    observer state (C x 8) ..., scale ..., zero_point ..., calib_grad_scale ...]
     # kind: 0 absent (a learned Parameter: an ordinary state_dict entry), 1 Python int, 2 Python float, 3 0-dim tensor,
     # 4 1-D tensor; +10 when the tensor was float32 (else float64).
+    # Version 3 (observers whose state is not [C, 8], e.g. MSEObserver's [C, 10]) appends the state width W to the header
+    # and the observer state is C x W; [C, 8] states are still written as version 2, byte for byte.
     _MAGIC, _HEADER = 20477.0, 13
 
     @staticmethod
@@ -147,10 +152,13 @@ class QuantizationManager(nn.Module):
         C = st.shape[0] if st is not None else 0
         parts = [self._pack_value(self.__dict__.get("scale")), self._pack_value(self.__dict__.get("zero_point")),
                  self._pack_value(getattr(self.quantizer, "calib_grad_scale", 1))]
-        head = [self._MAGIC, 2.0, float(bool(self.is_observer_qparam)), float(bool(self.is_learning_scale)),
-                float(bool(self.is_quantize)), float(bool(self._calibrated)), float(C)]
+        W = st.shape[1] if st is not None else 8
+        head = [self._MAGIC, 2.0 if W == 8 else 3.0, float(bool(self.is_observer_qparam)),
+                float(bool(self.is_learning_scale)), float(bool(self.is_quantize)), float(bool(self._calibrated)), float(C)]
         for kind, vals in parts:
             head += [float(kind), float(len(vals))]
+        if W != 8:
+            head.append(float(W))
         body = st.reshape(-1).tolist() if st is not None else []
         for _, vals in parts:
             body += vals
@@ -163,8 +171,14 @@ class QuantizationManager(nn.Module):
         C = int(v[6])
         kinds = [(int(v[7 + 2 * i]), int(v[8 + 2 * i])) for i in range(3)]
         off = self._HEADER
-        st = torch.tensor(v[off:off + 8 * C], dtype=torch.float64).reshape(C, 8) if C else None
-        off += 8 * C
+        W = 8
+        if v[1] == 3.0:
+            W = int(v[off])
+            off += 1
+        elif v[1] != 2.0:
+            raise ValueError(f"unsupported QuantizationManager extra state version {v[1]}")
+        st = torch.tensor(v[off:off + W * C], dtype=torch.float64).reshape(C, W) if C else None
+        off += W * C
         vals = []
         for kind, n in kinds:
             vals.append(self._unpack_value(kind, v[off:off + n]))
