@@ -38,6 +38,9 @@ def parse(argv=None):
     ap.add_argument("--cudnn-benchmark", action="store_true", help="autotuned (non-reproducible) cuDNN algorithms")
     ap.add_argument("--observer", default="MinMaxObserver",
                     help="weight observer by registry name, e.g. MSEObserver (clipping-range search at the weight width)")
+    ap.add_argument("--act-observer", default="MinMaxObserver",
+                    help="activation observer by registry name, e.g. PercentileObserver (histogram clip at the activation "
+                         "width); its histograms are merged exactly by the observer sync, so the digests still agree")
     return ap.parse_args(argv)
 
 
@@ -70,7 +73,7 @@ def run(args) -> dict:
     torch.manual_seed(0)
     model = getattr(yolov8, f"yolo_v8_{args.model}")(num_classes=20).to(dev)
     cfg = create_fuse_config_manager(FuseConfig(is_fuse_bn=False, bits_w=8, bits_a=8,  # BN kept: needed for re-estimation
-                                                observer_w_name=args.observer))
+                                                observer_w_name=args.observer, observer_a_name=args.act_observer))
     model = fuse_modules_unified(model, [["conv", "bn", "relu"]], config_manager=cfg)
     if args.channels_last:
         model.to(memory_format=torch.channels_last)
@@ -147,7 +150,9 @@ def run(args) -> dict:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
     t_cal, t_bn, sync_ms, t_fwd = (float(v) for v in t.tolist())
     n_img = args.batches * args.batch
-    return {"model": f"yolov8{args.model}", "weight_observer": args.observer, "n_gpus": world, "global_batches": args.batches, "batch": args.batch,
+    return {"model": f"yolov8{args.model}", "weight_observer": args.observer, **(
+                {"activation_observer": args.act_observer} if args.act_observer != "MinMaxObserver" else {}),
+            "n_gpus": world, "global_batches": args.batches, "batch": args.batch,
             "imgsz": args.imgsz, "channels_last": args.channels_last, "observer_rows_synced": rows,
             "calibration_s": t_cal, "images_per_s": n_img / t_cal, "calibration_images_per_s": n_img / t_cal,
             "calibration_forward_s": t_fwd, "sync_ms": sync_ms,

@@ -217,6 +217,34 @@ int vsiq_mse_search(const float *x, const vsiq_layout *layout, const double *sta
                     int symmetric, double eps, int n_candidates, double *err, double *alpha, void *workspace,
                     size_t workspace_bytes, vsiq_stream_t stream);
 
+/* ---- percentile observer: exact-bin histograms and the clip at a percentile ---------------------------------------
+ * One calibration call of observers/percentile.py's PercentileObserver after vsiq_observe / vsiq_ci_observe has produced
+ * this call's per-channel stats (state NULL).  B = n_bins bins per side, a power of two in 256..4096.  The state is
+ * [channels][VSIQ_HIST_STATE_HEAD + 2 * B] fp64:
+ *   0..7   vsiq_observe's running range and call statistics, exactly its rule (columns 2, 3 are then overwritten below)
+ *   8, 9   the clipped lo / hi
+ *   10, 11 bin exponents e_neg, e_pos: the bin width of a side is 2^e, e the smallest integer >= -149 with
+ *          m < B * 2^e for the side's extent m (-run_min, run_max)
+ *   12 ..  B counts of x < 0 (bin i: |x| in [i 2^e_neg, (i+1) 2^e_neg)), then B counts of x >= 0, -0.0 included
+ * A fresh state is zero except scale = 1 and e_neg = e_pos = -149.  A call first takes the new running range, coarsens
+ * the stored counts of a side whose exponent grows (old bin i -> new bin i >> delta, exact), then adds its values.  A
+ * channel whose call extrema are NaN keeps its counts; once its running range is not finite the counts are frozen and the
+ * clip is the running range.  The clip, from all counts so far: N = total count, T = floor((1 - percentile / 100) * N)
+ * (fp64, each operation rounded), hi = min(run_max, (j + 1) 2^e_pos) with j the smallest index whose counts above it sum
+ * to <= T, lo = max(run_min, -(j' + 1) 2^e_neg) likewise; columns 2, 3 = scale / zero-point of (lo, hi) with the
+ * vsiq_qparams_from_minmax formula.  percentile = 100 gives the min/max result bit for bit.  The counts depend only on the
+ * multiset of values observed (integer counts, power-of-two bins), not on call order or on how calls were split.
+ * layout: as vsiq_mse_search (channels_last [rows, C] read in place as {rows, C, 1}).  x is read once.  Workspace: the
+ * 256-byte header (left untouched) and a count area the call zero-fills itself.  Two launches (histogram + finalize).
+ * vsiq_hist_clip recomputes columns 2, 3, 8, 9 from the stored counts at another percentile, with no new data. */
+#define VSIQ_HIST_STATE_HEAD 12
+size_t vsiq_hist_observe_workspace_bytes(const vsiq_layout *layout, int n_bins); /* 0 for an invalid layout / n_bins */
+int vsiq_hist_observe(const float *x, const vsiq_layout *layout, const double *stats, double *state, int n_bins,
+                      double percentile, int bits, int symmetric, double eps, void *workspace, size_t workspace_bytes,
+                      vsiq_stream_t stream);
+int vsiq_hist_clip(double *state, int64_t channels, int n_bins, double percentile, int bits, int symmetric, double eps,
+                   vsiq_stream_t stream);
+
 /* ---- BN re-estimation under data parallelism: the per-layer exchange as ONE kernel over NVLink peer memory -------
  * reestimate_BN_stats (utils/estimate_bn.py:56-99) with the batch sharded over ranks needs sum x / sum x^2 of every rank
  * before a layer's output can be normalised (SURVEY.md 8e).  Instead of combine kernel -> ncclAllReduce -> moments kernel,

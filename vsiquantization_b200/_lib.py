@@ -17,6 +17,7 @@ MASK_ROUNDED, MASK_FUNLSQ = 0, 1
 PRE_NONE, PRE_RELU, PRE_SILU = 0, 1, 2
 STATS_WIDTH, STATE_WIDTH = 5, 8
 MSE_STATE_WIDTH = 10
+HIST_STATE_HEAD = 12  # percentile observer state: [C, HIST_STATE_HEAD + 2 * n_bins]
 
 c_void_p, c_int, c_int64, c_float, c_double, c_size_t = (
     ctypes.c_void_p, ctypes.c_int, ctypes.c_int64, ctypes.c_float, ctypes.c_double, ctypes.c_size_t)
@@ -103,6 +104,10 @@ _SIGNATURES = {
     "vsiq_mse_search_workspace_bytes": (c_size_t, [ctypes.POINTER(Layout), c_int]),
     "vsiq_mse_search": (c_int, [c_void_p, ctypes.POINTER(Layout), c_void_p, c_void_p, c_int, c_int, c_double, c_int, c_void_p,
                                 c_void_p, c_void_p, c_size_t, c_void_p]),
+    "vsiq_hist_observe_workspace_bytes": (c_size_t, [ctypes.POINTER(Layout), c_int]),
+    "vsiq_hist_observe": (c_int, [c_void_p, ctypes.POINTER(Layout), c_void_p, c_void_p, c_int, c_double, c_int, c_int,
+                                  c_double, c_void_p, c_size_t, c_void_p]),
+    "vsiq_hist_clip": (c_int, [c_void_p, c_int64, c_int, c_double, c_int, c_int, c_double, c_void_p]),
     "vsiq_peer_buffer_bytes": (c_size_t, []),
     "vsiq_peer_max_world": (c_int, []),
     "vsiq_peer_max_channels": (c_int, []),

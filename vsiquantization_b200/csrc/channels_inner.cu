@@ -19,8 +19,6 @@
 // Roofline: HBM; 8 B/element forward, 12 B/element backward, as for the NCHW kernels.
 #include <stdlib.h>
 
-#include <mutex>
-
 #include "ci_common.cuh"
 
 namespace vsiq {
@@ -774,19 +772,6 @@ __global__ void __launch_bounds__(kThreads + 32, 2)
                                            ws, o, use_ticket, t, active);
 }
 
-// opt in to > 48 KB of dynamic shared memory once per kernel instantiation and device (thread-safe)
-template <auto Kernel>  // a non-type parameter: every instantiation of the kernel gets its own flags
-static cudaError_t ci_set_smem_once(int device, int bytes) {
-    static std::mutex mu;
-    static bool done[64];
-    std::lock_guard<std::mutex> lk(mu);
-    if (device < 0 || device >= 64) return cudaErrorInvalidDevice;
-    if (done[device]) return cudaSuccess;
-    cudaError_t e = cudaFuncSetAttribute(Kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes);
-    if (e == cudaSuccess) done[device] = true;
-    return e;
-}
-
 }  // namespace vsiq
 
 using namespace vsiq;
@@ -934,7 +919,7 @@ extern "C" int vsiq_ci_lsq_bwd(const float* x, const float* bias, const float* g
 #define B(P, H, R, D)                                                                                                      \
     {                                                                                                                      \
         if (use_tma) {                                                                                                     \
-            if (cudaError_t ae = ci_set_smem_once<ci_bwd_tma_kernel<P, H, R, D>>(cur_dev, 3 * 2 * 16384)) return (int)ae;   \
+            if (cudaError_t ae = set_smem_once<ci_bwd_tma_kernel<P, H, R, D>>(cur_dev, 3 * 2 * 16384)) return (int)ae;   \
             ci_bwd_tma_kernel<P, H, R, D><<<grid, kThreads + 32, dyn_smem, st>>>(x, bias, g, dx, geo, qpd, workspace, o,    \
                                                                                 use_ticket, g_row_pitch);                 \
         } else {                                                                                                           \

@@ -17,6 +17,8 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
+#include <mutex>
+
 #include "../../include/vsiq.h"
 
 namespace vsiq {
@@ -631,6 +633,19 @@ int ci_tile_override();     // VSIQ_CI_TILE=<steps per tile>, else 0 (automatic)
 int pc_chunk_override();    // VSIQ_PC_CHUNK=<elements per unit of the NCHW per-channel schedule>, else 0 (automatic)
 int check_layout(const vsiq_layout* l);
 int fill_qp(const vsiq_qparams* in, QPDev* out);
+
+// opt in to > 48 KB of dynamic shared memory once per kernel instantiation and device (thread-safe)
+template <auto Kernel>  // a non-type parameter: every instantiation of the kernel gets its own flags
+static cudaError_t set_smem_once(int device, int bytes) {
+    static std::mutex mu;
+    static bool done[64];
+    std::lock_guard<std::mutex> lk(mu);
+    if (device < 0 || device >= 64) return cudaErrorInvalidDevice;
+    if (done[device]) return cudaSuccess;
+    cudaError_t e = cudaFuncSetAttribute(Kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes);
+    if (e == cudaSuccess) done[device] = true;
+    return e;
+}
 
 // ---------------------------------------------------------------------------------------------
 // Programmatic dependent launch (PDL)

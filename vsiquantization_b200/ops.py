@@ -607,6 +607,71 @@ def mse_search(x: torch.Tensor, ch_axis: Optional[int], state: torch.Tensor, bit
     return stats, err, alpha
 
 
+def _check_hist_args(n_bins: int, percentile: float) -> None:
+    n_bins = int(n_bins)
+    if not (256 <= n_bins <= 4096 and n_bins & (n_bins - 1) == 0):
+        raise ValueError("n_bins must be a power of two in 256..4096")
+    if not 0.0 < float(percentile) <= 100.0:
+        raise ValueError("percentile must be in (0, 100]")
+
+
+def new_percentile_state(channels: int, n_bins: int = 2048, device=None) -> torch.Tensor:
+    """[channels, 12 + 2 * n_bins] fp64 percentile observer state: new_observer_state's eight columns, the clipped lo / hi,
+    the bin exponents e_neg / e_pos (-149: the finest width, 2^-149), then n_bins counts of x < 0 and n_bins of x >= 0."""
+    _check_hist_args(n_bins, 100.0)
+    st = torch.zeros(channels, _lib.HIST_STATE_HEAD + 2 * int(n_bins), dtype=torch.float64, device=device)
+    st[:, 2] = 1.0
+    st[:, 10:12] = -149.0
+    return st
+
+
+def _check_hist_state(state: torch.Tensor, C: int, n_bins: int, device) -> None:
+    W = _lib.HIST_STATE_HEAD + 2 * int(n_bins)
+    if state.dtype != torch.float64 or not state.is_cuda or tuple(state.shape) != (C, W) or not state.is_contiguous() \
+            or state.device != device:
+        raise ValueError(f"percentile observer state must be a contiguous float64 tensor [{C}, {W}] on {device}")
+
+
+def hist_observe(x: torch.Tensor, ch_axis: Optional[int], state: torch.Tensor, n_bins: int = 2048,
+                 percentile: float = 99.99, bits: int = 8, symmetric: bool = True, eps: float = 1e-8) -> torch.Tensor:
+    """One calibration call of the percentile observer (vsiq_hist_observe): the min/max pass for this call's statistics,
+    then one histogram pass over x and the state update with the clip at `percentile`, all on the device (no host sync).
+    channels_last activations quantised along dim 1 are read in place (no layout conversion).  Returns stats [C, 5]."""
+    _check_hist_args(n_bins, percentile)
+    ci = ch_axis == 1 and ci_supported(x)
+    if not ci:
+        x = _dense_for(x, "x", ch_axis)
+    if ci:
+        N, C, H, W = x.shape
+        outer, inner = N * H * W, 1
+    else:
+        outer, C, inner = layout_of(x.shape, ch_axis)
+    lay = Layout(outer, C, inner)
+    _check_hist_state(state, C, n_bins, x.device)
+    stats = _ci_observe(x, None, bits, symmetric, eps, True) if ci else observe(x, ch_axis, None, bits, symmetric, eps)
+    with torch.cuda.device(x.device):
+        ws = _workspace(lib.vsiq_hist_observe_workspace_bytes(ctypes.byref(lay), int(n_bins)), x.device)
+        check(lib.vsiq_hist_observe(x.data_ptr(), ctypes.byref(lay), stats.data_ptr(), state.data_ptr(), int(n_bins),
+                                    float(percentile), int(bits), int(bool(symmetric)), float(eps), ws.data_ptr(),
+                                    ws.numel(), _stream_ptr()), "vsiq_hist_observe")
+        _count_launch(2)
+    return stats
+
+
+def hist_clip(state: torch.Tensor, n_bins: int, percentile: float, bits: int, symmetric: bool = True,
+              eps: float = 1e-8) -> None:
+    """Recompute the clip (columns 8, 9) and scale / zero-point (2, 3) of a percentile observer state in place from its
+    stored counts at `percentile` (vsiq_hist_clip): no new data, no host sync."""
+    _check_hist_args(n_bins, percentile)
+    if state.dim() != 2:
+        raise ValueError("percentile observer state must be [channels, 12 + 2 * n_bins]")
+    _check_hist_state(state, state.shape[0], n_bins, state.device)
+    with torch.cuda.device(state.device):
+        check(lib.vsiq_hist_clip(state.data_ptr(), state.shape[0], int(n_bins), float(percentile), int(bits),
+                                 int(bool(symmetric)), float(eps), _stream_ptr()), "vsiq_hist_clip")
+        _count_launch()
+
+
 def qparams_from_minmax(states: torch.Tensor, bits: torch.Tensor, symmetric: torch.Tensor, eps: float = 1e-8) -> None:
     """Recompute scale / zero-point of n observers in place from their running extrema [minmax.py:67-74]."""
     n = states.numel() // _lib.STATE_WIDTH

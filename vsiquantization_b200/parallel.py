@@ -22,6 +22,7 @@ import torch.distributed as dist
 
 STATE_WIDTH = 8  # run_min, run_max, scale, zero_point, n_calls, sum mean|x|, sum mean x, sum std
 MSE_STATE_WIDTH = 10  # STATE_WIDTH columns, then the running means of the chosen clipped min / max (observers/mse.py)
+HIST_STATE_HEAD = 12  # percentile observers (observers/percentile.py): [C, HIST_STATE_HEAD + 2 * n_bins]
 
 
 def _world(group=None) -> int:
@@ -84,6 +85,49 @@ def reduce_mse_states(states: torch.Tensor, group=None) -> torch.Tensor:
     return states
 
 
+def _hist_exponent(m: torch.Tensor, log2b: int) -> torch.Tensor:
+    """The smallest e >= -149 with m < 2^log2b * 2^e, per entry of a finite float64 m >= 0 (csrc/hist_observer.cu)."""
+    _, k = torch.frexp(torch.where(m > 0, m, torch.ones_like(m)))  # m = f * 2^k, f in [0.5, 1)
+    e = k.to(torch.int64) - log2b
+    return torch.where(m > 0, torch.clamp(e, min=-149), torch.full_like(e, -149))
+
+
+def reduce_percentile_states(states: torch.Tensor, n_bins: int, group=None) -> torch.Tensor:
+    """All-reduce a packed [rows, 12 + 2 * n_bins] fp64 percentile-observer block in place: columns 0..7 as
+    reduce_observer_states; per side the bin exponent of the reduced range (and at least every rank's own); each rank's
+    counts coarsened to it (old bin i -> new bin i >> delta, exact); the counts summed (exact on integer-valued fp64), so
+    every rank ends with the same bits -- the histogram a single process would hold after seeing every rank's calls.
+    Columns 2, 3, 8, 9 (the clip) are left to be recomputed (ops.hist_clip).  Device-agnostic."""
+    B = int(n_bins)
+    if B < 256 or B > 4096 or B & (B - 1):
+        raise ValueError("n_bins must be a power of two in 256..4096")
+    W = HIST_STATE_HEAD + 2 * B
+    if states.dtype != torch.float64 or states.dim() != 2 or states.shape[1] != W:
+        raise ValueError(f"states must be [rows, {W}] float64")
+    if _world(group) == 1:
+        return states
+    base = states[:, :STATE_WIDTH].contiguous()
+    reduce_observer_states(base, group)
+    states[:, :STATE_WIDTH] = base
+    lo, hi = states[:, 0], states[:, 1]
+    e_own = states[:, 10:12].to(torch.int64)
+    e = states[:, 10:12].contiguous()
+    dist.all_reduce(e, op=dist.ReduceOp.MAX, group=group)
+    e = e.to(torch.int64)
+    finite = (torch.isfinite(lo) & torch.isfinite(hi)).unsqueeze(1)
+    log2b = B.bit_length() - 1
+    e_range = torch.stack([_hist_exponent(-lo, log2b), _hist_exponent(hi, log2b)], dim=1)
+    e = torch.where(finite, torch.maximum(e, e_range), e)
+    counts = states[:, HIST_STATE_HEAD:].reshape(-1, 2, B)
+    shift = torch.clamp(e - e_own, 0, 62).unsqueeze(2)
+    idx = torch.bitwise_right_shift(torch.arange(B, device=states.device).expand_as(counts), shift)
+    merged = torch.zeros_like(counts).scatter_add_(2, idx, counts)
+    dist.all_reduce(merged, op=dist.ReduceOp.SUM, group=group)
+    states[:, HIST_STATE_HEAD:] = merged.reshape(-1, 2 * B)
+    states[:, 10:12] = e.to(torch.float64)
+    return states
+
+
 def sync_observers(model, group=None) -> int:
     """Make every rank's observers agree after sharded calibration; returns the number of observer rows synchronised.
     Scales / zero-points are recomputed from the reduced extrema exactly as observers/minmax.py:67-74 would."""
@@ -115,6 +159,20 @@ def sync_observers(model, group=None) -> int:
             o._host = None
             m._invalidate()
             rows_mse += k
+    # percentile observers (observers/percentile.py), found by class attribute: range and statistics like min/max
+    # observers, histograms merged exactly; each clip is then recomputed on the device at that observer's percentile
+    pct = [(m, o) for m, o in every if getattr(o, "keeps_histogram", False)]
+    for n_bins in sorted({o.n_bins for _, o in pct}):
+        same = [(m, o) for m, o in pct if o.n_bins == n_bins]
+        arena = torch.cat([o.state for _, o in same]).contiguous()
+        reduce_percentile_states(arena, n_bins, group)
+        row = 0
+        for m, o in same:
+            k = o.state.shape[0]
+            o.state.copy_(arena[row:row + k])
+            o.recompute_clip()  # also drops the manager's cached qparams (_on_change)
+            row += k
+        rows_mse += row
     rows_ema = rows_mse
     if ema:
         from .observers.moving_average import torch_qparams
