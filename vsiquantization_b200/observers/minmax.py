@@ -12,7 +12,8 @@ from typing import Optional
 
 import torch
 
-from .. import ops
+from .. import ops, parallel
+from .._lib import STATE_WIDTH
 from ..utils.registry import register_class
 from .base import BaseObserver
 
@@ -23,6 +24,16 @@ def _as_cuda(x: torch.Tensor) -> torch.Tensor:
     if not torch.cuda.is_available():
         raise RuntimeError("vsiquantization_b200 needs a CUDA device: there is no CPU fallback")
     return x.cuda()
+
+
+def qparam_args(observers) -> tuple:
+    """(bits, symmetric, eps) for one ops.qparams_from_minmax launch over the concatenated states of ``observers``."""
+    bits = torch.cat([torch.full((o.state.shape[0],), int(o.num_bits), dtype=torch.int32) for o in observers])
+    sym = torch.cat([torch.full((o.state.shape[0],), int(bool(o.symmetric)), dtype=torch.int32) for o in observers])
+    eps = {float(o.eps) for o in observers}
+    if len(eps) != 1:
+        raise ValueError("observers with different eps cannot be recomputed in one launch")
+    return bits, sym, eps.pop()
 
 
 @register_class
@@ -36,30 +47,33 @@ class MinMaxObserver(BaseObserver):
         self.eps = eps
         self.num_bits = num_bits
         self.ch_axis = ch_axis
-        self._state: Optional[torch.Tensor] = None  # [C, 8] fp64 on the device, see ops.new_observer_state
+        self._state: Optional[torch.Tensor] = None  # [C, W] fp64 on the device, see _new_state
         self._host = None                            # cached host copy of the state
         self.last_stats: Optional[torch.Tensor] = None
         self.last_count = 0
         self._on_change = None                       # set by the owning QuantizationManager (cache invalidation)
 
     # -- device state -----------------------------------------------------------------------------
-    def bind_state(self, state: torch.Tensor) -> None:
-        """Use a row block of a shared arena as this observer's state (parallel.ObserverArena)."""
-        if self._state is not None:
-            state.copy_(self._state)
-        self._state = state
-        self._host = None
+    def _new_state(self, channels: int, device) -> torch.Tensor:
+        """A fresh [channels, W] state in this observer's layout."""
+        return ops.new_observer_state(channels, device)
+
+    def _adapt_state(self, state: torch.Tensor) -> torch.Tensor:
+        """A loaded fp64 state in this observer's layout, or ValueError when it cannot be one."""
+        if state.dim() != 2 or state.shape[1] != STATE_WIDTH:
+            raise ValueError("observer state must be [channels, 8]")
+        return state
 
     def load_state(self, state: torch.Tensor) -> None:
-        """Restore a saved [C, 8] fp64 state (checkpoints; QuantizationManager.set_extra_state).  It goes to the GPU
-        when there is one; without one it stays on the host and the first kernel call fails loudly."""
-        if state.dim() != 2 or state.shape[1] != 8:
-            raise ValueError("observer state must be [channels, 8]")
-        state = state.detach().to(torch.float64)
+        """Restore a saved state (checkpoints; QuantizationManager.set_extra_state).  It goes to the GPU when there is
+        one; without one it stays on the host and the first kernel call fails loudly."""
+        state = self._adapt_state(state.detach().to(torch.float64))
         dev = self._state.device if self._state is not None else (torch.device("cuda") if torch.cuda.is_available()
                                                                    else state.device)
         if self._state is not None and self._state.shape == state.shape:
-            self._state.copy_(state)  # keeps arena bindings (parallel.py) intact
+            # in place: kernels hold pointers into the state (device_qparams() in bank.WeightBank's pointer table, CUDA
+            # graphs captured with fixed qparams), which a new tensor would leave stale
+            self._state.copy_(state)
         else:
             self._state = state.to(dev).contiguous().clone()
         self._host = None
@@ -67,7 +81,7 @@ class MinMaxObserver(BaseObserver):
     def _ensure_state(self, x: torch.Tensor) -> torch.Tensor:
         C = 1 if self.ch_axis is None else x.shape[self.ch_axis]
         if self._state is None:
-            self._state = ops.new_observer_state(C, x.device)
+            self._state = self._new_state(C, x.device)
         elif self._state.shape[0] != C:
             raise ValueError(f"observer saw {self._state.shape[0]} channels before, now {C}")
         elif self._state.device != x.device:
@@ -170,18 +184,38 @@ class MinMaxObserver(BaseObserver):
         return self.get_scale_zero_point()
 
     def lsq_init_scale(self, bits: int, out: Optional[torch.Tensor] = None, dtype=torch.float64) -> torch.Tensor:
+        """The reference rule on the call statistics (columns 4..7), whatever columns follow them."""
         if self._state is None:
-            raise RuntimeError("LSQObserver.lsq_init_scale() before any observe()")
+            raise RuntimeError(f"{type(self).__name__}.lsq_init_scale() before any observe()")
         C = self._state.shape[0]
         if out is None:
             out = torch.empty(C, dtype=dtype, device=self._state.device)
-        return ops.lsq_init_scale(self._state, bits, out)
+        return ops.lsq_init_scale(self._state[:, :STATE_WIDTH].contiguous(), bits, out)
 
     # device-side access for the sync-free manager path
     def device_qparams(self):
         """(scale, zero_point) views of the device state (fp64): usable directly as kernel qparams."""
         st = self._state
         return st[:, 2], st[:, 3]
+
+    # -- data-parallel merge (parallel.sync_observers) ------------------------------------------------
+    def sync_key(self) -> tuple:
+        """Observers with equal keys are merged together: their states are concatenated into one merge_states arena."""
+        return ("minmax",)
+
+    @classmethod
+    def merge_states(cls, arena: torch.Tensor, observers: list, group=None) -> None:
+        """Merge an arena (the concatenated states of ``observers``) over the ranks of ``group`` in place: running
+        extrema by MIN / MAX, call statistics summed, then scale / zero-point of every row from the merged range in one
+        launch."""
+        parallel.reduce_observer_states(arena, group)
+        ops.qparams_from_minmax(arena, *qparam_args(observers))
+
+    def after_merge(self) -> None:
+        """Runs once the merged rows are back in this observer's state: drop the host copies of the old ones."""
+        self._host = None
+        if self._on_change is not None:
+            self._on_change()
 
 
 @register_class

@@ -17,15 +17,15 @@ The per-channel vectors are tiny, so the running update is a handful of torch el
 synchronisation); ``ema_update_`` is device-agnostic and is checked bit for bit against torch's own observers on the CPU
 (tests/test_abi_and_host.py).  The state layout is the one of MinMaxObserver ([C, 8] fp64), so the manager's sync-free
 paths (device_qparams, lsq_init_scale, sync_observers' SUM columns) work unchanged.  Note that a MIN/MAX all-reduce is
-NOT the right exchange for moving averages: parallel.sync_observers averages these observers' running extrema over the
-ranks that have observed something and recomputes scale / zero-point with the formula above."""
+NOT the right exchange for moving averages: their merge (parallel.reduce_moving_average_states) averages the running
+extrema over the ranks that have observed something, and scale / zero-point are recomputed with the formula above."""
 from __future__ import annotations
 
 from typing import Optional
 
 import torch
 
-from .. import ops
+from .. import ops, parallel
 from ..utils.registry import register_class
 from .minmax import MinMaxObserver, _as_cuda
 
@@ -105,6 +105,21 @@ class MovingAverageMinMaxObserver(MinMaxObserver):
         st[:, 6] += mean
         st[:, 7] += torch.sqrt(torch.clamp(var, min=0.0))
         self._host = None
+
+    def sync_key(self) -> tuple:
+        return ("ema",)
+
+    @classmethod
+    def merge_states(cls, arena: torch.Tensor, observers: list, group=None) -> None:
+        parallel.reduce_moving_average_states(arena, group)
+
+    def after_merge(self) -> None:
+        """Scale / zero-point from the averaged running extrema with torch's formula, then drop the host copies."""
+        st = self._state
+        s, z = torch_qparams(st[:, 0].to(torch.float32), st[:, 1].to(torch.float32), self.quant_min, self.quant_max,
+                             bool(self.symmetric), float(self.eps))
+        st[:, 2], st[:, 3] = s.to(st.dtype), z.to(st.dtype)
+        super().after_merge()
 
 
 @register_class

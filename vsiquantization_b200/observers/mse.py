@@ -17,9 +17,10 @@ from typing import Optional
 
 import torch
 
-from .. import ops
+from .. import ops, parallel
+from .._lib import MSE_STATE_WIDTH, STATE_WIDTH
 from ..utils.registry import register_class
-from .minmax import MinMaxObserver, _as_cuda
+from .minmax import MinMaxObserver, _as_cuda, qparam_args
 
 
 @register_class
@@ -39,31 +40,18 @@ class MSEObserver(MinMaxObserver):
         self.last_alpha: Optional[torch.Tensor] = None
         self.keep_errors = False  # True: keep each call's E [C, K] and chosen alpha [C] on the device (diagnostics)
 
-    def load_state(self, state: torch.Tensor) -> None:
-        """Restore a saved [C, 10] state; a [C, 8] MinMax state is taken as a range whose clipped means are the range."""
-        if state.dim() != 2 or state.shape[1] not in (8, 10):
+    def _new_state(self, channels: int, device) -> torch.Tensor:
+        return ops.new_mse_state(channels, device)
+
+    def _adapt_state(self, state: torch.Tensor) -> torch.Tensor:
+        """A [C, 8] MinMax state is taken as a range whose clipped means are the range."""
+        if state.dim() != 2 or state.shape[1] not in (STATE_WIDTH, MSE_STATE_WIDTH):
             raise ValueError("MSE observer state must be [channels, 10] (or a [channels, 8] min/max state)")
-        state = state.detach().to(torch.float64)
-        if state.shape[1] == 8:
+        if state.shape[1] == STATE_WIDTH:
             state = torch.cat([state, state[:, 0:2]], dim=1)
-        dev = self._state.device if self._state is not None else (torch.device("cuda") if torch.cuda.is_available()
-                                                                   else state.device)
-        if self._state is not None and self._state.shape == state.shape:
-            self._state.copy_(state)
-        else:
-            self._state = state.to(dev).contiguous().clone()
-        self._host = None
+        return state
 
-    def _ensure_state(self, x: torch.Tensor) -> torch.Tensor:
-        C = 1 if self.ch_axis is None else x.shape[self.ch_axis]
-        if self._state is None:
-            self._state = ops.new_mse_state(C, x.device)
-        elif self._state.shape[0] != C:
-            raise ValueError(f"observer saw {self._state.shape[0]} channels before, now {C}")
-        elif self._state.device != x.device:
-            self._state = self._state.to(x.device)
-        return self._state
-
+    # getters only, so that assigning raises: MinMaxObserver's setters would recompute qparams from the unclipped range
     @property
     def min_val(self):
         """Running minimum (the unclipped range, as MinMaxObserver reports it)."""
@@ -83,11 +71,15 @@ class MSEObserver(MinMaxObserver):
         self.last_count = x.numel() // st.shape[0]
         self._host = None
 
-    def lsq_init_scale(self, bits: int, out: Optional[torch.Tensor] = None, dtype=torch.float64) -> torch.Tensor:
-        """The reference rule on the call statistics (columns 4..7), unchanged by the search."""
-        if self._state is None:
-            raise RuntimeError("MSEObserver.lsq_init_scale() before any observe()")
-        C = self._state.shape[0]
-        if out is None:
-            out = torch.empty(C, dtype=dtype, device=self._state.device)
-        return ops.lsq_init_scale(self._state[:, :8].contiguous(), bits, out)
+    def sync_key(self) -> tuple:
+        return ("mse",)
+
+    @classmethod
+    def merge_states(cls, arena: torch.Tensor, observers: list, group=None) -> None:
+        """Range and call statistics as MinMaxObserver, clipped means weighted by call counts; scale / zero-point of
+        every row from the merged means in one launch."""
+        parallel.reduce_mse_states(arena, group)
+        means = arena[:, :STATE_WIDTH].clone()
+        means[:, 0:2] = arena[:, 8:10]
+        ops.qparams_from_minmax(means, *qparam_args(observers))
+        arena[:, 2:4] = means[:, 2:4]

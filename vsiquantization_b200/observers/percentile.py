@@ -21,7 +21,7 @@ from typing import Optional
 
 import torch
 
-from .. import ops
+from .. import ops, parallel
 from .._lib import HIST_STATE_HEAD
 from ..utils.registry import register_class
 from .minmax import MinMaxObserver, _as_cuda
@@ -35,47 +35,28 @@ class PercentileObserver(MinMaxObserver):
 
     needs_quantizer_bits = True  # QuantizationManager passes bits_width (the clip's qparams are at the quantiser's width)
     observe_epilogue = None      # no fused form: fused layers run their separate calibration passes
-    keeps_histogram = True       # parallel.sync_observers merges the counts (reduce_percentile_states)
 
     def __init__(self, symmetric=True, num_bits=8, eps=1e-8, ch_axis: Optional[int] = None, percentile: float = 99.99,
                  n_bins: int = 2048):
         super().__init__(symmetric, num_bits, eps, ch_axis)
-        n_bins = int(n_bins)
-        if not (256 <= n_bins <= 4096 and n_bins & (n_bins - 1) == 0):
-            raise ValueError("n_bins must be a power of two in 256..4096")
-        if not 0.0 < float(percentile) <= 100.0:
-            raise ValueError("percentile must be in (0, 100]")
-        self.n_bins = n_bins
+        ops._check_hist_args(n_bins, percentile)
+        self.n_bins = int(n_bins)
         self.percentile = float(percentile)
 
     @property
     def state_width(self) -> int:
         return HIST_STATE_HEAD + 2 * self.n_bins
 
-    def load_state(self, state: torch.Tensor) -> None:
-        """Restore a saved [C, 12 + 2 * n_bins] state.  A [C, 8] min/max state cannot be taken: a percentile needs the
-        histogram."""
+    def _new_state(self, channels: int, device) -> torch.Tensor:
+        return ops.new_percentile_state(channels, self.n_bins, device)
+
+    def _adapt_state(self, state: torch.Tensor) -> torch.Tensor:
+        """A [C, 8] min/max state cannot be taken: a percentile needs the histogram."""
         if state.dim() != 2 or state.shape[1] != self.state_width:
             raise ValueError(f"percentile observer state must be [channels, {self.state_width}] (n_bins = {self.n_bins})")
-        state = state.detach().to(torch.float64)
-        dev = self._state.device if self._state is not None else (torch.device("cuda") if torch.cuda.is_available()
-                                                                   else state.device)
-        if self._state is not None and self._state.shape == state.shape:
-            self._state.copy_(state)
-        else:
-            self._state = state.to(dev).contiguous().clone()
-        self._host = None
+        return state
 
-    def _ensure_state(self, x: torch.Tensor) -> torch.Tensor:
-        C = 1 if self.ch_axis is None else x.shape[self.ch_axis]
-        if self._state is None:
-            self._state = ops.new_percentile_state(C, self.n_bins, x.device)
-        elif self._state.shape[0] != C:
-            raise ValueError(f"observer saw {self._state.shape[0]} channels before, now {C}")
-        elif self._state.device != x.device:
-            self._state = self._state.to(x.device)
-        return self._state
-
+    # getters only, so that assigning raises: MinMaxObserver's setters would recompute qparams from the unclipped range
     @property
     def min_val(self):
         """Running minimum (the unclipped range, as MinMaxObserver reports it)."""
@@ -96,8 +77,7 @@ class PercentileObserver(MinMaxObserver):
     def set_percentile(self, percentile: float) -> None:
         """Clip at another percentile of the histogram already gathered: scale / zero-point are recomputed on the device,
         no data is needed (sweep percentiles after one calibration pass)."""
-        if not 0.0 < float(percentile) <= 100.0:
-            raise ValueError("percentile must be in (0, 100]")
+        ops._check_hist_args(self.n_bins, percentile)
         self.percentile = float(percentile)
         self.recompute_clip()
 
@@ -109,11 +89,14 @@ class PercentileObserver(MinMaxObserver):
         if self._on_change is not None:
             self._on_change()
 
-    def lsq_init_scale(self, bits: int, out: Optional[torch.Tensor] = None, dtype=torch.float64) -> torch.Tensor:
-        """The reference rule on the call statistics (columns 4..7), unchanged by the clip."""
-        if self._state is None:
-            raise RuntimeError("PercentileObserver.lsq_init_scale() before any observe()")
-        C = self._state.shape[0]
-        if out is None:
-            out = torch.empty(C, dtype=dtype, device=self._state.device)
-        return ops.lsq_init_scale(self._state[:, :8].contiguous(), bits, out)
+    def sync_key(self) -> tuple:
+        return ("percentile", self.n_bins)
+
+    @classmethod
+    def merge_states(cls, arena: torch.Tensor, observers: list, group=None) -> None:
+        """Range and call statistics as MinMaxObserver, histograms merged exactly; each observer re-clips in
+        after_merge, at its own percentile."""
+        parallel.reduce_percentile_states(arena, observers[0].n_bins, group)
+
+    def after_merge(self) -> None:
+        self.recompute_clip()  # also drops the host copies (_on_change)

@@ -565,6 +565,29 @@ def ci_epilogue_observe(x: torch.Tensor, state: torch.Tensor, bits: int = 8, sym
     return y, stats
 
 
+def _check_state(state: torch.Tensor, C: int, width: int, what: str, device) -> None:
+    if state.dtype != torch.float64 or not state.is_cuda or tuple(state.shape) != (C, width) \
+            or not state.is_contiguous() or state.device != device:
+        raise ValueError(f"{what} state must be a contiguous float64 tensor [{C}, {width}] on {device}")
+
+
+def _observe_first(x: torch.Tensor, ch_axis: Optional[int], state: torch.Tensor, width: int, what: str, bits: int,
+                   symmetric: bool, eps: float):
+    """The head of an observer call that reads x again after the min/max pass (mse_search, hist_observe): channels_last
+    activations quantised along dim 1 are read in place, anything else as _dense_for leaves it; the [C, width] state is
+    checked; then the min/max pass gives this call's statistics.  Returns (x as read, Layout, stats [C, 5])."""
+    ci = ch_axis == 1 and ci_supported(x)
+    if ci:
+        N, C, H, W = x.shape
+        outer, inner = N * H * W, 1
+    else:
+        x = _dense_for(x, "x", ch_axis)
+        outer, C, inner = layout_of(x.shape, ch_axis)
+    _check_state(state, C, width, what, x.device)
+    stats = _ci_observe(x, None, bits, symmetric, eps, True) if ci else observe(x, ch_axis, None, bits, symmetric, eps)
+    return x, Layout(outer, C, inner), stats
+
+
 def new_mse_state(channels: int = 1, device=None) -> torch.Tensor:
     """[channels, 10] fp64 MSE observer state: new_observer_state's eight columns, then the running means of the chosen
     clipped min / max."""
@@ -579,22 +602,11 @@ def mse_search(x: torch.Tensor, ch_axis: Optional[int], state: torch.Tensor, bit
     search over n_candidates clipped ranges and the state update, all on the device (no host sync).  channels_last
     activations quantised along dim 1 are searched in place (no layout conversion).
     Returns (stats [C, 5], err [C, K] or None, alpha [C] or None)."""
-    ci = ch_axis == 1 and ci_supported(x)
-    if not ci:
-        x = _dense_for(x, "x", ch_axis)
-    if ci:
-        N, C, H, W = x.shape
-        outer, inner = N * H * W, 1
-    else:
-        outer, C, inner = layout_of(x.shape, ch_axis)
-    lay = Layout(outer, C, inner)
     K = int(n_candidates)
-    if state.dtype != torch.float64 or not state.is_cuda or tuple(state.shape) != (C, _lib.MSE_STATE_WIDTH) \
-            or not state.is_contiguous() or state.device != x.device:
-        raise ValueError(f"MSE observer state must be a contiguous float64 tensor [{C}, {_lib.MSE_STATE_WIDTH}] on {x.device}")
     if not 1 <= K <= 256:
         raise ValueError("n_candidates must be in 1..256")
-    stats = _ci_observe(x, None, bits, symmetric, eps, True) if ci else observe(x, ch_axis, None, bits, symmetric, eps)
+    x, lay, stats = _observe_first(x, ch_axis, state, _lib.MSE_STATE_WIDTH, "MSE observer", bits, symmetric, eps)
+    C = lay.channels
     with torch.cuda.device(x.device):
         err = torch.empty(C, K, dtype=torch.float64, device=x.device) if want_err else None
         alpha = torch.empty(C, dtype=torch.float64, device=x.device) if want_err else None
@@ -625,30 +637,14 @@ def new_percentile_state(channels: int, n_bins: int = 2048, device=None) -> torc
     return st
 
 
-def _check_hist_state(state: torch.Tensor, C: int, n_bins: int, device) -> None:
-    W = _lib.HIST_STATE_HEAD + 2 * int(n_bins)
-    if state.dtype != torch.float64 or not state.is_cuda or tuple(state.shape) != (C, W) or not state.is_contiguous() \
-            or state.device != device:
-        raise ValueError(f"percentile observer state must be a contiguous float64 tensor [{C}, {W}] on {device}")
-
-
 def hist_observe(x: torch.Tensor, ch_axis: Optional[int], state: torch.Tensor, n_bins: int = 2048,
                  percentile: float = 99.99, bits: int = 8, symmetric: bool = True, eps: float = 1e-8) -> torch.Tensor:
     """One calibration call of the percentile observer (vsiq_hist_observe): the min/max pass for this call's statistics,
     then one histogram pass over x and the state update with the clip at `percentile`, all on the device (no host sync).
     channels_last activations quantised along dim 1 are read in place (no layout conversion).  Returns stats [C, 5]."""
     _check_hist_args(n_bins, percentile)
-    ci = ch_axis == 1 and ci_supported(x)
-    if not ci:
-        x = _dense_for(x, "x", ch_axis)
-    if ci:
-        N, C, H, W = x.shape
-        outer, inner = N * H * W, 1
-    else:
-        outer, C, inner = layout_of(x.shape, ch_axis)
-    lay = Layout(outer, C, inner)
-    _check_hist_state(state, C, n_bins, x.device)
-    stats = _ci_observe(x, None, bits, symmetric, eps, True) if ci else observe(x, ch_axis, None, bits, symmetric, eps)
+    x, lay, stats = _observe_first(x, ch_axis, state, _lib.HIST_STATE_HEAD + 2 * int(n_bins), "percentile observer",
+                                   bits, symmetric, eps)
     with torch.cuda.device(x.device):
         ws = _workspace(lib.vsiq_hist_observe_workspace_bytes(ctypes.byref(lay), int(n_bins)), x.device)
         check(lib.vsiq_hist_observe(x.data_ptr(), ctypes.byref(lay), stats.data_ptr(), state.data_ptr(), int(n_bins),
@@ -665,7 +661,7 @@ def hist_clip(state: torch.Tensor, n_bins: int, percentile: float, bits: int, sy
     _check_hist_args(n_bins, percentile)
     if state.dim() != 2:
         raise ValueError("percentile observer state must be [channels, 12 + 2 * n_bins]")
-    _check_hist_state(state, state.shape[0], n_bins, state.device)
+    _check_state(state, state.shape[0], _lib.HIST_STATE_HEAD + 2 * int(n_bins), "percentile observer", state.device)
     with torch.cuda.device(state.device):
         check(lib.vsiq_hist_clip(state.data_ptr(), state.shape[0], int(n_bins), float(percentile), int(bits),
                                  int(bool(symmetric)), float(eps), _stream_ptr()), "vsiq_hist_clip")

@@ -20,9 +20,8 @@ from typing import Dict, List, Tuple
 import torch
 import torch.distributed as dist
 
-STATE_WIDTH = 8  # run_min, run_max, scale, zero_point, n_calls, sum mean|x|, sum mean x, sum std
-MSE_STATE_WIDTH = 10  # STATE_WIDTH columns, then the running means of the chosen clipped min / max (observers/mse.py)
-HIST_STATE_HEAD = 12  # percentile observers (observers/percentile.py): [C, HIST_STATE_HEAD + 2 * n_bins]
+from . import ops
+from ._lib import HIST_STATE_HEAD, MSE_STATE_WIDTH, STATE_WIDTH
 
 
 def _world(group=None) -> int:
@@ -98,9 +97,8 @@ def reduce_percentile_states(states: torch.Tensor, n_bins: int, group=None) -> t
     counts coarsened to it (old bin i -> new bin i >> delta, exact); the counts summed (exact on integer-valued fp64), so
     every rank ends with the same bits -- the histogram a single process would hold after seeing every rank's calls.
     Columns 2, 3, 8, 9 (the clip) are left to be recomputed (ops.hist_clip).  Device-agnostic."""
+    ops._check_hist_args(n_bins, 100.0)
     B = int(n_bins)
-    if B < 256 or B > 4096 or B & (B - 1):
-        raise ValueError("n_bins must be a power of two in 256..4096")
     W = HIST_STATE_HEAD + 2 * B
     if states.dtype != torch.float64 or states.dim() != 2 or states.shape[1] != W:
         raise ValueError(f"states must be [rows, {W}] float64")
@@ -128,94 +126,44 @@ def reduce_percentile_states(states: torch.Tensor, n_bins: int, group=None) -> t
     return states
 
 
+def reduce_moving_average_states(states: torch.Tensor, group=None) -> torch.Tensor:
+    """All-reduce a packed [rows, 8] fp64 moving-average observer block in place: the running min / max AVERAGED over
+    the ranks that have observed something (n_calls > 0; a rank without data carries no information) and rounded to fp32
+    like the running update, the call statistics summed.  Scale / zero-point are left to be recomputed.
+    Device-agnostic."""
+    if _world(group) == 1:
+        return states
+    has = (states[:, 4:5] > 0).to(states.dtype)
+    packed = torch.cat([states[:, 0:2] * has, has, states[:, 4:8]], dim=1).contiguous()
+    dist.all_reduce(packed, op=dist.ReduceOp.SUM, group=group)
+    n = torch.clamp(packed[:, 2:3], min=1.0)
+    states[:, 0:2] = (packed[:, 0:2] / n).to(torch.float32).to(states.dtype)
+    states[:, 4:8] = packed[:, 3:7]
+    return states
+
+
 def sync_observers(model, group=None) -> int:
     """Make every rank's observers agree after sharded calibration; returns the number of observer rows synchronised.
-    Scales / zero-points are recomputed from the reduced extrema exactly as observers/minmax.py:67-74 would."""
-    from . import ops
-    every = [(m, m.observer) for _, m in quantization_managers(model) if m.observer.state is not None]
-    # moving-average observers (observers/moving_average.py) hold averages, not extrema: their running min / max are
-    # AVERAGED over the ranks and their qparams recomputed with torch's formula; the call statistics are summed
-    ema = [(m, o) for m, o in every if hasattr(o, "averaging_constant")]
-    # MSE observers (observers/mse.py): range and statistics like min/max observers, clipped means weighted by call counts;
-    # scale / zero-point then come from the combined means
-    mse = [(m, o) for m, o in every if o.state.shape[1] == MSE_STATE_WIDTH]
-    entries = [(m, o) for m, o in every if not hasattr(o, "averaging_constant") and o.state.shape[1] == STATE_WIDTH]
-    rows_mse = 0
-    if mse:
-        arena = torch.cat([o.state for _, o in mse]).contiguous()
-        reduce_mse_states(arena, group)
-        means = arena[:, :STATE_WIDTH].clone()
-        means[:, 0:2] = arena[:, 8:10]
-        bits = torch.cat([torch.full((o.state.shape[0],), int(o.num_bits), dtype=torch.int32) for _, o in mse])
-        sym = torch.cat([torch.full((o.state.shape[0],), int(bool(o.symmetric)), dtype=torch.int32) for _, o in mse])
-        eps = {float(o.eps) for _, o in mse}
-        if len(eps) != 1:
-            raise ValueError("observers with different eps cannot be recomputed in one launch")
-        ops.qparams_from_minmax(means, bits, sym, eps.pop())
-        arena[:, 2:4] = means[:, 2:4]
-        for m, o in mse:
+
+    Observers with equal ``sync_key()`` share one arena: their states are concatenated, merged over the ranks by their
+    class's ``merge_states`` (the collectives above, then what can be recomputed on the whole arena), copied back, and
+    each observer finishes with ``after_merge()``.  Groups run in module order, which every rank shares."""
+    groups: Dict[tuple, list] = {}
+    for _, m in quantization_managers(model):
+        if m.observer.state is not None:
+            groups.setdefault(m.observer.sync_key(), []).append(m.observer)
+    rows = 0
+    for observers in groups.values():
+        arena = torch.cat([o.state for o in observers]).contiguous()
+        observers[0].merge_states(arena, observers, group)
+        at = 0
+        for o in observers:
             k = o.state.shape[0]
-            o.state.copy_(arena[rows_mse:rows_mse + k])
-            o._host = None
-            m._invalidate()
-            rows_mse += k
-    # percentile observers (observers/percentile.py), found by class attribute: range and statistics like min/max
-    # observers, histograms merged exactly; each clip is then recomputed on the device at that observer's percentile
-    pct = [(m, o) for m, o in every if getattr(o, "keeps_histogram", False)]
-    for n_bins in sorted({o.n_bins for _, o in pct}):
-        same = [(m, o) for m, o in pct if o.n_bins == n_bins]
-        arena = torch.cat([o.state for _, o in same]).contiguous()
-        reduce_percentile_states(arena, n_bins, group)
-        row = 0
-        for m, o in same:
-            k = o.state.shape[0]
-            o.state.copy_(arena[row:row + k])
-            o.recompute_clip()  # also drops the manager's cached qparams (_on_change)
-            row += k
-        rows_mse += row
-    rows_ema = rows_mse
-    if ema:
-        from .observers.moving_average import torch_qparams
-        arena = torch.cat([o.state for _, o in ema]).contiguous()
-        w = _world(group)
-        if w > 1:
-            # ranks that never observed (n_calls == 0) carry no information: weight by "has data"
-            has = (arena[:, 4:5] > 0).to(arena.dtype)
-            packed = torch.cat([arena[:, 0:2] * has, has, arena[:, 4:8]], dim=1).contiguous()
-            dist.all_reduce(packed, op=dist.ReduceOp.SUM, group=group)
-            n = torch.clamp(packed[:, 2:3], min=1.0)
-            arena[:, 0:2] = (packed[:, 0:2] / n).to(torch.float32).to(arena.dtype)
-            arena[:, 4:8] = packed[:, 3:7]
-        row = 0
-        for m, o in ema:
-            k = o.state.shape[0]
-            blk = arena[row:row + k]
-            s_, z_ = torch_qparams(blk[:, 0].to(torch.float32), blk[:, 1].to(torch.float32), o.quant_min, o.quant_max,
-                                   bool(o.symmetric), float(o.eps))
-            blk[:, 2], blk[:, 3] = s_.to(arena.dtype), z_.to(arena.dtype)
-            o.state.copy_(blk)
-            o._host = None
-            m._invalidate()
-            row += k
-        rows_ema += row
-    if not entries:
-        return rows_ema
-    arena = torch.cat([o.state for _, o in entries]).contiguous()
-    reduce_observer_states(arena, group)
-    bits = torch.cat([torch.full((o.state.shape[0],), int(o.num_bits), dtype=torch.int32) for _, o in entries])
-    sym = torch.cat([torch.full((o.state.shape[0],), int(bool(o.symmetric)), dtype=torch.int32) for _, o in entries])
-    eps = {float(o.eps) for _, o in entries}
-    if len(eps) != 1:
-        raise ValueError("observers with different eps cannot be recomputed in one launch")
-    ops.qparams_from_minmax(arena, bits, sym, eps.pop())
-    row = 0
-    for m, o in entries:
-        k = o.state.shape[0]
-        o.state.copy_(arena[row:row + k])
-        o._host = None
-        m._invalidate()
-        row += k
-    return row + rows_ema
+            o.state.copy_(arena[at:at + k])
+            o.after_merge()
+            at += k
+        rows += at
+    return rows
 
 
 class QParamGradBucket:

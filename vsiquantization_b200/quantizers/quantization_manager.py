@@ -32,6 +32,7 @@ from typing import List, Optional
 import torch
 import torch.nn as nn
 
+from .._lib import STATE_WIDTH
 from ..observers.minmax import MinMaxObserver  # noqa: F401  (registers the plugin classes)
 from ..observers.moving_average import MovingAverageMinMaxObserver  # noqa: F401
 from ..observers.mse import MSEObserver  # noqa: F401
@@ -153,12 +154,12 @@ class QuantizationManager(nn.Module):
         C = st.shape[0] if st is not None else 0
         parts = [self._pack_value(self.__dict__.get("scale")), self._pack_value(self.__dict__.get("zero_point")),
                  self._pack_value(getattr(self.quantizer, "calib_grad_scale", 1))]
-        W = st.shape[1] if st is not None else 8
-        head = [self._MAGIC, 2.0 if W == 8 else 3.0, float(bool(self.is_observer_qparam)),
+        W = st.shape[1] if st is not None else STATE_WIDTH
+        head = [self._MAGIC, 2.0 if W == STATE_WIDTH else 3.0, float(bool(self.is_observer_qparam)),
                 float(bool(self.is_learning_scale)), float(bool(self.is_quantize)), float(bool(self._calibrated)), float(C)]
         for kind, vals in parts:
             head += [float(kind), float(len(vals))]
-        if W != 8:
+        if W != STATE_WIDTH:
             head.append(float(W))
         body = st.reshape(-1).tolist() if st is not None else []
         for _, vals in parts:
@@ -172,7 +173,7 @@ class QuantizationManager(nn.Module):
         C = int(v[6])
         kinds = [(int(v[7 + 2 * i]), int(v[8 + 2 * i])) for i in range(3)]
         off = self._HEADER
-        W = 8
+        W = STATE_WIDTH
         if v[1] == 3.0:
             W = int(v[off])
             off += 1
