@@ -379,7 +379,8 @@ int vsiq_ci_observe(const float *x, int64_t rows, int64_t channels, double *stat
  * the launch geometry, the kernels read the device copy).  Pointers inside the table (x, qparams) must stay valid;
  * per-step buffers (y, g, dx, gradient outputs) are launch arguments.  pre_op must be VSIQ_PRE_NONE. */
 typedef struct vsiq_mt_entry {
-    const float *x;              /* weight [rows, inner] fp32 (any alignment; 32-byte aligned is the fast path) */
+    const float *x;              /* weight [rows, inner] fp32 (any alignment; 32-byte aligned is the fast path); may be NULL
+                                    when rows * inner == 0 */
     int64_t rows;                /* output channels */
     int64_t inner;               /* elements per output channel */
     int64_t out_offset;          /* element offset of this tensor inside the flat y (fwd) / dx (bwd) buffer; multiple of 8 */
@@ -400,7 +401,8 @@ typedef struct vsiq_mt_entry {
 #define VSIQ_MT_MAX_TENSORS 4096
 /* Validates the entries and fills their plan fields; *total_tiles receives the tile count of the whole table. */
 int vsiq_mt_plan(vsiq_mt_entry *table_host, int n, uint32_t *total_tiles);
-/* y_flat[out_offset + i] = fq(x[i]) for every tensor of the table: one launch. */
+/* y_flat[out_offset + i] = fq(x[i]) for every tensor of the table: one launch (none, and y_flat may be NULL, when no
+ * tensor of the table has an element; dx_flat likewise below). */
 int vsiq_mt_fake_quant_fwd(const vsiq_mt_entry *table_host, const vsiq_mt_entry *table_dev, int n, float *y_flat,
                            vsiq_stream_t stream);
 /* dx_flat[out_offset + i], dscale_flat[qp_offset + c] (fp64), dzp_flat[qp_offset + c] (fp32) for every tensor:

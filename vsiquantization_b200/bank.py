@@ -75,7 +75,12 @@ class _Plan:
         self.dev = raw.to(device)
         self.learns = any(it[5] for it in items)
         self.ws_bytes = int(lib.vsiq_mt_workspace_bytes(self.total_tiles))
-        self.bwd_launches = (n + _lib.MT_PACK - 1) // _lib.MT_PACK + (1 if self.learns else 0)
+        # what vsiq_mt_* launch: nothing for a table without tiles, one streaming launch per pack of MT_PACK tensors
+        # that has tiles, one combine launch when a learning entry has qparam channels
+        self.fwd_launches = 1 if self.total_tiles else 0
+        packs = sum(1 for lo in range(0, n, _lib.MT_PACK)
+                    if any(self.host[i].n_tiles for i in range(lo, min(lo + _lib.MT_PACK, n))))
+        self.bwd_launches = packs + (1 if self.learns and self.total_q else 0)
 
     def view(self, flat: torch.Tensor, i: int) -> torch.Tensor:
         w = self.items[i][1]
@@ -93,7 +98,7 @@ class _BankFunction(torch.autograd.Function):
             y_flat = torch.empty(plan.total_out, dtype=torch.float32, device=dev)
             check(lib.vsiq_mt_fake_quant_fwd(plan.host, plan.dev.data_ptr(), len(plan.items), y_flat.data_ptr(),
                                              ops._stream_ptr()), "vsiq_mt_fake_quant_fwd")
-            ops._count_launch()
+            ops._count_launch(plan.fwd_launches)
         return tuple(plan.view(y_flat, i) for i in range(len(plan.items)))
 
     @staticmethod

@@ -171,7 +171,8 @@ extern "C" int vsiq_mt_plan(vsiq_mt_entry* table, int n, uint32_t* total_tiles) 
     uint64_t tiles = 0;
     for (int i = 0; i < n; ++i) {
         vsiq_mt_entry& e = table[i];
-        if (!e.x || e.rows < 0 || e.inner < 0 || e.out_offset < 0 || (e.out_offset & 7) || e.qp_offset < 0)
+        // an entry without elements is never read: its x may be NULL (torch gives every empty tensor a NULL data_ptr)
+        if ((!e.x && e.rows && e.inner) || e.rows < 0 || e.inner < 0 || e.out_offset < 0 || (e.out_offset & 7) || e.qp_offset < 0)
             return VSIQ_ERR_INVALID_ARG;
         if (e.qp_channels != 1 && e.qp_channels != e.rows) return VSIQ_ERR_INVALID_ARG;
         if (e.learn < 0 || e.learn > 2) return VSIQ_ERR_INVALID_ARG;
@@ -206,9 +207,10 @@ static uint32_t mt_total_tiles(const vsiq_mt_entry* table, int n) { return table
 
 extern "C" int vsiq_mt_fake_quant_fwd(const vsiq_mt_entry* table_host, const vsiq_mt_entry* table_dev, int n,
                                       float* y_flat, vsiq_stream_t stream) {
-    if (!table_host || !table_dev || n < 1 || n > VSIQ_MT_MAX_TENSORS || !y_flat) return VSIQ_ERR_INVALID_ARG;
+    if (!table_host || !table_dev || n < 1 || n > VSIQ_MT_MAX_TENSORS) return VSIQ_ERR_INVALID_ARG;
     const uint32_t total = mt_total_tiles(table_host, n);
-    if (total == 0) return VSIQ_OK;
+    if (total == 0) return VSIQ_OK;  // nothing to write: y_flat may be NULL (torch's empty buffer)
+    if (!y_flat) return VSIQ_ERR_INVALID_ARG;
     const uint32_t grid = (total + kWarps - 1) / kWarps;
     mt_fwd_kernel<<<grid, kThreads, 0, (cudaStream_t)stream>>>(table_dev, n, total, y_flat);
     return (int)cudaGetLastError();
@@ -219,8 +221,9 @@ extern "C" size_t vsiq_mt_workspace_bytes(uint32_t total_tiles) { return kWsHead
 extern "C" int vsiq_mt_lsq_bwd(const vsiq_mt_entry* table_host, const vsiq_mt_entry* table_dev, int n,
                                const float* const* g, float* dx_flat, double* dscale_flat, float* dzp_flat,
                                void* workspace, size_t workspace_bytes, vsiq_stream_t stream) {
-    if (!table_host || !table_dev || n < 1 || n > VSIQ_MT_MAX_TENSORS || !g || !dx_flat) return VSIQ_ERR_INVALID_ARG;
+    if (!table_host || !table_dev || n < 1 || n > VSIQ_MT_MAX_TENSORS || !g) return VSIQ_ERR_INVALID_ARG;
     const uint32_t total = mt_total_tiles(table_host, n);
+    if (!dx_flat && total) return VSIQ_ERR_INVALID_ARG;  // a table without tiles writes no dx
     bool learns = false;
     for (int i = 0; i < n; ++i) {
         if (!g[i] && table_host[i].n_tiles) return VSIQ_ERR_INVALID_ARG;
@@ -242,8 +245,8 @@ extern "C" int vsiq_mt_lsq_bwd(const vsiq_mt_entry* table_host, const vsiq_mt_en
                                                                   partials);
         if (cudaError_t err = cudaGetLastError()) return (int)err;
     }
-    if (learns) {
-        const int64_t total_q = table_host[n - 1].qp_offset + table_host[n - 1].qp_channels;
+    const int64_t total_q = table_host[n - 1].qp_offset + table_host[n - 1].qp_channels;
+    if (learns && total_q > 0) {  // learning entries with zero channels (rows == 0, per channel) have nothing to combine
         int64_t grid = (total_q + kWarps - 1) / kWarps;
         if (grid > 1184) grid = 1184;
         mt_combine_kernel<<<(unsigned)grid, kThreads, 0, (cudaStream_t)stream>>>(table_dev, n, total_q, partials,
