@@ -123,3 +123,70 @@ def observe(x, ch_axis, st: np.ndarray, n_bins: int = 2048, percentile: float = 
         st[c, 6] += mean
         st[c, 7] += np.sqrt(var if var > 0.0 else 0.0)
     clip(st, B, percentile, bits, symmetric, eps)
+
+
+def entropy_fold(st_row: np.ndarray, n_bins: int):
+    """(H, e): both sides of one channel's counts coarsened to e = max(e_neg, e_pos) and added, then H[0] = H[1] (the
+    search's working copy; the state is not modified)."""
+    B = n_bins
+    e_neg, e_pos = int(st_row[10]), int(st_row[11])
+    e = max(e_neg, e_pos)
+    H = (coarsen(st_row[HEAD:HEAD + B].astype(np.int64), e - e_neg)
+         + coarsen(st_row[HEAD + B:HEAD + 2 * B].astype(np.int64), e - e_pos))
+    H[0] = H[1]
+    return H, e
+
+
+def entropy_levels(run_min: float, bits: int, symmetric: bool) -> int:
+    """nq: 2^bits for an asymmetric grid over [0, hi], else 2^(bits - 1)."""
+    return 2 ** bits if (not symmetric and run_min >= 0.0) else 2 ** (bits - 1)
+
+
+def kl_divergence(H: np.ndarray, i: int, nq: int) -> float:
+    """D_i = KL(P || Q) of threshold i over the magnitude histogram H, as plain direct sums in fp64."""
+    P = H[:i].astype(np.float64)
+    P[i - 1] += float(H[i:].sum())  # the outliers into the last bin
+    Hi = H[:i].astype(np.float64)
+    k = (np.arange(i, dtype=np.int64) * nq) // i  # chunk of bin j: floor(j nq / i)
+    nonzero = Hi != 0
+    mass = np.bincount(k, weights=Hi, minlength=nq)  # chunk sums, bin by bin
+    count = np.bincount(k, weights=nonzero.astype(np.float64), minlength=nq)
+    Q = np.where(nonzero, mass[k] / np.maximum(count[k], 1.0), 0.0)
+    if np.any((P > 0) & (Q == 0)):
+        return np.inf
+    p = P / P.sum()
+    q = Q / Q.sum()
+    m = p > 0
+    return float(np.sum(p[m] * np.log(p[m] / q[m])))
+
+
+def entropy_clip(st: np.ndarray, n_bins: int, start_bin: int, bits: int, symmetric: bool, eps: float = 1e-8):
+    """The entropy observer's search (include/vsiq.h, vsiq_hist_entropy_clip): columns 8, 9 and 2, 3 of every channel
+    from its counts, in place.  Returns the divergences [C, n_bins + 1] (NaN where i is no candidate)."""
+    B = n_bins
+    div = np.full((st.shape[0], B + 1), np.nan)
+    for c in range(st.shape[0]):
+        run_min, run_max = st[c, 0], st[c, 1]
+        lo, hi = run_min, run_max
+        if np.isfinite(run_min) and np.isfinite(run_max):
+            H, e = entropy_fold(st[c], B)
+            nz = np.flatnonzero(H)
+            n_used = int(nz[-1]) + 1 if nz.size else 0
+            nq = entropy_levels(run_min, bits, symmetric)
+            best, best_i = np.inf, -1
+            for i in range(max(start_bin, nq), n_used + 1):
+                d = kl_divergence(H, i, nq)
+                div[c, i] = d
+                if np.isnan(d):
+                    d = np.inf
+                if d <= best:  # increasing i: ties go to the larger threshold
+                    best, best_i = d, i
+            if best_i >= 0:
+                amax = best_i * 2.0 ** e
+                if -amax > lo:
+                    lo = -amax
+                if amax < hi:
+                    hi = amax
+        st[c, 8], st[c, 9] = lo, hi
+        st[c, 2], st[c, 3] = qparams(lo, hi, bits, symmetric, eps)
+    return div

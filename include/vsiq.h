@@ -245,6 +245,31 @@ int vsiq_hist_observe(const float *x, const vsiq_layout *layout, const double *s
 int vsiq_hist_clip(double *state, int64_t channels, int n_bins, double percentile, int bits, int symmetric, double eps,
                    vsiq_stream_t stream);
 
+/* ---- entropy observer: the KL-divergence clip searched over the percentile observer's histograms ----------------
+ * Recomputes columns 2, 3, 8, 9 of a [channels][VSIQ_HIST_STATE_HEAD + 2 * B] state (vsiq_hist_observe's layout, counts
+ * and exponents read only) as observers/entropy.py's EntropyObserver does after every call.  Per channel whose running
+ * range (columns 0, 1) is finite:
+ *   1. e = max(e_neg, e_pos); both sides coarsened to e (old bin i -> i >> (e - e_side)) and added into one magnitude
+ *      histogram H[0..B); then H[0] = H[1] in the search's working copy (the exact zeros of a ReLU output).
+ *   2. nq = 2^bits when asymmetric and run_min >= 0, else 2^(bits - 1).
+ *   3. candidates i in [max(start_bin, nq), n_used], n_used = 1 + the highest non-zero bin of H; none: the clip is the
+ *      running range.
+ *   4. D_i = KL(P || Q) in fp64: P = H[0..i) plus the outlier mass sum H[i..B) in bin i - 1; Q = H[0..i) without the
+ *      outliers, bin j in chunk floor(j nq / i), each chunk's mass spread evenly over its non-zero bins; both normalised;
+ *      D_i = sum_{p_j > 0} p_j ln(p_j / q_j), +inf when some p_j > 0 has q_j = 0.
+ *   5. i* = argmin D_i, ties to the largest i, NaN as +inf; amax = i* 2^e, lo = max(run_min, -amax),
+ *      hi = min(run_max, amax).
+ *   6. columns 8, 9 = (lo, hi); 2, 3 = their vsiq_qparams_from_minmax scale / zero-point.
+ * A channel whose running range is not finite keeps it.  start_bin = n_bins gives the min/max result bit for bit.
+ * n_bins: a power of two in 256..4096; start_bin: 1..n_bins; bits: 2..8.  divergences (optional, NULL: none):
+ * [channels][n_bins + 1] fp64, entry i = D_i, NaN where i is no candidate.  Workspace: the 256-byte header (left zero)
+ * and one record per scoring CTA.  Deterministic (every D_i one thread's sequential sum, a total-order argmin), no host
+ * synchronisation, graph-capturable.  Two launches (score + finalize). */
+size_t vsiq_hist_entropy_workspace_bytes(int64_t channels, int n_bins); /* 0 for invalid channels / n_bins */
+int vsiq_hist_entropy_clip(double *state, int64_t channels, int n_bins, int start_bin, int bits, int symmetric,
+                           double eps, double *divergences, void *workspace, size_t workspace_bytes,
+                           vsiq_stream_t stream);
+
 /* ---- BN re-estimation under data parallelism: the per-layer exchange as ONE kernel over NVLink peer memory -------
  * reestimate_BN_stats (utils/estimate_bn.py:56-99) with the batch sharded over ranks needs sum x / sum x^2 of every rank
  * before a layer's output can be normalised (SURVEY.md 8e).  Instead of combine kernel -> ncclAllReduce -> moments kernel,

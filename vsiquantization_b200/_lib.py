@@ -108,6 +108,9 @@ _SIGNATURES = {
     "vsiq_hist_observe": (c_int, [c_void_p, ctypes.POINTER(Layout), c_void_p, c_void_p, c_int, c_double, c_int, c_int,
                                   c_double, c_void_p, c_size_t, c_void_p]),
     "vsiq_hist_clip": (c_int, [c_void_p, c_int64, c_int, c_double, c_int, c_int, c_double, c_void_p]),
+    "vsiq_hist_entropy_workspace_bytes": (c_size_t, [c_int64, c_int]),
+    "vsiq_hist_entropy_clip": (c_int, [c_void_p, c_int64, c_int, c_int, c_int, c_int, c_double, c_void_p, c_void_p,
+                                       c_size_t, c_void_p]),
     "vsiq_peer_buffer_bytes": (c_size_t, []),
     "vsiq_peer_max_world": (c_int, []),
     "vsiq_peer_max_channels": (c_int, []),

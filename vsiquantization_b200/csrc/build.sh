@@ -12,7 +12,7 @@ OBJ="$(mktemp -d)"
 trap 'rm -rf "$OBJ"' EXIT
 FLAGS=(-gencode arch=compute_100a,code=sm_100a -O3 -std=c++17 -lineinfo -ccbin "$HOSTCXX" -Xcompiler -fPIC,-O2,-Wall ${VSIQ_NVCC_EXTRA:-})
 pids=()
-for f in abi fake_quant observer bn_fold channels_inner multi_tensor host_pipeline peer_exchange mse_search hist_observer; do
+for f in abi fake_quant observer bn_fold channels_inner multi_tensor host_pipeline peer_exchange mse_search hist_observer hist_entropy; do
     "$NVCC" "${FLAGS[@]}" -c "$HERE/$f.cu" -o "$OBJ/$f.o" &
     pids+=($!)
 done

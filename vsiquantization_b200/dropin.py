@@ -24,6 +24,7 @@ _TIER2 = {
     "observers.minmax": "vsiquantization_b200.observers.minmax",
     "observers.mse": "vsiquantization_b200.observers.mse",
     "observers.percentile": "vsiquantization_b200.observers.percentile",
+    "observers.entropy": "vsiquantization_b200.observers.entropy",
     "quantizers.base": "vsiquantization_b200.quantizers.base",
     "quantizers.uniform": "vsiquantization_b200.quantizers.uniform",
     "quantizers.quantization_manager": "vsiquantization_b200.quantizers.quantization_manager",
@@ -35,12 +36,15 @@ _TIER2 = {
 }
 
 
-def install_plugins(registry=None, mse_observer: bool = False, percentile_observer: bool = False):
+def install_plugins(registry=None, mse_observer: bool = False, percentile_observer: bool = False,
+                    entropy_observer: bool = False):
     """Register UniformQuantizer / LSQQuantizer / MinMaxObserver / LSQObserver (and this package's moving-average
     observers) in the REFERENCE's CLASS_REGISTRY (utils/registry.py:2; a later registration overwrites, :26).  Returns the
-    registry dict.  mse_observer=True also registers MSEObserver, percentile_observer=True PercentileObserver; the
-    reference's own QuantizationManager builds every observer at 8 bits (quantization_manager.py:41-42), so under Tier 1
-    they search / clip at 8 bits -- Tier 2's manager hands them the quantiser's width."""
+    registry dict.  mse_observer=True also registers MSEObserver, percentile_observer=True PercentileObserver,
+    entropy_observer=True EntropyObserver; the reference's own QuantizationManager builds every observer at 8 bits
+    (quantization_manager.py:41-42), so under Tier 1 they search / clip at 8 bits -- Tier 2's manager hands them the
+    quantiser's width."""
+    from .observers.entropy import EntropyObserver
     from .observers.minmax import LSQObserver, MinMaxObserver
     from .observers.moving_average import MovingAverageMinMaxObserver, MovingAveragePerChannelMinMaxObserver
     from .observers.mse import MSEObserver
@@ -50,7 +54,7 @@ def install_plugins(registry=None, mse_observer: bool = False, percentile_observ
         registry = importlib.import_module("utils.registry").CLASS_REGISTRY  # the reference's module
     for cls in (UniformQuantizer, LSQQuantizer, MinMaxObserver, LSQObserver, MovingAverageMinMaxObserver,
                 MovingAveragePerChannelMinMaxObserver) + ((MSEObserver,) if mse_observer else ()) \
-            + ((PercentileObserver,) if percentile_observer else ()):
+            + ((PercentileObserver,) if percentile_observer else ()) + ((EntropyObserver,) if entropy_observer else ()):
         registry[cls.__name__] = cls
     return registry
 

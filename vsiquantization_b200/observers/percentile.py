@@ -27,21 +27,21 @@ from ..utils.registry import register_class
 from .minmax import MinMaxObserver, _as_cuda
 
 
-@register_class
-class PercentileObserver(MinMaxObserver):
-    """State: [C, 12 + 2 * n_bins] fp64 on the device -- MinMaxObserver's eight columns (scale / zero-point those of the
+class HistogramObserver(MinMaxObserver):
+    """What the histogram observers share: MinMaxObserver's running state plus per-channel exact-bin histograms, in a
+    [C, 12 + 2 * n_bins] fp64 state on the device -- MinMaxObserver's eight columns (scale / zero-point those of the
     clipped range), the clipped lo / hi, the bin exponents of the negative and positive side, then the counts of x < 0
-    and of x >= 0 (see include/vsiq.h, vsiq_hist_observe)."""
+    and of x >= 0 (see include/vsiq.h, vsiq_hist_observe).  Subclasses choose the clip (recompute_clip); the histogram
+    and its cross-rank merge are the same, so one subclass's checkpoint loads into another."""
 
     needs_quantizer_bits = True  # QuantizationManager passes bits_width (the clip's qparams are at the quantiser's width)
     observe_epilogue = None      # no fused form: fused layers run their separate calibration passes
+    _kind = "histogram observer"
 
-    def __init__(self, symmetric=True, num_bits=8, eps=1e-8, ch_axis: Optional[int] = None, percentile: float = 99.99,
-                 n_bins: int = 2048):
+    def __init__(self, symmetric=True, num_bits=8, eps=1e-8, ch_axis: Optional[int] = None, n_bins: int = 2048):
         super().__init__(symmetric, num_bits, eps, ch_axis)
-        ops._check_hist_args(n_bins, percentile)
+        ops._check_hist_args(n_bins, 100.0)
         self.n_bins = int(n_bins)
-        self.percentile = float(percentile)
 
     @property
     def state_width(self) -> int:
@@ -51,9 +51,9 @@ class PercentileObserver(MinMaxObserver):
         return ops.new_percentile_state(channels, self.n_bins, device)
 
     def _adapt_state(self, state: torch.Tensor) -> torch.Tensor:
-        """A [C, 8] min/max state cannot be taken: a percentile needs the histogram."""
+        """A [C, 8] min/max state cannot be taken: the clip needs the histogram."""
         if state.dim() != 2 or state.shape[1] != self.state_width:
-            raise ValueError(f"percentile observer state must be [channels, {self.state_width}] (n_bins = {self.n_bins})")
+            raise ValueError(f"{self._kind} state must be [channels, {self.state_width}] (n_bins = {self.n_bins})")
         return state
 
     # getters only, so that assigning raises: MinMaxObserver's setters would recompute qparams from the unclipped range
@@ -65,6 +65,34 @@ class PercentileObserver(MinMaxObserver):
     @property
     def max_val(self):
         return self._scalar(1, 0)
+
+    def recompute_clip(self) -> None:
+        raise NotImplementedError
+
+    def sync_key(self) -> tuple:
+        return ("percentile", self.n_bins)
+
+    @classmethod
+    def merge_states(cls, arena: torch.Tensor, observers: list, group=None) -> None:
+        """Range and call statistics as MinMaxObserver, histograms merged exactly; each observer re-clips in
+        after_merge, by its own rule."""
+        parallel.reduce_percentile_states(arena, observers[0].n_bins, group)
+
+    def after_merge(self) -> None:
+        self.recompute_clip()  # also drops the host copies (_on_change)
+
+
+@register_class
+class PercentileObserver(HistogramObserver):
+    """Clip at a percentile of the histogram (see the module docstring)."""
+
+    _kind = "percentile observer"
+
+    def __init__(self, symmetric=True, num_bits=8, eps=1e-8, ch_axis: Optional[int] = None, percentile: float = 99.99,
+                 n_bins: int = 2048):
+        super().__init__(symmetric, num_bits, eps, ch_axis, n_bins)
+        ops._check_hist_args(n_bins, percentile)
+        self.percentile = float(percentile)
 
     def observe(self, x):
         x = _as_cuda(x.detach())
@@ -88,15 +116,3 @@ class PercentileObserver(MinMaxObserver):
         self._host = None
         if self._on_change is not None:
             self._on_change()
-
-    def sync_key(self) -> tuple:
-        return ("percentile", self.n_bins)
-
-    @classmethod
-    def merge_states(cls, arena: torch.Tensor, observers: list, group=None) -> None:
-        """Range and call statistics as MinMaxObserver, histograms merged exactly; each observer re-clips in
-        after_merge, at its own percentile."""
-        parallel.reduce_percentile_states(arena, observers[0].n_bins, group)
-
-    def after_merge(self) -> None:
-        self.recompute_clip()  # also drops the host copies (_on_change)

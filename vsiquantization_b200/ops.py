@@ -668,6 +668,39 @@ def hist_clip(state: torch.Tensor, n_bins: int, percentile: float, bits: int, sy
         _count_launch()
 
 
+def _check_entropy_args(n_bins: int, start_bin: int, bits: int) -> None:
+    _check_hist_args(n_bins, 100.0)
+    if not 1 <= int(start_bin) <= int(n_bins):
+        raise ValueError("start_bin must be in 1..n_bins")
+    if not 2 <= int(bits) <= 8:
+        raise ValueError("bits must be in 2..8")
+
+
+def hist_entropy_clip(state: torch.Tensor, n_bins: int, start_bin: int, bits: int, symmetric: bool = True,
+                      eps: float = 1e-8, divergences: Optional[torch.Tensor] = None) -> Optional[torch.Tensor]:
+    """Recompute the clip (columns 8, 9) and scale / zero-point (2, 3) of a percentile / entropy observer state in place
+    by the KL-divergence search over its stored counts (vsiq_hist_entropy_clip): no new data, no host sync.
+    divergences: an optional [C, n_bins + 1] float64 tensor on the state's device that receives D_i of every candidate
+    threshold i (NaN where i is no candidate); returned."""
+    _check_entropy_args(n_bins, start_bin, bits)
+    if state.dim() != 2:
+        raise ValueError("entropy observer state must be [channels, 12 + 2 * n_bins]")
+    C = state.shape[0]
+    _check_state(state, C, _lib.HIST_STATE_HEAD + 2 * int(n_bins), "entropy observer", state.device)
+    if divergences is not None:
+        if divergences.dtype != torch.float64 or tuple(divergences.shape) != (C, int(n_bins) + 1) \
+                or not divergences.is_contiguous() or divergences.device != state.device:
+            raise ValueError(f"divergences must be a contiguous float64 tensor [{C}, {int(n_bins) + 1}] on {state.device}")
+    with torch.cuda.device(state.device):
+        ws = _workspace(lib.vsiq_hist_entropy_workspace_bytes(C, int(n_bins)), state.device)
+        check(lib.vsiq_hist_entropy_clip(state.data_ptr(), C, int(n_bins), int(start_bin), int(bits),
+                                         int(bool(symmetric)), float(eps),
+                                         divergences.data_ptr() if divergences is not None else None, ws.data_ptr(),
+                                         ws.numel(), _stream_ptr()), "vsiq_hist_entropy_clip")
+        _count_launch(2)
+    return divergences
+
+
 def qparams_from_minmax(states: torch.Tensor, bits: torch.Tensor, symmetric: torch.Tensor, eps: float = 1e-8) -> None:
     """Recompute scale / zero-point of n observers in place from their running extrema [minmax.py:67-74]."""
     n = states.numel() // _lib.STATE_WIDTH

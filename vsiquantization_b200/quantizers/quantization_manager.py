@@ -33,7 +33,8 @@ import torch
 import torch.nn as nn
 
 from .._lib import STATE_WIDTH
-from ..observers.minmax import MinMaxObserver  # noqa: F401  (registers the plugin classes)
+from ..observers.entropy import EntropyObserver  # noqa: F401  (registers the plugin classes)
+from ..observers.minmax import MinMaxObserver  # noqa: F401
 from ..observers.moving_average import MovingAverageMinMaxObserver  # noqa: F401
 from ..observers.mse import MSEObserver  # noqa: F401
 from ..observers.percentile import PercentileObserver  # noqa: F401
@@ -50,7 +51,7 @@ class QuantizationManager(nn.Module):
         super().__init__()
         self.quantizer = CLASS_REGISTRY[quantizer_name](bits_width, is_symmetric)
         if observer_bits is None and getattr(CLASS_REGISTRY[observer_name], "needs_quantizer_bits", False):
-            observer_bits = bits_width  # an observer whose result depends on the quantiser's width (MSE, Percentile)
+            observer_bits = bits_width  # an observer whose result depends on the quantiser's width (MSE, the histograms)
         if observer_bits is None:
             self.observer = CLASS_REGISTRY[observer_name](is_symmetric)  # num_bits stays 8, like the reference
         else:
