@@ -7,11 +7,9 @@
 //   fake-quant of W': quantizers/uniform.py:54-55,95
 //
 // Roofline: HBM, 8 algorithmic bytes per element (read W, write W'), +4 when Wq is also written.
-#include "common.cuh"
+#include "reduce.cuh"
 
 namespace vsiq {
-
-constexpr int kFoldPartialWidth = 6;
 
 template <bool WANT_Q, bool WANT_STATS>
 struct FoldOp : OpBase {
@@ -61,13 +59,12 @@ __global__ void __launch_bounds__(kThreads)
                    const float* __restrict__ beta, const float* __restrict__ mean, const float* __restrict__ var,
                    float eps, Tiles tiles, float* __restrict__ W_out, float* __restrict__ b_out,
                    float* __restrict__ Wq_out, QPDev qpd, int qp_per_channel, double* __restrict__ stats, void* ws) {
-    __shared__ double s_red[kWarps][kFoldPartialWidth];
+    __shared__ StatsRec s_red[kWarps];
     constexpr int NOUT = WANT_Q ? 2 : 1;
     const float* const in[1] = {W};
     float* outs[2] = {W_out, Wq_out};
     float* const(&out)[NOUT] = reinterpret_cast<float* const(&)[NOUT]>(outs);
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    const bool leader = GROUP == 32 ? lane == 0 : threadIdx.x == 0;
+    const bool leader = GROUP == 32 ? (threadIdx.x & 31) == 0 : threadIdx.x == 0;
 
     FoldOp<WANT_Q, WANT_STATS> op;
     if (WANT_STATS) op.reset_stats();
@@ -85,53 +82,16 @@ __global__ void __launch_bounds__(kThreads)
     }
     if (!WANT_STATS) return;
 
-    // per-tensor statistics of W': one partial per group, combined by the last CTA
+    // per-tensor statistics of W': one record per group (fminf / fmaxf drop NaN, so a NaN seen turns both into NaN),
+    // combined by a warp of the last CTA
     double* partials = ws_partials(ws);
-    {
-        float mn = warp_min(op.bad ? NAN : op.mn), mx = warp_max(op.bad ? NAN : op.mx);
-        double sa = warp_sum(op.sa), s1 = warp_sum(op.s1), s2 = warp_sum(op.s2);
-        if (GROUP == 32) {
-            if (lane == 0) {
-                double* p = partials + (size_t)group_index<32>() * kFoldPartialWidth;
-                p[0] = (double)mn; p[1] = (double)mx; p[2] = sa; p[3] = s1; p[4] = s2;
-            }
-        } else {
-            if (lane == 0) {
-                s_red[warp][0] = (double)mn; s_red[warp][1] = (double)mx;
-                s_red[warp][2] = sa; s_red[warp][3] = s1; s_red[warp][4] = s2;
-            }
-            __syncthreads();
-            if (threadIdx.x == 0) {
-                float a = (float)s_red[0][0], b = (float)s_red[0][1];
-                double x2 = s_red[0][2], x3 = s_red[0][3], x4 = s_red[0][4];
-#pragma unroll
-                for (int w = 1; w < kWarps; ++w) {
-                    a = nanmin(a, (float)s_red[w][0]);
-                    b = nanmax(b, (float)s_red[w][1]);
-                    x2 += s_red[w][2]; x3 += s_red[w][3]; x4 += s_red[w][4];
-                }
-                double* p = partials + (size_t)blockIdx.x * kFoldPartialWidth;
-                p[0] = (double)a; p[1] = (double)b; p[2] = x2; p[3] = x3; p[4] = x4;
-            }
-        }
-    }
-    if (!last_cta_ticket((unsigned int*)ws, GROUP == 32 ? lane == 0 : threadIdx.x == 0)) return;
-    if (warp == 0) {
-        const uint32_t n_slots = group_count<GROUP>();
-        float mn = INFINITY, mx = -INFINITY;
-        double sa = 0.0, s1 = 0.0, s2 = 0.0;
-        for (uint32_t i = lane; i < n_slots; i += 32) {
-            const double* p = partials + (size_t)i * kFoldPartialWidth;
-            mn = nanmin(mn, (float)__ldcg(p));
-            mx = nanmax(mx, (float)__ldcg(p + 1));
-            sa += __ldcg(p + 2); s1 += __ldcg(p + 3); s2 += __ldcg(p + 4);
-        }
-        mn = warp_min(mn); mx = warp_max(mx);
-        sa = warp_sum(sa); s1 = warp_sum(s1); s2 = warp_sum(s2);
-        if (lane == 0) {
-            stats[0] = (double)mn; stats[1] = (double)mx; stats[2] = sa; stats[3] = s1; stats[4] = s2;
-        }
-    }
+    const StatsRec rec = block_record<GROUP>(
+        StatsRec{op.bad ? NAN : op.mn, op.bad ? NAN : op.mx, op.sa, op.s1, op.s2}, s_red);
+    if (leader) rec.store(partials + (size_t)group_index<GROUP>() * StatsRec::kSlot);
+    if (!last_cta_ticket((unsigned int*)ws, leader)) return;
+    ObserveOut o = {};
+    o.stats = stats;
+    if (threadIdx.x < 32) combine_channel<32>(partials, cta_records(group_count<GROUP>()), 1, 0, o, s_red);
 }
 
 // upper bound of groups any launch of this kernel can have (partials are per group)
@@ -152,7 +112,7 @@ using namespace vsiq;
 
 extern "C" size_t vsiq_bn_fold_workspace_bytes(int64_t channels, int64_t inner) {
     if (channels <= 0 || inner <= 0) return 0;
-    return kWsHeader + fold_max_groups(channels, inner) * kFoldPartialWidth * sizeof(double);
+    return kWsHeader + fold_max_groups(channels, inner) * StatsRec::kSlot * sizeof(double);
 }
 
 extern "C" int vsiq_bn_fold(const float* W, const float* bias, const float* gamma, const float* beta,

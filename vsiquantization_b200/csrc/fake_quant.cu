@@ -11,6 +11,7 @@
 // write dx; the mask is recomputed from x, per-channel outputs are O(C)), fused fwd+bwd 16.
 #include "common.cuh"
 #include "quant_ops.cuh"
+#include "reduce.cuh"
 
 namespace vsiq {
 
@@ -201,156 +202,64 @@ __global__ void __launch_bounds__(kThreads, 4)
 }
 
 // LSQ backward.  Every tile emits one partial record {E, B} (fp32 inside a warp, fp64 across warps);
-// the records of a channel are then combined in a fixed order in fp64 and scaled by the grad-scale:
+// the records of a channel are then combined in a fixed order in fp64 and scaled by the grad-scale (reduce.cuh):
 //   * small launches (a single wave of CTAs): by the last CTA to finish, in the same launch;
-//   * large launches: by lsq_finalize_kernel on the same stream, so the streaming CTAs retire without a
+//   * large launches: by finalize_kernel on the same stream, so the streaming CTAs retire without a
 //     fence or an atomic (a per-CTA __threadfence would expose the store latency of every tile).
 // Tile index = (o * C + c) * chunks + k, so channel c owns `outer * chunks` records.
 struct LsqOut {
+    QPDev qpd;
     void* dscale;
     void* dzp;
     int ds_f64, dz_f64;
     double gs_host;
     const float* gs_dev;
     int want_dz;
-};
-
-__device__ __forceinline__ void lsq_store_channel(const LsqOut& o, const QPDev& qpd, int64_t c, double e, double b) {
-    const double gs = o.gs_host * (o.gs_dev ? (double)__ldg(o.gs_dev) : 1.0);
-    const QP p = load_qp(qpd, c);
-    const double ds = gs * e;
-    if (o.ds_f64)
-        ((double*)o.dscale)[c] = ds;
-    else
-        ((float*)o.dscale)[c] = (float)ds;
-    if (o.want_dz) {
-        const float zr = rintf(p.zf);
-        const bool cz = qpd.zp_learned ? ((zr >= p.lo) && (zr <= p.hi)) : true;
-        const double dz = cz ? -gs * (double)p.s * b : 0.0;  // sum (g*s)*(m-1) = -s * sum_{clamped} g
-        if (o.dz_f64)
-            ((double*)o.dzp)[c] = dz;
+    __device__ __forceinline__ void store(int64_t c, const LsqRec& r) const {
+        const double gs = gs_host * (gs_dev ? (double)__ldg(gs_dev) : 1.0);
+        double ds, dz;
+        lsq_channel_grads(gs, r.e, r.b, qpd, c, &ds, &dz);
+        if (ds_f64)
+            ((double*)dscale)[c] = ds;
         else
-            ((float*)o.dzp)[c] = (float)dz;
-    }
-}
-
-// one THREAD combines channel c (few records per channel, many channels)
-__device__ __forceinline__ void lsq_combine_thread(const double* partials, const Tiles& tiles, int64_t outer, int64_t c,
-                                                   const LsqOut& o, const QPDev& qpd) {
-    const uint32_t items = (uint32_t)outer * tiles.chunks;
-    double e = 0.0, b = 0.0;
-    for (uint32_t i = 0; i < items; ++i) {
-        const size_t slot = record_slot(tiles, (uint32_t)outer, (uint32_t)c, i);
-        e += __ldcg(partials + 2 * slot);
-        b += __ldcg(partials + 2 * slot + 1);
-    }
-    lsq_store_channel(o, qpd, c, e, b);
-}
-
-// one warp combines channel c
-__device__ __forceinline__ void lsq_combine_warp(const double* partials, const Tiles& tiles, int64_t outer, int64_t c,
-                                                 const LsqOut& o, const QPDev& qpd) {
-    const int lane = threadIdx.x & 31;
-    const uint32_t items = (uint32_t)outer * tiles.chunks;
-    double e = 0.0, b = 0.0;
-    for (uint32_t i = lane; i < items; i += 32) {
-        const size_t slot = record_slot(tiles, (uint32_t)outer, (uint32_t)c, i);
-        e += __ldcg(partials + 2 * slot);
-        b += __ldcg(partials + 2 * slot + 1);
-    }
-    e = warp_sum(e);
-    b = warp_sum(b);
-    if (lane == 0) lsq_store_channel(o, qpd, c, e, b);
-}
-
-// a whole CTA combines channel c (long rows / per tensor: many records per channel)
-__device__ __forceinline__ void lsq_combine_cta(const double* partials, const Tiles& tiles, int64_t outer, int64_t c,
-                                                const LsqOut& o, const QPDev& qpd, double (*s_red)[2]) {
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    const uint32_t items = (uint32_t)outer * tiles.chunks;
-    double e = 0.0, b = 0.0;
-#pragma unroll 4
-    for (uint32_t i = threadIdx.x; i < items; i += kThreads) {
-        const size_t slot = record_slot(tiles, (uint32_t)outer, (uint32_t)c, i);
-        e += __ldcg(partials + 2 * slot);
-        b += __ldcg(partials + 2 * slot + 1);
-    }
-    e = warp_sum(e);
-    b = warp_sum(b);
-    __syncthreads();
-    if (lane == 0) {
-        s_red[warp][0] = e;
-        s_red[warp][1] = b;
-    }
-    __syncthreads();
-    if (threadIdx.x == 0) {
-        double es = 0.0, bs = 0.0;
-#pragma unroll
-        for (int w = 0; w < kWarps; ++w) {
-            es += s_red[w][0];
-            bs += s_red[w][1];
+            ((float*)dscale)[c] = (float)ds;
+        if (want_dz) {
+            if (dz_f64)
+                ((double*)dzp)[c] = dz;
+            else
+                ((float*)dzp)[c] = (float)dz;
         }
-        lsq_store_channel(o, qpd, c, es, bs);
     }
-}
+};
 
 template <int GROUP, int V, int MASK_MODE, bool WANT_DZ, bool RELU>
 __global__ void __launch_bounds__(kThreads, 3)  // <= 85 registers: three CTAs per SM (the RELU variants drifted to 95-110)
     lsq_bwd_kernel(const float* __restrict__ x, const float* __restrict__ g, float* __restrict__ dx, Tiles tiles,
-                   QPDev qpd, void* ws, LsqOut o, int64_t outer, int use_ticket) {
-    __shared__ double s_red[kWarps][2];
+                   void* ws, LsqOut o, int64_t outer, int use_ticket) {
+    __shared__ LsqRec s_red[kWarps];
     pdl_launch_dependents();
     const float* const in[2] = {x, g};
     float* const out[1] = {dx};
     double* partials = ws_partials(ws);
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const bool leader = GROUP == 32 ? (threadIdx.x & 31) == 0 : threadIdx.x == 0;
 
     LsqBwdOp<MASK_MODE, WANT_DZ, RELU> op;
     int64_t cur_channel = -1;
     for (uint32_t t = group_index<GROUP>(); t < tiles.n_tiles; t += group_count<GROUP>()) {
         const TileCursor<GROUP> c = tile_at<GROUP>(tiles, t);
         if (c.channel != cur_channel) {
-            op.p = load_qp(qpd, c.channel);
+            op.p = load_qp(o.qpd, c.channel);
             cur_channel = c.channel;
         }
         op.e_acc = 0.0f;
         op.b_acc = 0.0f;
         span_apply<GROUP, V, 2, 1>(in, out, c.offset, c.len, op);
-        const float e = warp_sum(op.e_acc);
-        const float b = WANT_DZ ? warp_sum(op.b_acc) : 0.0f;
-        if (GROUP == 32) {
-            if (lane == 0) {
-                partials[2 * (size_t)t] = (double)e;
-                partials[2 * (size_t)t + 1] = (double)b;
-            }
-        } else {
-            __syncthreads();  // s_red free again
-            if (lane == 0) {
-                s_red[warp][0] = (double)e;
-                s_red[warp][1] = (double)b;
-            }
-            __syncthreads();
-            if (threadIdx.x == 0) {
-                double es = 0.0, bs = 0.0;
-#pragma unroll
-                for (int w = 0; w < kWarps; ++w) {
-                    es += s_red[w][0];
-                    bs += s_red[w][1];
-                }
-                partials[2 * (size_t)t] = es;
-                partials[2 * (size_t)t + 1] = bs;
-            }
-        }
+        const LsqRec rec = block_record<GROUP>(LsqSums<float, WANT_DZ>{op.e_acc, op.b_acc}, s_red);
+        if (leader) rec.store(partials + (size_t)t * LsqRec::kSlot);
     }
     if (!use_ticket) return;
-    if (!last_cta_ticket((unsigned int*)ws, GROUP == 32 ? lane == 0 : threadIdx.x == 0)) return;
-    if ((uint32_t)outer * tiles.chunks <= kThreadCombineMaxItems) {
-        for (int64_t c = threadIdx.x; c < tiles.channels; c += kThreads) lsq_combine_thread(partials, tiles, outer, c, o, qpd);
-    } else if (tiles.channels < kWarps) {
-        for (int64_t c = 0; c < tiles.channels; ++c) lsq_combine_cta(partials, tiles, outer, c, o, qpd, s_red);
-    } else {
-        for (int64_t c = warp; c < tiles.channels; c += kWarps) lsq_combine_warp(partials, tiles, outer, c, o, qpd);
-    }
+    if (!last_cta_ticket((unsigned int*)ws, leader)) return;
+    combine_in_last_cta(partials, tiles, outer, o, s_red);
 }
 
 // Per-tensor LSQ backward (rows == 1): no tile ever needs its own record, so CTAs are persistent, steal 8192-element
@@ -360,16 +269,15 @@ __global__ void __launch_bounds__(kThreads, 3)  // <= 85 registers: three CTAs p
 template <int V, int MASK_MODE, bool WANT_DZ, bool RELU>
 __global__ void __launch_bounds__(kThreads, 3)  // <= 85 registers: three CTAs per SM (the RELU variants drifted to 95-110)
     lsq_bwd_pt_kernel(const float* __restrict__ x, const float* __restrict__ g, float* __restrict__ dx, Tiles tiles,
-                      QPDev qpd, void* ws, LsqOut o) {
-    __shared__ double s_red[kWarps][2];
+                      void* ws, LsqOut o) {
+    __shared__ LsqRec s_red[kWarps];
     __shared__ uint32_t s_tile[2];
     const float* const in[2] = {x, g};
     float* const out[1] = {dx};
     double* partials = ws_partials(ws);
     unsigned int* counter = (unsigned int*)ws + 1;
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     LsqBwdOp<MASK_MODE, WANT_DZ, RELU> op;
-    op.p = load_qp(qpd, 0);
+    op.p = load_qp(o.qpd, 0);
     double e_run = 0.0, b_run = 0.0;
     TileQueue tq;
     tq_init(tq, counter, tiles.n_tiles, s_tile);
@@ -381,46 +289,28 @@ __global__ void __launch_bounds__(kThreads, 3)  // <= 85 registers: three CTAs p
         e_run += (double)op.e_acc;
         if (WANT_DZ) b_run += (double)op.b_acc;
     }
-    const double e = warp_sum(e_run);
-    const double b = WANT_DZ ? warp_sum(b_run) : 0.0;
-    if (lane == 0) {
-        s_red[warp][0] = e;
-        s_red[warp][1] = b;
-    }
-    __syncthreads();
-    if (threadIdx.x == 0) {
-        double es = 0.0, bs = 0.0;
-#pragma unroll
-        for (int w = 0; w < kWarps; ++w) {
-            es += s_red[w][0];
-            bs += s_red[w][1];
-        }
-        partials[2 * (size_t)blockIdx.x] = es;
-        partials[2 * (size_t)blockIdx.x + 1] = bs;
-    }
+    const LsqRec rec = block_record<kThreads>(LsqSums<double, WANT_DZ>{e_run, b_run}, s_red);
+    if (threadIdx.x == 0) rec.store(partials + (size_t)blockIdx.x * LsqRec::kSlot);
     if (!last_cta_ticket((unsigned int*)ws, threadIdx.x == 0)) return;
     if (threadIdx.x == 0) *counter = 0;  // every other CTA has left its tile loop
-    Tiles rec = tiles;  // one record per CTA
-    rec.channels = 1;
-    rec.chunks = gridDim.x;
-    lsq_combine_cta(partials, rec, 1, 0, o, qpd, s_red);
+    combine_channel<kThreads>(partials, cta_records(gridDim.x), 1, 0, o, s_red);
 }
 
 // Per-channel LSQ backward on [outer, C, inner] with the channel-item schedule (see PcGeom): one flush per CTA.
 template <int GROUP, int V, bool WANT_DZ, bool RELU>
 __global__ void __launch_bounds__(kThreads, 3)  // <= 85 registers: three CTAs per SM (the RELU variants drifted to 95-110)
     lsq_bwd_pc_kernel(const float* __restrict__ x, const float* __restrict__ g, float* __restrict__ dx, PcGeom geo,
-                      QPDev qpd, void* ws, LsqOut o, int use_ticket) {
-    __shared__ double s_red[kWarps][2];
+                      void* ws, LsqOut o, int use_ticket) {
+    __shared__ LsqRec s_red[kWarps];
     pdl_launch_dependents();
     const float* const in[2] = {x, g};
     float* const out[1] = {dx};
     double* partials = ws_partials(ws);
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const int warp = threadIdx.x >> 5;
     const uint32_t C = (uint32_t)geo.channels;
     const uint32_t c = blockIdx.x % C, j = blockIdx.x / C;
     LsqBwdOp<VSIQ_MASK_ROUNDED, WANT_DZ, RELU> op;
-    op.p = load_qp(qpd, c);
+    op.p = load_qp(o.qpd, c);
     double e_run = 0.0, b_run = 0.0;
     const uint32_t first = GROUP == 32 ? j + (uint32_t)warp * geo.k : j;
     const uint32_t step = GROUP == 32 ? geo.k * kWarps : geo.k;
@@ -436,60 +326,11 @@ __global__ void __launch_bounds__(kThreads, 3)  // <= 85 registers: three CTAs p
         e_run += (double)op.e_acc;
         if (WANT_DZ) b_run += (double)op.b_acc;
     }
-    const double e = warp_sum(e_run);
-    const double b = WANT_DZ ? warp_sum(b_run) : 0.0;
-    if (lane == 0) {
-        s_red[warp][0] = e;
-        s_red[warp][1] = b;
-    }
-    __syncthreads();
-    if (threadIdx.x == 0) {
-        double es = 0.0, bs = 0.0;
-#pragma unroll
-        for (int w = 0; w < kWarps; ++w) {
-            es += s_red[w][0];
-            bs += s_red[w][1];
-        }
-        const size_t slot = (size_t)c * geo.k + j;
-        partials[2 * slot] = es;
-        partials[2 * slot + 1] = bs;
-    }
+    const LsqRec rec = block_record<kThreads>(LsqSums<double, WANT_DZ>{e_run, b_run}, s_red);
+    if (threadIdx.x == 0) rec.store(partials + ((size_t)c * geo.k + j) * LsqRec::kSlot);
     if (!use_ticket) return;
     if (!last_cta_ticket((unsigned int*)ws, threadIdx.x == 0)) return;
-    Tiles rec;  // k records per channel, contiguous
-    rec.rows = geo.channels;
-    rec.channels = geo.channels;
-    rec.inner = 0;
-    rec.chunks = geo.k;
-    rec.n_tiles = C * geo.k;
-    rec.tile = 0;
-    if (geo.k <= kThreadCombineMaxItems) {
-        for (int64_t cc = threadIdx.x; cc < geo.channels; cc += kThreads) lsq_combine_thread(partials, rec, 1, cc, o, qpd);
-    } else if (geo.channels < kWarps) {
-        for (int64_t cc = 0; cc < geo.channels; ++cc) lsq_combine_cta(partials, rec, 1, cc, o, qpd, s_red);
-    } else {
-        for (int64_t cc = warp; cc < geo.channels; cc += kWarps) lsq_combine_warp(partials, rec, 1, cc, o, qpd);
-    }
-}
-
-// MODE 0: thread per channel, 1: warp per channel, 2: CTA per channel
-template <int MODE>
-__global__ void __launch_bounds__(kThreads)
-    lsq_finalize_kernel(Tiles tiles, QPDev qpd, const void* ws, LsqOut o, int64_t outer) {
-    __shared__ double s_red[kWarps][2];
-    const double* partials = (const double*)((const char*)ws + kWsHeader);
-    pdl_wait();  // launched as a programmatic dependent of the streaming kernel: its records are complete from here on
-    if (MODE == 0) {
-        for (int64_t c = (int64_t)blockIdx.x * kThreads + threadIdx.x; c < tiles.channels; c += (int64_t)gridDim.x * kThreads)
-            lsq_combine_thread(partials, tiles, outer, c, o, qpd);
-    } else if (MODE == 2) {
-        for (int64_t c = blockIdx.x; c < tiles.channels; c += gridDim.x)
-            lsq_combine_cta(partials, tiles, outer, c, o, qpd, s_red);
-    } else {
-        for (int64_t c = (int64_t)blockIdx.x * kWarps + (threadIdx.x >> 5); c < tiles.channels;
-             c += (int64_t)gridDim.x * kWarps)
-            lsq_combine_warp(partials, tiles, outer, c, o, qpd);
-    }
+    combine_in_last_cta(partials, item_records(geo), 1, o, s_red);
 }
 
 // ------------------------------------------------------------------------------------ launchers
@@ -637,16 +478,8 @@ extern "C" int vsiq_fake_quant_fwd_bwd(const float* x, const float* g, float* y,
     return (int)cudaGetLastError();
 }
 
-// Partials: 2 doubles per slot; slots = tiles (multi-row) or launched groups (single row) -- sized for
-// the larger of the two so the caller need not know the launch geometry.
 extern "C" size_t vsiq_lsq_bwd_workspace_bytes(const vsiq_layout* layout) {
-    if (check_layout(layout)) return 0;
-    Tiles tc, tw;
-    size_t slots = 1;
-    if (make_tiles<kThreads>(layout->outer, layout->channels, layout->inner, &tc)) slots = tc.n_tiles;
-    if (layout->inner < kWarpGroupMaxInner && make_tiles<32>(layout->outer, layout->channels, layout->inner, &tw))
-        slots = tw.n_tiles > slots ? tw.n_tiles : slots;
-    return kWsHeader + 2 * slots * 2 * sizeof(double);  // x2: the per-channel schedule may use 4096-element units
+    return reduce_workspace_bytes(layout, LsqRec::kSlot);
 }
 
 extern "C" int vsiq_lsq_bwd(const float* x, const float* g, float* dx, void* dscale, int dscale_dtype, void* dzp,
@@ -659,8 +492,8 @@ extern "C" int vsiq_lsq_bwd(const float* x, const float* g, float* dx, void* dsc
     if (mask_mode == VSIQ_MASK_FUNLSQ && (dzp || (qp && qp->pre_op != VSIQ_PRE_NONE))) return VSIQ_ERR_UNSUPPORTED;
     if ((dscale_dtype != VSIQ_F32 && dscale_dtype != VSIQ_F64) || (dzp && dzp_dtype != VSIQ_F32 && dzp_dtype != VSIQ_F64))
         return VSIQ_ERR_INVALID_ARG;
-    QPDev qpd;
-    if (int e = fill_qp(qp, &qpd)) return e;
+    LsqOut lo;
+    if (int e = fill_qp(qp, &lo.qpd)) return e;
     if (qp->pre_op == VSIQ_PRE_SILU) return VSIQ_ERR_UNSUPPORTED;
     if (!workspace || workspace_bytes < vsiq_lsq_bwd_workspace_bytes(layout)) return VSIQ_ERR_WORKSPACE;
     cudaStream_t st = (cudaStream_t)stream;
@@ -673,9 +506,7 @@ extern "C" int vsiq_lsq_bwd(const float* x, const float* g, float* dx, void* dsc
     if (!x || !g || !dx) return VSIQ_ERR_INVALID_ARG;
     const bool warp_group = layout->inner < kWarpGroupMaxInner;
     const bool vec8 = aligned32(x) && aligned32(g) && aligned32(dx);
-    Tiles tiles;
-    LsqOut lo;
-    const bool per_tensor_dyn = layout->outer == 1 && layout->channels == 1 && !warp_group;
+    const bool relu = qp->pre_op == VSIQ_PRE_RELU;
     lo.dscale = dscale;
     lo.dzp = dzp;
     lo.ds_f64 = dscale_dtype == VSIQ_F64;
@@ -683,9 +514,42 @@ extern "C" int vsiq_lsq_bwd(const float* x, const float* g, float* dx, void* dsc
     lo.gs_host = grad_scale_host;
     lo.gs_dev = grad_scale_dev;
     lo.want_dz = dzp != nullptr;
+    DeviceProps dprops;
+    if (int e = get_device_props(&dprops)) return e;
+    PcGeom pc;
+    if (mask_mode == VSIQ_MASK_ROUNDED && layout->channels > 1 &&
+        make_pc_geom(layout->outer, layout->channels, layout->inner, warp_group, dprops.sm_count, &pc) &&
+        (size_t)pc.channels * pc.k * LsqRec::kSlot * sizeof(double) + kWsHeader <= workspace_bytes) {
+        const int grid = (int)(pc.channels * pc.k);
+        // one partial wave: the last CTA combines; more: no ticket, no fence -- the combine kernel is a programmatic dependent
+        const int use_ticket = grid <= dprops.sm_count * 4 ? 1 : 0;
+#define PC(G, V, Z, R) lsq_bwd_pc_kernel<G, V, Z, R><<<grid, kThreads, 0, st>>>(x, g, dx, pc, workspace, lo, use_ticket)
+#define PC2(G, V, Z) { if (relu) PC(G, V, Z, true); else PC(G, V, Z, false); }
+#define PC1(G, V) { if (dzp) PC2(G, V, true) else PC2(G, V, false) }
+        if (warp_group) { if (vec8) PC1(32, 8) else PC1(32, 1) } else { if (vec8) PC1(kThreads, 8) else PC1(kThreads, 1) }
+#undef PC1
+#undef PC2
+#undef PC
+        if (!use_ticket) launch_finalize<LsqRec>(item_records(pc), 1, false, workspace, lo, st);
+        return (int)cudaGetLastError();
+    }
+    Tiles tiles;
+    if (layout->outer == 1 && layout->channels == 1 && !warp_group) {  // per tensor: persistent CTAs
+        if (!make_tiles<kThreads>(1, 1, layout->inner, &tiles)) return VSIQ_ERR_INVALID_ARG;
+        const uint32_t cap = (uint32_t)dprops.sm_count * 3u;
+        const int grid = (int)(tiles.n_tiles < cap ? tiles.n_tiles : cap);
+#define PT(V, M, Z, R) lsq_bwd_pt_kernel<V, M, Z, R><<<grid, kThreads, 0, st>>>(x, g, dx, tiles, workspace, lo)
+#define PT2(V, M, Z) { if (relu) PT(V, M, Z, true); else PT(V, M, Z, false); }
+#define PT1(V) { if (mask_mode == VSIQ_MASK_FUNLSQ) PT(V, VSIQ_MASK_FUNLSQ, false, false); else if (dzp) PT2(V, VSIQ_MASK_ROUNDED, true) else PT2(V, VSIQ_MASK_ROUNDED, false) }
+        if (vec8) PT1(8) else PT1(1)
+#undef PT1
+#undef PT2
+#undef PT
+        return (int)cudaGetLastError();
+    }
 #define LAUNCH(G, V, M, Z)                                                                                     \
     {                                                                                                          \
-        if (qp->pre_op == VSIQ_PRE_RELU) {                                                                     \
+        if (relu) {                                                                                            \
             LAUNCH_R(G, V, M, Z, true);                                                                        \
         } else {                                                                                               \
             LAUNCH_R(G, V, M, Z, false);                                                                       \
@@ -698,75 +562,10 @@ extern "C" int vsiq_lsq_bwd(const float* x, const float* g, float* dx, void* dsc
             return VSIQ_ERR_INVALID_ARG;                                                                       \
         int grid = launch_grid(ctas_for_tiles<G>(tiles.n_tiles));                                              \
         if (grid < 0) return -grid;                                                                            \
-        const int use_ticket = (grid <= dprops.sm_count * 4 && tiles.n_tiles <= kTicketMaxRecords) ? 1 : 0;             \
-        lsq_bwd_kernel<G, V, M, Z, R><<<grid, kThreads, 0, st>>>(x, g, dx, tiles, qpd, workspace, lo,          \
-                                                              layout->outer, use_ticket);                      \
-        if (!use_ticket) {                                                                                     \
-            const int64_t items = layout->outer * (int64_t)tiles.chunks;                                       \
-            if (items <= kThreadCombineMaxItems) {                                                             \
-                int64_t fg = (layout->channels + kThreads - 1) / kThreads;                                     \
-                launch_pdl(lsq_finalize_kernel<0>, dim3((unsigned)(fg < 4096 ? fg : 4096)), dim3(kThreads), 0, st, tiles, qpd, workspace, lo, \
-                                                                                          layout->outer);      \
-            } else if (items >= 512) {                                                                         \
-                int fgrid = (int)(layout->channels < 1024 ? layout->channels : 1024);                          \
-                launch_pdl(lsq_finalize_kernel<2>, dim3((unsigned)fgrid), dim3(kThreads), 0, st, tiles, qpd, workspace, lo, layout->outer);  \
-            } else {                                                                                           \
-                int64_t fg = (layout->channels + kWarps - 1) / kWarps;                                         \
-                launch_pdl(lsq_finalize_kernel<1>, dim3((unsigned)(fg < 4096 ? fg : 4096)), dim3(kThreads), 0, st, tiles, qpd, workspace, lo, \
-                                                                                          layout->outer);      \
-            }                                                                                                  \
-        }                                                                                                      \
-    }
-    PcGeom pc;
-    DeviceProps dprops;
-    if (int e = get_device_props(&dprops)) return e;
-    if (mask_mode == VSIQ_MASK_ROUNDED && layout->channels > 1 &&
-        make_pc_geom(layout->outer, layout->channels, layout->inner, warp_group, dprops.sm_count, &pc) &&
-        (size_t)pc.channels * pc.k * 2 * sizeof(double) + kWsHeader <= workspace_bytes) {
-        const int grid = (int)(pc.channels * pc.k);
-        // one partial wave: the last CTA combines; more: no ticket, no fence -- the combine kernel is a programmatic dependent
-        const int use_ticket = grid <= dprops.sm_count * 4 ? 1 : 0;
-        const bool relu = qp->pre_op == VSIQ_PRE_RELU;
-#define PC(G, V, Z, R) lsq_bwd_pc_kernel<G, V, Z, R><<<grid, kThreads, 0, st>>>(x, g, dx, pc, qpd, workspace, lo, use_ticket)
-#define PC2(G, V, Z) { if (relu) PC(G, V, Z, true); else PC(G, V, Z, false); }
-#define PC1(G, V) { if (dzp) PC2(G, V, true) else PC2(G, V, false) }
-        if (warp_group) { if (vec8) PC1(32, 8) else PC1(32, 1) } else { if (vec8) PC1(kThreads, 8) else PC1(kThreads, 1) }
-#undef PC1
-#undef PC2
-#undef PC
-        if (!use_ticket) {
-            Tiles rec;
-            rec.rows = pc.channels;
-            rec.channels = pc.channels;
-            rec.inner = 0;
-            rec.chunks = pc.k;
-            rec.n_tiles = (uint32_t)grid;
-            rec.tile = 0;
-            if (pc.k <= kThreadCombineMaxItems) {
-                int64_t fg = (pc.channels + kThreads - 1) / kThreads;
-                launch_pdl(lsq_finalize_kernel<0>, dim3((unsigned)(fg < 4096 ? fg : 4096)), dim3(kThreads), 0, st, rec, qpd, workspace, lo, 1);
-            } else {
-                int64_t fg = (pc.channels + kWarps - 1) / kWarps;
-                launch_pdl(lsq_finalize_kernel<1>, dim3((unsigned)(fg < 4096 ? fg : 4096)), dim3(kThreads), 0, st, rec, qpd, workspace, lo, 1);
-            }
-        }
-        return (int)cudaGetLastError();
-    }
-    if (per_tensor_dyn) {
-        if (!make_tiles<kThreads>(1, 1, layout->inner, &tiles)) return VSIQ_ERR_INVALID_ARG;
-        DeviceProps dp;
-        if (int e = get_device_props(&dp)) return e;
-        const uint32_t cap = (uint32_t)dp.sm_count * 3u;
-        const int grid = (int)(tiles.n_tiles < cap ? tiles.n_tiles : cap);
-        const bool relu = qp->pre_op == VSIQ_PRE_RELU;
-#define PT(V, M, Z, R) lsq_bwd_pt_kernel<V, M, Z, R><<<grid, kThreads, 0, st>>>(x, g, dx, tiles, qpd, workspace, lo)
-#define PT2(V, M, Z) { if (relu) PT(V, M, Z, true); else PT(V, M, Z, false); }
-#define PT1(V) { if (mask_mode == VSIQ_MASK_FUNLSQ) PT(V, VSIQ_MASK_FUNLSQ, false, false); else if (dzp) PT2(V, VSIQ_MASK_ROUNDED, true) else PT2(V, VSIQ_MASK_ROUNDED, false) }
-        if (vec8) PT1(8) else PT1(1)
-#undef PT1
-#undef PT2
-#undef PT
-        return (int)cudaGetLastError();
+        const int use_ticket = (grid <= dprops.sm_count * 4 && tiles.n_tiles <= kTicketMaxRecords) ? 1 : 0;   \
+        lsq_bwd_kernel<G, V, M, Z, R><<<grid, kThreads, 0, st>>>(x, g, dx, tiles, workspace, lo, layout->outer, \
+                                                              use_ticket);                                     \
+        if (!use_ticket) launch_finalize<LsqRec>(tiles, layout->outer, true, workspace, lo, st);               \
     }
 #define CALL(G, V)                                   \
     {                                                \

@@ -149,15 +149,11 @@ __global__ void __launch_bounds__(kThreads)
         es = warp_sum(es);
         bs = warp_sum(bs);
         if (lane == 0) {
-            const QPDev qpd = mt_qpdev(e);
-            const QP p = load_qp(qpd, c);
             const double gs = e.grad_scale * (e.grad_scale_dev ? (double)__ldg(e.grad_scale_dev) : 1.0);
-            if (dscale_flat) dscale_flat[q] = gs * es;
-            if (dzp_flat && e.learn > 1) {
-                const float zr = rintf(p.zf);
-                const bool cz = qpd.zp_learned ? ((zr >= p.lo) && (zr <= p.hi)) : true;
-                dzp_flat[q] = cz ? (float)(-gs * (double)p.s * bs) : 0.0f;  // sum (g*s)*(m-1) = -s * sum_{clamped} g
-            }
+            double ds, dz;
+            lsq_channel_grads(gs, es, bs, mt_qpdev(e), c, &ds, &dz);
+            if (dscale_flat) dscale_flat[q] = ds;
+            if (dzp_flat && e.learn > 1) dzp_flat[q] = (float)dz;
         }
     }
 }

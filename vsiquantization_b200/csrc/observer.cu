@@ -12,10 +12,9 @@
 //
 // Roofline: HBM, 4 algorithmic bytes per element (one read of x; the reference makes five passes).
 #include "ci_common.cuh"
+#include "reduce.cuh"
 
 namespace vsiq {
-
-constexpr int kPartialWidth = 6;  // min, max, sum|x|, sum x, sum x^2, nan flag
 
 struct StatsOp : OpBase {
     float mn, mx;        // NaN-propagating extrema (FMNMX.NAN): a NaN input sticks, exactly torch.min / torch.max -- one
@@ -43,164 +42,31 @@ struct StatsOp : OpBase {
         s2 += (double)f2;
         fa = f1 = f2 = 0.0f;
     }
+    __device__ __forceinline__ StatsRec rec() const { return {mn, mx, sa, s1, s2}; }
 };
 
-// Reduce a group's StatsOp into one partial record (valid in thread 0 of the group / lane 0).
-template <int GROUP>
-__device__ __forceinline__ void stats_group_reduce(StatsOp& op, double (&out)[kPartialWidth],
-                                                   double (*s_red)[kPartialWidth]) {
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    float mn = warp_min(op.mn);
-    float mx = warp_max(op.mx);
-    double sa = warp_sum(op.sa), s1 = warp_sum(op.s1), s2 = warp_sum(op.s2);
-    if (GROUP == 32) {
-        out[0] = (double)mn;
-        out[1] = (double)mx;
-        out[2] = sa;
-        out[3] = s1;
-        out[4] = s2;
-        out[5] = 0.0;
-        return;
-    }
-    __syncthreads();
-    if (lane == 0) {
-        s_red[warp][0] = (double)mn;
-        s_red[warp][1] = (double)mx;
-        s_red[warp][2] = sa;
-        s_red[warp][3] = s1;
-        s_red[warp][4] = s2;
-    }
-    __syncthreads();
-    if (threadIdx.x == 0) {
-        float a = (float)s_red[0][0], b = (float)s_red[0][1];
-        double x2 = s_red[0][2], x3 = s_red[0][3], x4 = s_red[0][4];
-#pragma unroll
-        for (int w = 1; w < kWarps; ++w) {
-            a = nanmin(a, (float)s_red[w][0]);
-            b = nanmax(b, (float)s_red[w][1]);
-            x2 += s_red[w][2];
-            x3 += s_red[w][3];
-            x4 += s_red[w][4];
-        }
-        out[0] = (double)a;
-        out[1] = (double)b;
-        out[2] = x2;
-        out[3] = x3;
-        out[4] = x4;
-        out[5] = 0.0;
-    }
-}
-
-// What the combine step produces / updates for one channel.
-struct ObserveOut {
-    double* stats;  // [C][VSIQ_STATS_WIDTH] or null
-    double* state;  // [C][VSIQ_STATE_WIDTH] or null
-    int bits;
-    int symmetric;
-    double eps;
-    double count;   // elements per channel = outer * inner
-};
-
-__device__ __forceinline__ void observe_store_channel(const ObserveOut& o, int64_t c, float mn, float mx, double sa,
-                                                      double s1, double s2) {
-    if (o.stats) {
-        double* d = o.stats + c * VSIQ_STATS_WIDTH;
-        d[0] = (double)mn;
-        d[1] = (double)mx;
-        d[2] = sa;
-        d[3] = s1;
-        d[4] = s2;
-    }
-    if (o.state) observer_state_update(o.state + c * VSIQ_STATE_WIDTH, mn, mx, sa, s1, s2, o.count, o.bits, o.symmetric, o.eps);
-}
-
-// Combine the records of channel c: STRIDE threads cooperate (32 = one warp, kThreads = the whole CTA).
-template <int STRIDE>
-__device__ __forceinline__ void observe_combine(const double* partials, const Tiles& tiles, int64_t outer, int64_t c,
-                                                const ObserveOut& o, double (*s_red)[kPartialWidth]) {
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    const int tid = STRIDE == 1 ? 0 : (STRIDE == 32 ? lane : (int)threadIdx.x);
-    const uint32_t items = (uint32_t)outer * tiles.chunks;
-    float mn = INFINITY, mx = -INFINITY;
-    double sa = 0.0, s1 = 0.0, s2 = 0.0;
-#pragma unroll 2
-    for (uint32_t i = tid; i < items; i += STRIDE) {
-        const double* p = partials + (size_t)record_slot(tiles, (uint32_t)outer, (uint32_t)c, i) * kPartialWidth;
-        mn = nanmin(mn, (float)__ldcg(p));
-        mx = nanmax(mx, (float)__ldcg(p + 1));
-        sa += __ldcg(p + 2);
-        s1 += __ldcg(p + 3);
-        s2 += __ldcg(p + 4);
-    }
-    if (STRIDE == 1) {  // one thread owns the channel
-        observe_store_channel(o, c, mn, mx, sa, s1, s2);
-        return;
-    }
-    mn = warp_min(mn);
-    mx = warp_max(mx);
-    sa = warp_sum(sa);
-    s1 = warp_sum(s1);
-    s2 = warp_sum(s2);
-    if (STRIDE == 32) {
-        if (lane == 0) observe_store_channel(o, c, mn, mx, sa, s1, s2);
-        return;
-    }
-    __syncthreads();
-    if (lane == 0) {
-        s_red[warp][0] = (double)mn;
-        s_red[warp][1] = (double)mx;
-        s_red[warp][2] = sa;
-        s_red[warp][3] = s1;
-        s_red[warp][4] = s2;
-    }
-    __syncthreads();
-    if (threadIdx.x == 0) {
-        float a = (float)s_red[0][0], b = (float)s_red[0][1];
-        double x2 = s_red[0][2], x3 = s_red[0][3], x4 = s_red[0][4];
-#pragma unroll
-        for (int w = 1; w < kWarps; ++w) {
-            a = nanmin(a, (float)s_red[w][0]);
-            b = nanmax(b, (float)s_red[w][1]);
-            x2 += s_red[w][2];
-            x3 += s_red[w][3];
-            x4 += s_red[w][4];
-        }
-        observe_store_channel(o, c, a, b, x2, x3, x4);
-    }
-}
-
-// One record per tile; combined by the last CTA (small launches) or by observe_finalize_kernel (large ones).
+// One record per tile; combined by the last CTA (small launches) or by finalize_kernel (large ones).
 template <int GROUP, int V>
 __global__ void __launch_bounds__(kThreads)
     observe_kernel(const float* __restrict__ x, Tiles tiles, int64_t outer, void* ws, ObserveOut o, int use_ticket) {
-    __shared__ double s_red[kWarps][kPartialWidth];
+    __shared__ StatsRec s_red[kWarps];
     pdl_launch_dependents();
     const float* const in[1] = {x};
     float* const out[1] = {nullptr};
     double* partials = ws_partials(ws);
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const bool leader = GROUP == 32 ? (threadIdx.x & 31) == 0 : threadIdx.x == 0;
 
     StatsOp op;
     for (uint32_t t = group_index<GROUP>(); t < tiles.n_tiles; t += group_count<GROUP>()) {
         const TileCursor<GROUP> c = tile_at<GROUP>(tiles, t);
         op.reset();
         span_apply<GROUP, V, 1, 0>(in, out, c.offset, c.len, op);
-        double rec[kPartialWidth];
-        stats_group_reduce<GROUP>(op, rec, s_red);
-        if ((GROUP == 32 && lane == 0) || (GROUP != 32 && threadIdx.x == 0)) {
-#pragma unroll
-            for (int k = 0; k < kPartialWidth; ++k) partials[(size_t)t * kPartialWidth + k] = rec[k];
-        }
+        const StatsRec rec = block_record<GROUP>(op.rec(), s_red);
+        if (leader) rec.store(partials + (size_t)t * StatsRec::kSlot);
     }
     if (!use_ticket) return;
-    if (!last_cta_ticket((unsigned int*)ws, GROUP == 32 ? lane == 0 : threadIdx.x == 0)) return;
-    if ((uint32_t)outer * tiles.chunks <= kThreadCombineMaxItems) {
-        for (int64_t c = threadIdx.x; c < tiles.channels; c += kThreads) observe_combine<1>(partials, tiles, outer, c, o, s_red);
-    } else if (tiles.channels < kWarps) {
-        for (int64_t c = 0; c < tiles.channels; ++c) observe_combine<kThreads>(partials, tiles, outer, c, o, s_red);
-    } else {
-        for (int64_t c = warp; c < tiles.channels; c += kWarps) observe_combine<32>(partials, tiles, outer, c, o, s_red);
-    }
+    if (!last_cta_ticket((unsigned int*)ws, leader)) return;
+    combine_in_last_cta(partials, tiles, outer, o, s_red);
 }
 
 // Per-tensor observer (rows == 1): persistent CTAs on the look-ahead tile queue, statistics carried in registers,
@@ -208,7 +74,7 @@ __global__ void __launch_bounds__(kThreads)
 template <int V>
 __global__ void __launch_bounds__(kThreads)
     observe_pt_kernel(const float* __restrict__ x, Tiles tiles, void* ws, ObserveOut o) {
-    __shared__ double s_red[kWarps][kPartialWidth];
+    __shared__ StatsRec s_red[kWarps];
     __shared__ uint32_t s_tile[2];
     const float* const in[1] = {x};
     float* const out[1] = {nullptr};
@@ -222,18 +88,11 @@ __global__ void __launch_bounds__(kThreads)
         const TileCursor<kThreads> c = tile_at<kThreads>(tiles, t);
         span_apply<kThreads, V, 1, 0>(in, out, c.offset, c.len, op);
     }
-    double rec[kPartialWidth];
-    stats_group_reduce<kThreads>(op, rec, s_red);
-    if (threadIdx.x == 0) {
-#pragma unroll
-        for (int k = 0; k < kPartialWidth; ++k) partials[(size_t)blockIdx.x * kPartialWidth + k] = rec[k];
-    }
+    const StatsRec rec = block_record<kThreads>(op.rec(), s_red);
+    if (threadIdx.x == 0) rec.store(partials + (size_t)blockIdx.x * StatsRec::kSlot);
     if (!last_cta_ticket((unsigned int*)ws, threadIdx.x == 0)) return;
     if (threadIdx.x == 0) *counter = 0;
-    Tiles recs = tiles;
-    recs.channels = 1;
-    recs.chunks = gridDim.x;
-    observe_combine<kThreads>(partials, recs, 1, 0, o, s_red);
+    combine_channel<kThreads>(partials, cta_records(gridDim.x), 1, 0, o, s_red);
 }
 
 // Per-channel observer on [outer, C, inner] with the channel-item schedule (PcGeom): one record per CTA.  This is the
@@ -241,7 +100,7 @@ __global__ void __launch_bounds__(kThreads)
 template <int GROUP, int V>
 __global__ void __launch_bounds__(kThreads)
     observe_pc_kernel(const float* __restrict__ x, PcGeom geo, void* ws, ObserveOut o, int use_ticket) {
-    __shared__ double s_red[kWarps][kPartialWidth];
+    __shared__ StatsRec s_red[kWarps];
     pdl_launch_dependents();
     const float* const in[1] = {x};
     float* const out[1] = {nullptr};
@@ -260,29 +119,12 @@ __global__ void __launch_bounds__(kThreads)
         const int len = rem < geo.chunk ? (int)rem : geo.chunk;
         span_apply<GROUP, V, 1, 0>(in, out, ((int64_t)n * C + c) * geo.inner + start, len, op);
     }
-    double rec[kPartialWidth];
-    stats_group_reduce<kThreads>(op, rec, s_red);  // whole CTA -> one record (warps hold different units of channel c)
-    if (threadIdx.x == 0) {
-        const size_t slot = (size_t)c * geo.k + j;
-#pragma unroll
-        for (int q = 0; q < kPartialWidth; ++q) partials[slot * kPartialWidth + q] = rec[q];
-    }
+    // whole CTA -> one record (warps hold different units of channel c)
+    const StatsRec rec = block_record<kThreads>(op.rec(), s_red);
+    if (threadIdx.x == 0) rec.store(partials + ((size_t)c * geo.k + j) * StatsRec::kSlot);
     if (!use_ticket) return;
     if (!last_cta_ticket((unsigned int*)ws, threadIdx.x == 0)) return;
-    Tiles recs;
-    recs.rows = geo.channels;
-    recs.channels = geo.channels;
-    recs.inner = 0;
-    recs.chunks = geo.k;
-    recs.n_tiles = C * geo.k;
-    recs.tile = 0;
-    if (geo.k <= kThreadCombineMaxItems) {
-        for (int64_t cc = threadIdx.x; cc < geo.channels; cc += kThreads) observe_combine<1>(partials, recs, 1, cc, o, s_red);
-    } else if (geo.channels < kWarps) {
-        for (int64_t cc = 0; cc < geo.channels; ++cc) observe_combine<kThreads>(partials, recs, 1, cc, o, s_red);
-    } else {
-        for (int64_t cc = warp; cc < geo.channels; cc += kWarps) observe_combine<32>(partials, recs, 1, cc, o, s_red);
-    }
+    combine_in_last_cta(partials, item_records(geo), 1, o, s_red);
 }
 
 // ---------------------------------------------------------------------------------------------------------------
@@ -454,7 +296,7 @@ __global__ void __launch_bounds__(kThreads)
             x3 += s_red[w][lane][3];
             x4 += s_red[w][lane][4];
         }
-        observe_store_channel(o, c, a, bq, x2, x3, x4);
+        o.store(c, StatsRec{a, bq, x2, x3, x4});
     }
 }
 
@@ -474,7 +316,7 @@ __global__ void __launch_bounds__(kThreads, 3)
     ci_epilogue_observe_kernel(const float* __restrict__ x, const float* __restrict__ p0, const float* __restrict__ var,
                                const float* __restrict__ gamma, const float* __restrict__ beta, float eps,
                                float* __restrict__ y, CiGeom geo, void* ws, ObserveOut o) {
-    __shared__ double s_red[kWarps][kPartialWidth];
+    __shared__ StatsRec s_red[kWarps];
     __shared__ uint32_t s_tile[2];
     const int t = threadIdx.x;
     const bool active = t < geo.threads;
@@ -533,43 +375,12 @@ __global__ void __launch_bounds__(kThreads, 3)
         }
         if (!ci_sched_next(geo, sc, s_tile, t, r)) break;
     }
-    double rec[kPartialWidth];
-    stats_group_reduce<kThreads>(op, rec, s_red);
+    const StatsRec rec = block_record<kThreads>(op.rec(), s_red);
     double* partials = ws_partials(ws);
-    if (threadIdx.x == 0) {
-#pragma unroll
-        for (int k = 0; k < kPartialWidth; ++k) partials[(size_t)blockIdx.x * kPartialWidth + k] = rec[k];
-    }
+    if (threadIdx.x == 0) rec.store(partials + (size_t)blockIdx.x * StatsRec::kSlot);
     if (!last_cta_ticket((unsigned int*)ws, threadIdx.x == 0)) return;
     if (threadIdx.x == 0) *((unsigned int*)ws + 1) = 0;  // tile counter of the dynamic schedule
-    Tiles recs;
-    recs.rows = 1;
-    recs.channels = 1;
-    recs.inner = 0;
-    recs.chunks = gridDim.x;
-    recs.n_tiles = gridDim.x;
-    recs.tile = 0;
-    observe_combine<kThreads>(partials, recs, 1, 0, o, s_red);
-}
-
-// MODE 0: thread per channel, 1: warp per channel, 2: CTA per channel
-template <int MODE>
-__global__ void __launch_bounds__(kThreads)
-    observe_finalize_kernel(Tiles tiles, int64_t outer, const void* ws, ObserveOut o) {
-    __shared__ double s_red[kWarps][kPartialWidth];
-    const double* partials = (const double*)((const char*)ws + kWsHeader);
-    pdl_wait();  // a programmatic dependent of the streaming kernel
-    if (MODE == 0) {
-        for (int64_t c = (int64_t)blockIdx.x * kThreads + threadIdx.x; c < tiles.channels; c += (int64_t)gridDim.x * kThreads)
-            observe_combine<1>(partials, tiles, outer, c, o, s_red);
-    } else if (MODE == 2) {
-        for (int64_t c = blockIdx.x; c < tiles.channels; c += gridDim.x)
-            observe_combine<kThreads>(partials, tiles, outer, c, o, s_red);
-    } else {
-        for (int64_t c = (int64_t)blockIdx.x * kWarps + (threadIdx.x >> 5); c < tiles.channels;
-             c += (int64_t)gridDim.x * kWarps)
-            observe_combine<32>(partials, tiles, outer, c, o, s_red);
-    }
+    combine_channel<kThreads>(partials, cta_records(gridDim.x), 1, 0, o, s_red);
 }
 
 __global__ void qparams_kernel(double* state, int64_t n, const int32_t* __restrict__ bits,
@@ -629,13 +440,7 @@ __global__ void bn_reestimate_finish_kernel(const float* __restrict__ mean_sum, 
 using namespace vsiq;
 
 extern "C" size_t vsiq_observe_workspace_bytes(const vsiq_layout* layout) {
-    if (check_layout(layout)) return 0;
-    Tiles tc, tw;
-    size_t slots = 1;
-    if (make_tiles<kThreads>(layout->outer, layout->channels, layout->inner, &tc)) slots = tc.n_tiles;
-    if (layout->inner < kWarpGroupMaxInner && make_tiles<32>(layout->outer, layout->channels, layout->inner, &tw))
-        slots = tw.n_tiles > slots ? tw.n_tiles : slots;
-    return kWsHeader + 2 * slots * kPartialWidth * sizeof(double);  // x2: the per-channel schedule may use 4096-element units
+    return reduce_workspace_bytes(layout, StatsRec::kSlot);
 }
 
 extern "C" int vsiq_observe(const float* x, const vsiq_layout* layout, double* stats, double* state, int bits,
@@ -649,25 +454,19 @@ extern "C" int vsiq_observe(const float* x, const vsiq_layout* layout, double* s
     cudaStream_t st = (cudaStream_t)stream;
     const bool warp_group = layout->inner < kWarpGroupMaxInner;
     const bool vec8 = aligned32(x);
-    Tiles tiles;
     ObserveOut oo;
     oo.stats = stats;
-    const bool per_tensor_dyn = layout->outer == 1 && layout->channels == 1 && !warp_group;
     oo.state = state;
     oo.bits = bits;
     oo.symmetric = symmetric;
     oo.eps = eps;
     oo.count = (double)layout->outer * (double)layout->inner;
-    oo.bits = bits;
-    oo.symmetric = symmetric;
-    oo.eps = eps;
-    oo.count = (double)layout->outer * (double)layout->inner;
-    PcGeom pc;
     DeviceProps dprops;
     if (int e = get_device_props(&dprops)) return e;
+    PcGeom pc;
     if (layout->channels > 1 &&
         make_pc_geom(layout->outer, layout->channels, layout->inner, warp_group, dprops.sm_count, &pc) &&
-        (size_t)pc.channels * pc.k * kPartialWidth * sizeof(double) + kWsHeader <= workspace_bytes) {
+        (size_t)pc.channels * pc.k * StatsRec::kSlot * sizeof(double) + kWsHeader <= workspace_bytes) {
         const int grid = (int)(pc.channels * pc.k);
         const int use_ticket = grid <= dprops.sm_count * 4 ? 1 : 0;  // else: combine kernel as a programmatic dependent
         if (warp_group) {
@@ -677,33 +476,13 @@ extern "C" int vsiq_observe(const float* x, const vsiq_layout* layout, double* s
             if (vec8) observe_pc_kernel<kThreads, 8><<<grid, kThreads, 0, st>>>(x, pc, workspace, oo, use_ticket);
             else observe_pc_kernel<kThreads, 1><<<grid, kThreads, 0, st>>>(x, pc, workspace, oo, use_ticket);
         }
-        if (!use_ticket) {
-            Tiles recs;
-            recs.rows = pc.channels;
-            recs.channels = pc.channels;
-            recs.inner = 0;
-            recs.chunks = pc.k;
-            recs.n_tiles = (uint32_t)grid;
-            recs.tile = 0;
-            if (pc.k <= kThreadCombineMaxItems) {
-                int64_t fg = (pc.channels + kThreads - 1) / kThreads;
-                launch_pdl(observe_finalize_kernel<0>, dim3((unsigned)(fg < 4096 ? fg : 4096)), dim3(kThreads), 0, st, recs, 1, workspace, oo);
-            } else {
-                int64_t fg = (pc.channels + kWarps - 1) / kWarps;
-                launch_pdl(observe_finalize_kernel<1>, dim3((unsigned)(fg < 4096 ? fg : 4096)), dim3(kThreads), 0, st, recs, 1, workspace, oo);
-            }
-        }
+        if (!use_ticket) launch_finalize<StatsRec>(item_records(pc), 1, false, workspace, oo, st);
         return (int)cudaGetLastError();
     }
-    if (per_tensor_dyn) {
-        oo.bits = bits;
-        oo.symmetric = symmetric;
-        oo.eps = eps;
-        oo.count = (double)layout->inner;
+    Tiles tiles;
+    if (layout->outer == 1 && layout->channels == 1 && !warp_group) {  // per tensor: persistent CTAs
         if (!make_tiles<kThreads>(1, 1, layout->inner, &tiles)) return VSIQ_ERR_INVALID_ARG;
-        DeviceProps dp;
-        if (int e = get_device_props(&dp)) return e;
-        const uint32_t cap = (uint32_t)dp.sm_count * 4u;
+        const uint32_t cap = (uint32_t)dprops.sm_count * 4u;
         const int grid = (int)(tiles.n_tiles < cap ? tiles.n_tiles : cap);
         if (vec8)
             observe_pt_kernel<8><<<grid, kThreads, 0, st>>>(x, tiles, workspace, oo);
@@ -719,23 +498,9 @@ extern "C" int vsiq_observe(const float* x, const vsiq_layout* layout, double* s
         uint32_t want = G == kThreads ? tiles.n_tiles : (tiles.n_tiles + kWarps - 1) / kWarps;                  \
         int grid = launch_grid(want);                                                                           \
         if (grid < 0) return -grid;                                                                             \
-        const int use_ticket = (grid <= dprops.sm_count * 4 && tiles.n_tiles <= kTicketMaxRecords) ? 1 : 0;              \
+        const int use_ticket = (grid <= dprops.sm_count * 4 && tiles.n_tiles <= kTicketMaxRecords) ? 1 : 0;    \
         observe_kernel<G, V><<<grid, kThreads, 0, st>>>(x, tiles, layout->outer, workspace, oo, use_ticket);    \
-        if (!use_ticket) {                                                                                      \
-            const int64_t items = layout->outer * (int64_t)tiles.chunks;                                        \
-            if (items <= kThreadCombineMaxItems) {                                                              \
-                int64_t fg = (layout->channels + kThreads - 1) / kThreads;                                      \
-                launch_pdl(observe_finalize_kernel<0>, dim3((unsigned)(fg < 4096 ? fg : 4096)), dim3(kThreads), 0, st, tiles, layout->outer, \
-                                                                                              workspace, oo);   \
-            } else if (items >= 512) {                                                                          \
-                int fgrid = (int)(layout->channels < 1024 ? layout->channels : 1024);                           \
-                launch_pdl(observe_finalize_kernel<2>, dim3((unsigned)fgrid), dim3(kThreads), 0, st, tiles, layout->outer, workspace, oo);    \
-            } else {                                                                                            \
-                int64_t fg = (layout->channels + kWarps - 1) / kWarps;                                          \
-                launch_pdl(observe_finalize_kernel<1>, dim3((unsigned)(fg < 4096 ? fg : 4096)), dim3(kThreads), 0, st, tiles, layout->outer, \
-                                                                                              workspace, oo);   \
-            }                                                                                                   \
-        }                                                                                                       \
+        if (!use_ticket) launch_finalize<StatsRec>(tiles, layout->outer, true, workspace, oo, st);             \
     }
     if (warp_group) {
         if (vec8) CALL(32, 8) else CALL(32, 1)

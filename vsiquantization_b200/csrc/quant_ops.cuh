@@ -113,4 +113,14 @@ struct LsqBwdOp : QuantOpBase {
     }
 };
 
+// dscale and dzero_point of channel c from its combined LsqBwdOp sums E and B and the grad-scale gs
+__device__ __forceinline__ void lsq_channel_grads(double gs, double e, double b, const QPDev& qpd, int64_t c, double* ds,
+                                                  double* dz) {
+    const QP p = load_qp(qpd, c);
+    *ds = gs * e;
+    const float zr = rintf(p.zf);
+    const bool cz = qpd.zp_learned ? ((zr >= p.lo) && (zr <= p.hi)) : true;
+    *dz = cz ? -gs * (double)p.s * b : 0.0;  // sum (g*s)*(m-1) = -s * sum_{clamped} g
+}
+
 }  // namespace vsiq
