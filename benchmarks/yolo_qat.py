@@ -96,6 +96,8 @@ def build_model(args, device):
     model = getattr(yolov8, f"yolo_v8_{args.model}")(num_classes=20).to(device)
     qname = "LSQQuantizer" if args.lsq else "UniformQuantizer"
     oname = "LSQObserver" if args.lsq else "MinMaxObserver"
+    if args.fp8:  # FP8 E4M3 weights and activations (8-bit, symmetric by definition)
+        qname = "FP8Quantizer"
     cfg = FuseConfig(observer_w_name=oname, quantizer_w_name=qname, observer_a_name=oname, quantizer_a_name=qname,
                      w_symmetric=not args.asym, a_symmetric=not args.asym, is_fuse_bn=not args.keep_bn,
                      bits_w=args.w_bits, bits_a=args.a_bits,
@@ -335,6 +337,7 @@ def run(args) -> dict:
     res = {"model": f"yolov8{args.model}", "fused_layers": n_fused, "batch_per_gpu": args.batch, "imgsz": args.imgsz,
            "n_gpus": world, "steps": args.steps, "ms_per_step": ms / args.steps,
            "images_per_s": args.batch * world * args.steps / (ms * 1e-3), "quant_impl": args.quant_impl,
+           "fp8": bool(args.fp8),
            "w_bits": args.w_bits, "a_bits": args.a_bits, "asymmetric": args.asym, "per_channel": args.per_channel,
            "lsq": args.lsq, "mixed": args.mixed, "cuda_graph": args.cuda_graph, "channels_last": args.channels_last,
            "weight_bank": bool(bank is not None and (bank.last_used or args.cuda_graph)), "prefetch": pre is not None,
@@ -378,6 +381,7 @@ def parse(argv=None):
     ap.add_argument("--asym", action="store_true")
     ap.add_argument("--per-channel", action="store_true")
     ap.add_argument("--lsq", action="store_true")
+    ap.add_argument("--fp8", action="store_true", help="FP8 E4M3 weights and activations (FP8Quantizer) instead of integers")
     ap.add_argument("--mixed", action="store_true")
     ap.add_argument("--keep-bn", action="store_true")
     ap.add_argument("--calib-batches", type=int, default=2)

@@ -72,6 +72,12 @@ enum {
     VSIQ_MASK_FUNLSQ = 1   /* reference dead code FunLSQ: strict bounds on the unrounded x/s (uniform.py:144-150) */
 };
 
+/* FP8 value grids of the vsiq_fp8_* entry points (F = the largest finite value) */
+enum {
+    VSIQ_FP8_E4M3 = 1, /* float8_e4m3fn, F = 448 */
+    VSIQ_FP8_E5M2 = 2  /* float8_e5m2,   F = 57344 */
+};
+
 typedef struct vsiq_layout {
     int64_t outer;
     int64_t channels;
@@ -152,6 +158,46 @@ int vsiq_lsq_bwd(const float *x, const float *g, float *dx, void *dscale, int ds
                  int dzp_dtype, const vsiq_layout *layout, const vsiq_qparams *qp, double grad_scale_host,
                  const float *grad_scale_dev, int mask_mode, void *workspace, size_t workspace_bytes,
                  vsiq_stream_t stream);
+
+/* ---- FP8 fake-quant (E4M3 / E5M2) ---------------------------------------------------------
+ * The same layouts, qparams and rules as the integer entry points above, with the rounding step on the FP8 value set
+ * named by fp8_format (VSIQ_FP8_E4M3: F = 448, VSIQ_FP8_E5M2: F = 57344) instead of the integers.  Per element:
+ *   v = x / s;  c = clamp(v, -F, F);  q = value of fp8_rne(c);  y = q * s            (each op rounded once, fp32)
+ *   m = (c == v)   inclusive at +-F, false for NaN;  dx = (g * s) * m / s           (as vsiq_fake_quant_bwd_ste)
+ *   dscale[c] = gs * sum g * (q - m * v)                                             (as vsiq_lsq_bwd with z = 0)
+ * fp8_rne rounds to the nearest FP8 value, ties to an even mantissa; -0.0 stays -0.0 and NaN stays NaN.  The caller's gs
+ * is (F * numel / channels) ** -0.5 [* calib_grad_scale].  Symmetric only: qp->qmin == qp->qmax == 0 (else
+ * VSIQ_ERR_INVALID_ARG); qp->zero_point NULL, qp->zp_host 0 and qp->zp_learned 0 (else VSIQ_ERR_UNSUPPORTED).  An unknown
+ * fp8_format is VSIQ_ERR_INVALID_ARG.  pre_op VSIQ_PRE_RELU is fused as in the integer entry points; VSIQ_PRE_SILU is
+ * VSIQ_ERR_UNSUPPORTED here and fused by the channels_last entry points vsiq_ci_fp8_*. */
+/* y (optional when codes is given) and codes (optional): one byte per element, the float8_e4m3fn / float8_e5m2 encoding of
+ * q.  With codes: pre_op VSIQ_PRE_NONE, x (and y) 32-byte aligned, codes 16-byte aligned, else VSIQ_ERR_UNSUPPORTED. */
+int vsiq_fp8_fake_quant_fwd(const float *x, float *y, void *codes, const vsiq_layout *layout, const vsiq_qparams *qp,
+                            int fp8_format, vsiq_stream_t stream);
+int vsiq_fp8_fake_quant_bwd_ste(const float *x, const float *g, float *dx, const vsiq_layout *layout,
+                                const vsiq_qparams *qp, int fp8_format, vsiq_stream_t stream);
+/* Workspace: vsiq_lsq_bwd_workspace_bytes.  dzp must be NULL and mask_mode VSIQ_MASK_ROUNDED (else VSIQ_ERR_UNSUPPORTED).
+ * Deterministic like vsiq_lsq_bwd. */
+int vsiq_fp8_lsq_bwd(const float *x, const float *g, float *dx, void *dscale, int dscale_dtype, void *dzp, int dzp_dtype,
+                     const vsiq_layout *layout, const vsiq_qparams *qp, int fp8_format, double grad_scale_host,
+                     const float *grad_scale_dev, int mask_mode, void *workspace, size_t workspace_bytes,
+                     vsiq_stream_t stream);
+/* The channels_last epilogue on the FP8 grids: vsiq_ci_fake_quant_fwd / vsiq_ci_lsq_bwd (below) with the element arithmetic
+ * of the FP8 entry points above applied to act(x + bias[c]) (SiLU included); the same layout, alignment, workspace
+ * (vsiq_ci_workspace_bytes) and determinism rules.  dzp must be NULL (VSIQ_ERR_UNSUPPORTED); dscale and dbias come from
+ * the one backward pass. */
+int vsiq_ci_fp8_fake_quant_fwd(const float *x, const float *bias, float *y, int64_t rows, int64_t channels,
+                               const vsiq_qparams *qp, int64_t qp_channels, int fp8_format, void *workspace,
+                               size_t workspace_bytes, vsiq_stream_t stream);
+int vsiq_ci_fp8_lsq_bwd(const float *x, const float *bias, const float *g, float *dx, void *dscale, int dscale_dtype,
+                        void *dzp, int dzp_dtype, float *dbias, int64_t rows, int64_t channels, const vsiq_qparams *qp,
+                        int64_t qp_channels, int fp8_format, double grad_scale_host, const float *grad_scale_dev,
+                        int64_t g_row_pitch, void *workspace, size_t workspace_bytes, vsiq_stream_t stream);
+/* The FP8 scale of each channel from an observer's chosen range: scale[c] = max(|lo[c]|, |hi[c]|) / F, or 1.0 when that
+ * maximum is zero or not finite.  lo / hi: device fp64 arrays read at c * stride; scale: `channels` device fp64 values,
+ * overwritten in place.  No host synchronisation. */
+int vsiq_fp8_scale_from_range(const double *lo, const double *hi, int64_t stride, int64_t channels, int fp8_format,
+                              double *scale, vsiq_stream_t stream);
 
 /* ---- (1)+(2) observer ---------------------------------------------------------------------
  * One pass over x producing, per channel, {min, max, sum|x|, sum x, sum x^2} (fp64; min/max are the

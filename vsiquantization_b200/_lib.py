@@ -15,6 +15,8 @@ LIB_PATH = os.environ.get("VSIQ_LIB") or os.path.join(_HERE, "libvsiq.so")  # VS
 F32, F64 = 0, 1
 MASK_ROUNDED, MASK_FUNLSQ = 0, 1
 PRE_NONE, PRE_RELU, PRE_SILU = 0, 1, 2
+FP8_E4M3, FP8_E5M2 = 1, 2
+FP8_MAX = {FP8_E4M3: 448.0, FP8_E5M2: 57344.0}  # largest finite value of each format
 STATS_WIDTH, STATE_WIDTH = 5, 8
 MSE_STATE_WIDTH = 10
 HIST_STATE_HEAD = 12  # percentile observer state: [C, HIST_STATE_HEAD + 2 * n_bins]
@@ -71,6 +73,18 @@ _SIGNATURES = {
     "vsiq_lsq_bwd_workspace_bytes": (c_size_t, [ctypes.POINTER(Layout)]),
     "vsiq_lsq_bwd": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_int, ctypes.POINTER(Layout),
                              ctypes.POINTER(QParams), c_double, c_void_p, c_int, c_void_p, c_size_t, c_void_p]),
+    "vsiq_fp8_fake_quant_fwd": (c_int, [c_void_p, c_void_p, c_void_p, ctypes.POINTER(Layout), ctypes.POINTER(QParams), c_int,
+                                        c_void_p]),
+    "vsiq_fp8_fake_quant_bwd_ste": (c_int, [c_void_p, c_void_p, c_void_p, ctypes.POINTER(Layout), ctypes.POINTER(QParams),
+                                            c_int, c_void_p]),
+    "vsiq_fp8_lsq_bwd": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_int, ctypes.POINTER(Layout),
+                                 ctypes.POINTER(QParams), c_int, c_double, c_void_p, c_int, c_void_p, c_size_t, c_void_p]),
+    "vsiq_ci_fp8_fake_quant_fwd": (c_int, [c_void_p, c_void_p, c_void_p, c_int64, c_int64, ctypes.POINTER(QParams), c_int64,
+                                           c_int, c_void_p, c_size_t, c_void_p]),
+    "vsiq_ci_fp8_lsq_bwd": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_int, c_void_p,
+                                    c_int64, c_int64, ctypes.POINTER(QParams), c_int64, c_int, c_double, c_void_p, c_int64,
+                                    c_void_p, c_size_t, c_void_p]),
+    "vsiq_fp8_scale_from_range": (c_int, [c_void_p, c_void_p, c_int64, c_int64, c_int, c_void_p, c_void_p]),
     "vsiq_observe_workspace_bytes": (c_size_t, [ctypes.POINTER(Layout)]),
     "vsiq_observe": (c_int, [c_void_p, ctypes.POINTER(Layout), c_void_p, c_void_p, c_int, c_int, c_double, c_void_p,
                              c_size_t, c_void_p]),

@@ -203,7 +203,8 @@ class WeightBank:
 
     # ---- per step -------------------------------------------------------------------------------------
     def _collect(self):
-        """[(manager, weight, scale, zero_point, spec, learn, gs_host, gs_dev)] or None when any layer is not bankable."""
+        """[(manager, weight, scale, zero_point, spec, learn, gs_host, gs_dev)] of every layer but the FP8 ones, or None
+        when one of those is not bankable (or there is none)."""
         items, sig = [], []
         grad_on = torch.is_grad_enabled()
         device = None
@@ -211,6 +212,8 @@ class WeightBank:
             mgr = layer.weight_quantizer
             w, _ = layer.get_weight_bias()
             q = mgr.quantizer
+            if getattr(q, "fp8_format", 0):
+                continue  # the multi-tensor kernels know integer grids only: FP8 weights keep their per-layer launch
             collecting = (not mgr.is_learning_scale) and mgr.is_observer_qparam
             if (not mgr.is_quantize or collecting or not isinstance(w, torch.Tensor) or not w.is_cuda
                     or w.dtype != torch.float32 or w.dim() < 2 or not _dense_in_memory(w)
@@ -257,6 +260,8 @@ class WeightBank:
             sig.append((w.data_ptr(), tuple(w.stride()), scale.data_ptr() if s_t else float(scale),
                         zp.data_ptr() if z_t else float(zp), learn, gs_host, spec.qmin, spec.qmax, spec.zp_learned,
                         gs_dev is not None))
+        if not items:
+            return None, None
         return items, (tuple(sig), str(device))
 
     def prepare(self) -> bool:

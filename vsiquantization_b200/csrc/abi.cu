@@ -134,6 +134,26 @@ int fill_qp(const vsiq_qparams* in, QPDev* out) {
     return VSIQ_OK;
 }
 
+int fill_qp_fp8(const vsiq_qparams* in, int fp8_format, QPDev* out) {
+    if (!in || (fp8_format != VSIQ_FP8_E4M3 && fp8_format != VSIQ_FP8_E5M2)) return VSIQ_ERR_INVALID_ARG;
+    if (in->qmin != 0 || in->qmax != 0) return VSIQ_ERR_INVALID_ARG;  // the grid comes from fp8_format
+    if (in->pre_op != VSIQ_PRE_NONE && in->pre_op != VSIQ_PRE_RELU && in->pre_op != VSIQ_PRE_SILU) return VSIQ_ERR_INVALID_ARG;
+    if (in->scale_dtype != VSIQ_F32 && in->scale_dtype != VSIQ_F64) return VSIQ_ERR_INVALID_ARG;
+    // symmetric only: no zero-point tensor, a zero host zero-point, nothing learned
+    if (in->zero_point || in->zp_host != 0.0f || in->zp_learned) return VSIQ_ERR_UNSUPPORTED;
+    out->scale = in->scale;
+    out->zp = nullptr;
+    out->scale_f64 = in->scale_dtype == VSIQ_F64;
+    out->zp_f64 = 0;
+    out->scale_host = in->scale_host;
+    out->zp_host = 0.0f;
+    out->zp_learned = 0;
+    const float F = fp8_max(fp8_format);
+    out->lo = out->tlo = -F;
+    out->hi = out->thi = F;
+    return VSIQ_OK;
+}
+
 }  // namespace vsiq
 
 extern "C" int vsiq_version(void) { return VSIQ_VERSION; }

@@ -145,7 +145,7 @@ __device__ __forceinline__ void ci_leave(void* ws) {
 }
 
 // ---------------------------------------------------------------------------------------------- forward
-template <bool PCQ, bool BIAS, int ACT>
+template <bool PCQ, bool BIAS, int ACT, int GRID = kGridInt>
 __global__ void __launch_bounds__(kThreads, 3)  // 80 registers, 3 CTAs per SM: measured 5.84 -> 6.39 TB/s on [64,32,320,320]
     ci_fwd_kernel(const float* __restrict__ x, const float* __restrict__ bias, float* __restrict__ y, CiGeom geo,
                   QPDev qpd, void* ws) {
@@ -187,13 +187,13 @@ __global__ void __launch_bounds__(kThreads, 3)  // 80 registers, 3 CTAs per SM: 
                     for (int e = 0; e < kCiVec; ++e) {
                         const float xe = act_fwd<ACT>(BIAS ? __fadd_rn(vin[j].v[e], bv[e]) : vin[j].v[e]);
                         guard_note(guard, xe);
-                        out.v[e] = dequant(elem_fast(xe, p[e]).q, p[e]);
+                        out.v[e] = dequant(elem_fast<GRID>(xe, p[e]).q, p[e]);
                     }
                     if (guard_bad(guard)) {
 #pragma unroll
                         for (int e = 0; e < kCiVec; ++e) {
                             const float xe = act_fwd<ACT>(BIAS ? __fadd_rn(vin[j].v[e], bv[e]) : vin[j].v[e]);
-                            out.v[e] = dequant(elem_slow(xe, p[e]).q, p[e]);
+                            out.v[e] = dequant(elem_slow<GRID>(xe, p[e]).q, p[e]);
                         }
                     }
                     st4(const_cast<float*>(xp) + j * stride + dy, out);
@@ -339,7 +339,7 @@ __global__ void __launch_bounds__(kThreads, 3)
 
 // --------------------------------------------------------------------------------------------- backward
 // The element arithmetic of one vector (four channels): dx, and the LSQ terms when WANT_DS.
-template <bool BIAS, int ACT, bool WANT_DS>
+template <bool BIAS, int ACT, bool WANT_DS, int GRID = kGridInt>
 __device__ __forceinline__ void ci_bwd_vec(const Vec4& vx, const Vec4& vg, const QP (&p)[kCiVec], const float (&bv)[kCiVec],
                                            uint32_t seed, Vec4& out, float (&te)[kCiVec], float (&tb)[kCiVec],
                                            float (&tdb)[kCiVec]) {
@@ -353,7 +353,7 @@ __device__ __forceinline__ void ci_bwd_vec(const Vec4& vx, const Vec4& vg, const
         const float ge = vg.v[e];
         guard_note(guard, xe);
         guard_note(guard, ge);
-        const Elem el = elem_fast(xe, p[e]);
+        const Elem el = elem_fast<GRID>(xe, p[e]);
         out.v[e] = act_bwd<ACT>(xb, dx_fast(ge, el.m, p[e]));
         if (WANT_DS) {
             // g * ((q - z) - m * v): v is finite on this path, so the masked product is a predicated subtraction
@@ -369,7 +369,7 @@ __device__ __forceinline__ void ci_bwd_vec(const Vec4& vx, const Vec4& vg, const
             const float xb = BIAS ? __fadd_rn(vx.v[e], bv[e]) : vx.v[e];
             const float xe = act_fwd<ACT>(xb);
             const float ge = vg.v[e];
-            const Elem el = elem_slow(xe, p[e]);
+            const Elem el = elem_slow<GRID>(xe, p[e]);
             out.v[e] = act_bwd<ACT>(xb, dx_slow(ge, el.m, p[e]));
             if (WANT_DS) {
                 const float dd = __fsub_rn(el.q, p[e].z);
@@ -483,7 +483,7 @@ __device__ __forceinline__ void ci_bwd_flush(const double (&acc_e)[kCiVec], cons
 
 // Direct-load backward: used when grad_output is pitched (a channel slice of a wider NHWC tensor, which is what the
 // backward of torch.cat hands out: row r of g starts at g + r * g_pitch) or when VSIQ_CI_TMA=0.
-template <bool PCQ, bool BIAS, int ACT, bool WANT_DS>
+template <bool PCQ, bool BIAS, int ACT, bool WANT_DS, int GRID = kGridInt>
 __global__ void __launch_bounds__(kThreads, 2)
     ci_bwd_kernel(const float* __restrict__ x, const float* __restrict__ bias, const float* __restrict__ g,
                   float* __restrict__ dx, CiGeom geo, QPDev qpd, void* ws, CiOut o, int use_ticket, int64_t g_pitch) {
@@ -536,7 +536,7 @@ __global__ void __launch_bounds__(kThreads, 2)
                 for (int j = 0; j < kCiUnroll; ++j) {
                     if (s + j >= r.s1) continue;
                     Vec4 out;
-                    ci_bwd_vec<BIAS, ACT, WANT_DS>(vx[j], vg[j], p, bv, seed, out, te, tb, tdb);
+                    ci_bwd_vec<BIAS, ACT, WANT_DS, GRID>(vx[j], vg[j], p, bv, seed, out, te, tb, tdb);
                     st4(const_cast<float*>(xp) + j * stride + ddx, out);
                 }
                 if ((++it & (kCiBatches - 1)) == 0 || s + kCiUnroll >= r.s1) {
@@ -613,7 +613,7 @@ struct CiRing {
     int64_t vec0[kCiStages];   // its first vector
 };
 
-template <bool PCQ, bool BIAS, int ACT, bool WANT_DS>
+template <bool PCQ, bool BIAS, int ACT, bool WANT_DS, int GRID = kGridInt>
 __global__ void __launch_bounds__(kThreads + 32, 2)
     ci_bwd_tma_kernel(const float* __restrict__ x, const float* __restrict__ bias, const float* __restrict__ g,
                       float* __restrict__ dx, CiGeom geo, QPDev qpd, void* ws, CiOut o, int use_ticket, int64_t g_pitch) {
@@ -735,7 +735,7 @@ __global__ void __launch_bounds__(kThreads + 32, 2)
                 const Vec4 vx = lds4(xs + (size_t)u * kCiVec);
                 const Vec4 vg = lds4(gs + (size_t)u * kCiVec);
                 Vec4 out;
-                ci_bwd_vec<BIAS, ACT, WANT_DS>(vx, vg, p, bv, seed, out, te, tb, tdb);
+                ci_bwd_vec<BIAS, ACT, WANT_DS, GRID>(vx, vg, p, bv, seed, out, te, tb, tdb);
                 st4(dx + (v0 + u) * kCiVec, out);
             }
         }
@@ -784,11 +784,12 @@ extern "C" size_t vsiq_ci_workspace_bytes(int64_t rows, int64_t channels) {
     return kWsHeader + (size_t)sms * 2 * (size_t)(3 * channels) * sizeof(double);
 }
 
-extern "C" int vsiq_ci_fake_quant_fwd(const float* x, const float* bias, float* y, int64_t rows, int64_t channels,
-                                      const vsiq_qparams* qp, int64_t qp_channels, void* workspace,
-                                      size_t workspace_bytes, vsiq_stream_t stream) {
+// The launch bodies of the integer entry points and their FP8 siblings (GRID: common.cuh)
+template <int GRID>
+static int ci_fwd_impl(const float* x, const float* bias, float* y, int64_t rows, int64_t channels, const vsiq_qparams* qp,
+                       int64_t qp_channels, void* workspace, size_t workspace_bytes, vsiq_stream_t stream) {
     QPDev qpd;
-    if (int e = fill_qp(qp, &qpd)) return e;
+    if (int e = GRID == kGridInt ? fill_qp(qp, &qpd) : fill_qp_fp8(qp, GRID, &qpd)) return e;
     if (rows == 0) return VSIQ_OK;
     if (!x || !y) return VSIQ_ERR_INVALID_ARG;
     if (qp_channels != 1 && qp_channels != channels) return VSIQ_ERR_INVALID_ARG;
@@ -802,12 +803,28 @@ extern "C" int vsiq_ci_fake_quant_fwd(const float* x, const float* bias, float* 
     cudaStream_t st = (cudaStream_t)stream;
     const bool pcq = qp_channels == channels && channels > 1, hb = bias != nullptr;
     const int act = qp->pre_op;  // VSIQ_PRE_* == kAct*
-#define F(P, B, A) ci_fwd_kernel<P, B, A><<<grid, kThreads, 0, st>>>(x, bias, y, geo, qpd, workspace)
+#define F(P, B, A) ci_fwd_kernel<P, B, A, GRID><<<grid, kThreads, 0, st>>>(x, bias, y, geo, qpd, workspace)
 #define F2(P, B) { if (act == kActRelu) F(P, B, kActRelu); else if (act == kActSilu) F(P, B, kActSilu); else F(P, B, kActNone); }
     if (pcq) { if (hb) F2(true, true) else F2(true, false) } else { if (hb) F2(false, true) else F2(false, false) }
 #undef F2
 #undef F
     return (int)cudaGetLastError();
+}
+
+extern "C" int vsiq_ci_fake_quant_fwd(const float* x, const float* bias, float* y, int64_t rows, int64_t channels,
+                                      const vsiq_qparams* qp, int64_t qp_channels, void* workspace,
+                                      size_t workspace_bytes, vsiq_stream_t stream) {
+    return ci_fwd_impl<kGridInt>(x, bias, y, rows, channels, qp, qp_channels, workspace, workspace_bytes, stream);
+}
+
+extern "C" int vsiq_ci_fp8_fake_quant_fwd(const float* x, const float* bias, float* y, int64_t rows, int64_t channels,
+                                          const vsiq_qparams* qp, int64_t qp_channels, int fp8_format, void* workspace,
+                                          size_t workspace_bytes, vsiq_stream_t stream) {
+    if (fp8_format == VSIQ_FP8_E4M3)
+        return ci_fwd_impl<VSIQ_FP8_E4M3>(x, bias, y, rows, channels, qp, qp_channels, workspace, workspace_bytes, stream);
+    if (fp8_format == VSIQ_FP8_E5M2)
+        return ci_fwd_impl<VSIQ_FP8_E5M2>(x, bias, y, rows, channels, qp, qp_channels, workspace, workspace_bytes, stream);
+    return VSIQ_ERR_INVALID_ARG;
 }
 
 extern "C" int vsiq_ci_fake_quant_fwd2(const float* x, const float* bias, float* y, float* y2, int64_t rows,
@@ -864,13 +881,13 @@ extern "C" int vsiq_ci_bn_normalize(const float* x, const float* mean, const flo
     return (int)cudaGetLastError();
 }
 
-extern "C" int vsiq_ci_lsq_bwd(const float* x, const float* bias, const float* g, float* dx, void* dscale,
-                               int dscale_dtype, void* dzp, int dzp_dtype, float* dbias, int64_t rows, int64_t channels,
-                               const vsiq_qparams* qp, int64_t qp_channels, double grad_scale_host,
-                               const float* grad_scale_dev, int64_t g_row_pitch, void* workspace,
-                               size_t workspace_bytes, vsiq_stream_t stream) {
+template <int GRID>
+static int ci_lsq_bwd_impl(const float* x, const float* bias, const float* g, float* dx, void* dscale, int dscale_dtype,
+                           void* dzp, int dzp_dtype, float* dbias, int64_t rows, int64_t channels, const vsiq_qparams* qp,
+                           int64_t qp_channels, double grad_scale_host, const float* grad_scale_dev, int64_t g_row_pitch,
+                           void* workspace, size_t workspace_bytes, vsiq_stream_t stream) {
     QPDev qpd;
-    if (int e = fill_qp(qp, &qpd)) return e;
+    if (int e = GRID == kGridInt ? fill_qp(qp, &qpd) : fill_qp_fp8(qp, GRID, &qpd)) return e;
     if (qp_channels != 1 && qp_channels != channels) return VSIQ_ERR_INVALID_ARG;
     if (dzp && !dscale) return VSIQ_ERR_INVALID_ARG;
     if (g_row_pitch == 0) g_row_pitch = channels;
@@ -919,11 +936,13 @@ extern "C" int vsiq_ci_lsq_bwd(const float* x, const float* bias, const float* g
 #define B(P, H, R, D)                                                                                                      \
     {                                                                                                                      \
         if (use_tma) {                                                                                                     \
-            if (cudaError_t ae = set_smem_once<ci_bwd_tma_kernel<P, H, R, D>>(cur_dev, 3 * 2 * 16384)) return (int)ae;   \
-            ci_bwd_tma_kernel<P, H, R, D><<<grid, kThreads + 32, dyn_smem, st>>>(x, bias, g, dx, geo, qpd, workspace, o,    \
+            if (cudaError_t ae = set_smem_once<ci_bwd_tma_kernel<P, H, R, D, GRID>>(cur_dev, 3 * 2 * 16384))             \
+                return (int)ae;                                                                                            \
+            ci_bwd_tma_kernel<P, H, R, D, GRID><<<grid, kThreads + 32, dyn_smem, st>>>(x, bias, g, dx, geo, qpd, workspace, \
+                                                                                o,                                         \
                                                                                 use_ticket, g_row_pitch);                 \
         } else {                                                                                                           \
-            ci_bwd_kernel<P, H, R, D><<<grid, kThreads, 0, st>>>(x, bias, g, dx, geo, qpd, workspace, o, use_ticket,        \
+            ci_bwd_kernel<P, H, R, D, GRID><<<grid, kThreads, 0, st>>>(x, bias, g, dx, geo, qpd, workspace, o, use_ticket,  \
                                                                  g_row_pitch);                                            \
         }                                                                                                                  \
     }
@@ -941,4 +960,30 @@ extern "C" int vsiq_ci_lsq_bwd(const float* x, const float* bias, const float* g
             return (int)fe;
     }
     return (int)cudaGetLastError();
+}
+
+extern "C" int vsiq_ci_lsq_bwd(const float* x, const float* bias, const float* g, float* dx, void* dscale,
+                               int dscale_dtype, void* dzp, int dzp_dtype, float* dbias, int64_t rows, int64_t channels,
+                               const vsiq_qparams* qp, int64_t qp_channels, double grad_scale_host,
+                               const float* grad_scale_dev, int64_t g_row_pitch, void* workspace,
+                               size_t workspace_bytes, vsiq_stream_t stream) {
+    return ci_lsq_bwd_impl<kGridInt>(x, bias, g, dx, dscale, dscale_dtype, dzp, dzp_dtype, dbias, rows, channels, qp,
+                                     qp_channels, grad_scale_host, grad_scale_dev, g_row_pitch, workspace, workspace_bytes,
+                                     stream);
+}
+
+extern "C" int vsiq_ci_fp8_lsq_bwd(const float* x, const float* bias, const float* g, float* dx, void* dscale,
+                                   int dscale_dtype, void* dzp, int dzp_dtype, float* dbias, int64_t rows, int64_t channels,
+                                   const vsiq_qparams* qp, int64_t qp_channels, int fp8_format, double grad_scale_host,
+                                   const float* grad_scale_dev, int64_t g_row_pitch, void* workspace,
+                                   size_t workspace_bytes, vsiq_stream_t stream) {
+    if (fp8_format != VSIQ_FP8_E4M3 && fp8_format != VSIQ_FP8_E5M2) return VSIQ_ERR_INVALID_ARG;
+    if (dzp) return VSIQ_ERR_UNSUPPORTED;  // symmetric: no zero-point gradient
+    return fp8_format == VSIQ_FP8_E4M3
+               ? ci_lsq_bwd_impl<VSIQ_FP8_E4M3>(x, bias, g, dx, dscale, dscale_dtype, nullptr, dzp_dtype, dbias, rows,
+                                                channels, qp, qp_channels, grad_scale_host, grad_scale_dev, g_row_pitch,
+                                                workspace, workspace_bytes, stream)
+               : ci_lsq_bwd_impl<VSIQ_FP8_E5M2>(x, bias, g, dx, dscale, dscale_dtype, nullptr, dzp_dtype, dbias, rows,
+                                                channels, qp, qp_channels, grad_scale_host, grad_scale_dev, g_row_pitch,
+                                                workspace, workspace_bytes, stream);
 }

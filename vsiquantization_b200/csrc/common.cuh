@@ -172,14 +172,53 @@ __device__ __forceinline__ float clamp_t(float t, const QP& p) { return min_nan(
 __device__ __forceinline__ float quantize_t(float t, const QP& p) { return rintf(clamp_t(t, p)); }
 __device__ __forceinline__ float dequant(float q, const QP& p) { return __fmul_rn(__fsub_rn(q, p.z), p.s); }
 
+// ---- value grids ----------------------------------------------------------------------------------------------------
+// GRID selects what the rounding step maps onto: kGridInt = the integers (rint), VSIQ_FP8_E4M3 / VSIQ_FP8_E5M2 = the
+// finite values of that FP8 format (round to nearest, ties to an even mantissa).  An FP8 grid has no zero-point
+// (t = v, so a -0.0 quotient keeps its sign) and its QP carries lo = tlo = -F, hi = thi = F: clamp_t is then
+// torch.clamp(v, -F, F) and m = (clamp == v) its backward mask, inclusive at +-F and false for NaN.
+constexpr int kGridInt = 0;
+__host__ __device__ constexpr float fp8_max(int grid) { return grid == VSIQ_FP8_E4M3 ? 448.0f : 57344.0f; }
+
+// Two floats (|v| <= F or NaN, i.e. already clamped) to two FP8 codes in one F2FP: `lo` in the low byte.  satfinite only
+// matters for NaN (which stays NaN); the clamp has already kept every finite value inside the format's range.
+template <int GRID>
+__device__ __forceinline__ uint16_t fp8_pack2(float lo, float hi) {
+    uint16_t p;
+    if (GRID == VSIQ_FP8_E4M3)
+        asm("cvt.rn.satfinite.e4m3x2.f32 %0, %1, %2;" : "=h"(p) : "f"(hi), "f"(lo));
+    else
+        asm("cvt.rn.satfinite.e5m2x2.f32 %0, %1, %2;" : "=h"(p) : "f"(hi), "f"(lo));
+    return p;
+}
+// ... and their values back (exact: every FP8 value is an fp16 value is an fp32 value)
+template <int GRID>
+__device__ __forceinline__ void fp8_unpack2(uint16_t p, float& lo, float& hi) {
+    uint32_t h;
+    if (GRID == VSIQ_FP8_E4M3)
+        asm("cvt.rn.f16x2.e4m3x2 %0, %1;" : "=r"(h) : "h"(p));
+    else
+        asm("cvt.rn.f16x2.e5m2x2 %0, %1;" : "=r"(h) : "h"(p));
+    asm("{.reg .f16 l, u; mov.b32 {l, u}, %2; cvt.f32.f16 %0, l; cvt.f32.f16 %1, u;}" : "=f"(lo), "=f"(hi) : "r"(h));
+}
+// the rounding step of the element functions: t is already clamp_t'ed
+template <int GRID>
+__device__ __forceinline__ float grid_round(float t) {
+    if (GRID == kGridInt) return rintf(t);
+    float q, unused;
+    fp8_unpack2<GRID>(fp8_pack2<GRID>(t, 0.0f), q, unused);
+    return q;
+}
+
 // The IEEE division is the only out-of-line piece: scalar in, scalar out, so the call passes everything in registers and
 // no caller ever has to park its QP (or the op that holds it) in local memory for the sake of this rare path.
 static __device__ __noinline__ float div_ieee(float a, float b) { return __fdiv_rn(a, b); }
+template <int GRID = kGridInt>
 __device__ __forceinline__ Elem elem_slow(float x, const QP& p) {
     Elem e;
     e.v = div_ieee(x, p.s);
-    e.t = __fadd_rn(e.v, p.z);
-    e.q = quantize_t(e.t, p);
+    e.t = GRID == kGridInt ? __fadd_rn(e.v, p.z) : e.v;
+    e.q = grid_round<GRID>(clamp_t(e.t, p));
     e.m = (e.t >= p.tlo) && (e.t <= p.thi);
     return e;
 }
@@ -233,12 +272,13 @@ __device__ __forceinline__ float div_fast(float x, const QP& p) {
     const float q2 = __fmaf_rn(e1, p.r, q1);
     return copysignf(q2, q0);
 }
+template <int GRID = kGridInt>
 __device__ __forceinline__ Elem elem_fast(float x, const QP& p) {
     Elem e;
     e.v = div_fast(x, p);
-    e.t = __fadd_rn(e.v, p.z);
+    e.t = GRID == kGridInt ? __fadd_rn(e.v, p.z) : e.v;
     const float tc = clamp_t(e.t, p);
-    e.q = rintf(tc);
+    e.q = grid_round<GRID>(tc);
     e.m = (tc == e.t);  // clamped value unchanged <=> in range (false for NaN)
     return e;
 }
@@ -633,6 +673,7 @@ int ci_tile_override();     // VSIQ_CI_TILE=<steps per tile>, else 0 (automatic)
 int pc_chunk_override();    // VSIQ_PC_CHUNK=<elements per unit of the NCHW per-channel schedule>, else 0 (automatic)
 int check_layout(const vsiq_layout* l);
 int fill_qp(const vsiq_qparams* in, QPDev* out);
+int fill_qp_fp8(const vsiq_qparams* in, int fp8_format, QPDev* out);  // FP8 grid: qmin == qmax == 0, no zero-point
 
 // opt in to > 48 KB of dynamic shared memory once per kernel instantiation and device (thread-safe)
 template <auto Kernel>  // a non-type parameter: every instantiation of the kernel gets its own flags

@@ -31,21 +31,21 @@ __device__ __forceinline__ void run_elementwise(const float* const (&in)[NIN], f
     }
 }
 
-template <int GROUP, int V, bool RELU>
+template <int GROUP, int V, bool RELU, int GRID = kGridInt>
 __global__ void __launch_bounds__(kThreads) fq_fwd_kernel(const float* __restrict__ x, float* __restrict__ y,
                                                           Tiles tiles, QPDev qpd) {
     const float* const in[1] = {x};
     float* const out[1] = {y};
-    run_elementwise<GROUP, V, FwdOp<RELU>, 1, 1>(in, out, tiles, qpd);
+    run_elementwise<GROUP, V, FwdOp<RELU, GRID>, 1, 1>(in, out, tiles, qpd);
 }
 
-template <int GROUP, int V, bool RELU>
+template <int GROUP, int V, bool RELU, int GRID = kGridInt>
 __global__ void __launch_bounds__(kThreads) fq_bwd_ste_kernel(const float* __restrict__ x,
                                                               const float* __restrict__ g,
                                                               float* __restrict__ dx, Tiles tiles, QPDev qpd) {
     const float* const in[2] = {x, g};
     float* const out[1] = {dx};
-    run_elementwise<GROUP, V, SteBwdOp<RELU>, 2, 1>(in, out, tiles, qpd);
+    run_elementwise<GROUP, V, SteBwdOp<RELU, GRID>, 2, 1>(in, out, tiles, qpd);
 }
 
 template <int GROUP, int V>
@@ -201,6 +201,102 @@ __global__ void __launch_bounds__(kThreads, 4)
     }
 }
 
+// FP8 code export: the byte the F2FP conversion produces IS the deployable float8 value, so one 256-bit load becomes four
+// packed conversions and one 64-bit store; y (optional) is unpacked from the same bytes.  Same tiles and alignment rules as
+// the integer export.  Roofline: HBM, 5 B per element (+4 with y).
+template <int GRID, bool WANT_Y>
+__global__ void __launch_bounds__(kThreads, 4)
+    fq_fp8_codes_kernel(const float* __restrict__ x, float* __restrict__ y, uint8_t* __restrict__ codes, Tiles tiles,
+                        QPDev qpd) {
+    const int tid = threadIdx.x;
+    int64_t cur_channel = -1;
+    QP p;
+    uint32_t seed = 0;
+    constexpr int kCodeUnroll = 4;
+    for (uint32_t t = blockIdx.x; t < tiles.n_tiles; t += gridDim.x) {
+        const TileCursor<kThreads> c = tile_at<kThreads>(tiles, t);
+        if (c.channel != cur_channel) {
+            p = load_qp(qpd, c.channel);
+            seed = guard_seed(p.fast);
+            cur_channel = c.channel;
+        }
+        const int64_t off = c.offset;
+        int head = (int)((kVec - (off & (kVec - 1))) & (kVec - 1));
+        head = head < c.len ? head : c.len;
+        const int nvec = (c.len - head) / kVec;
+        const int tail0 = head + nvec * kVec;
+        const float* xb = x + off + head;
+        // ---- ragged head and tail: IEEE division, one element per thread
+        const int ragged = head + (c.len - tail0);
+        for (int k = tid; k < ragged; k += kThreads) {
+            const int64_t i = off + (k < head ? k : tail0 + (k - head));
+            const uint16_t pk = fp8_pack2<GRID>(clamp_t(div_ieee(ld_stream1(x + i), p.s), p), 0.0f);
+            codes[i] = (uint8_t)(pk & 0xffu);
+            if (WANT_Y) {
+                float q, unused;
+                fp8_unpack2<GRID>(pk, q, unused);
+                y[i] = dequant(q, p);
+            }
+        }
+        // ---- vector body
+        for (int v0 = tid; v0 < nvec; v0 += kThreads * kCodeUnroll) {
+            Vec<kVec> vin[kCodeUnroll];
+#pragma unroll
+            for (int j = 0; j < kCodeUnroll; ++j) {
+                const int v = v0 + j * kThreads;
+                if (v < nvec) vin[j] = ld_stream(xb + (int64_t)v * kVec, (Vec<kVec>*)nullptr);
+            }
+#pragma unroll
+            for (int j = 0; j < kCodeUnroll; ++j) {
+                const int v = v0 + j * kThreads;
+                if (v >= nvec) continue;
+                FastGuard guard;
+                guard_reset(guard, seed);
+                float tc[kVec];
+#pragma unroll
+                for (int e = 0; e < kVec; ++e) {
+                    guard_note(guard, vin[j].v[e]);
+                    tc[e] = clamp_t(div_fast(vin[j].v[e], p), p);
+                }
+                if (guard_bad(guard)) {
+#pragma unroll
+                    for (int e = 0; e < kVec; ++e) tc[e] = clamp_t(div_ieee(vin[j].v[e], p.s), p);
+                }
+                uint32_t w[2];
+                Vec<kVec> vy;
+#pragma unroll
+                for (int k = 0; k < kVec / 2; ++k) {
+                    const uint16_t pk = fp8_pack2<GRID>(tc[2 * k], tc[2 * k + 1]);
+                    if (k & 1)
+                        w[k >> 1] |= (uint32_t)pk << 16;
+                    else
+                        w[k >> 1] = pk;
+                    if (WANT_Y) {
+                        float q0, q1;
+                        fp8_unpack2<GRID>(pk, q0, q1);
+                        vy.v[2 * k] = dequant(q0, p);
+                        vy.v[2 * k + 1] = dequant(q1, p);
+                    }
+                }
+                const int64_t i = off + head + (int64_t)v * kVec;
+                *reinterpret_cast<uint2*>(codes + i) = make_uint2(w[0], w[1]);
+                if (WANT_Y) st_stream(y + i, vy);
+            }
+        }
+    }
+}
+
+// FP8 scale of each channel from an observer's chosen range: amax / F with amax = max(|lo|, |hi|); 1.0 when amax is zero
+// or not finite, so an all-zero channel stays exactly zero.  lo / hi are strided fp64 columns of the observer state.
+__global__ void fp8_scale_from_range_kernel(const double* lo, const double* hi, int64_t stride, int64_t channels, double F,
+                                            double* scale) {
+    const int64_t c = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (c >= channels) return;
+    const double a = fabs(lo[c * stride]), b = fabs(hi[c * stride]);
+    const double amax = b > a ? b : a;
+    scale[c] = (amax > 0.0 && amax <= 1.7976931348623157e308) ? amax / F : 1.0;
+}
+
 // LSQ backward.  Every tile emits one partial record {E, B} (fp32 inside a warp, fp64 across warps);
 // the records of a channel are then combined in a fixed order in fp64 and scaled by the grad-scale (reduce.cuh):
 //   * small launches (a single wave of CTAs): by the last CTA to finish, in the same launch;
@@ -232,7 +328,7 @@ struct LsqOut {
     }
 };
 
-template <int GROUP, int V, int MASK_MODE, bool WANT_DZ, bool RELU>
+template <int GROUP, int V, int MASK_MODE, bool WANT_DZ, bool RELU, int GRID = kGridInt>
 __global__ void __launch_bounds__(kThreads, 3)  // <= 85 registers: three CTAs per SM (the RELU variants drifted to 95-110)
     lsq_bwd_kernel(const float* __restrict__ x, const float* __restrict__ g, float* __restrict__ dx, Tiles tiles,
                    void* ws, LsqOut o, int64_t outer, int use_ticket) {
@@ -243,7 +339,7 @@ __global__ void __launch_bounds__(kThreads, 3)  // <= 85 registers: three CTAs p
     double* partials = ws_partials(ws);
     const bool leader = GROUP == 32 ? (threadIdx.x & 31) == 0 : threadIdx.x == 0;
 
-    LsqBwdOp<MASK_MODE, WANT_DZ, RELU> op;
+    LsqBwdOp<MASK_MODE, WANT_DZ, RELU, GRID> op;
     int64_t cur_channel = -1;
     for (uint32_t t = group_index<GROUP>(); t < tiles.n_tiles; t += group_count<GROUP>()) {
         const TileCursor<GROUP> c = tile_at<GROUP>(tiles, t);
@@ -266,7 +362,7 @@ __global__ void __launch_bounds__(kThreads, 3)  // <= 85 registers: three CTAs p
 // tiles from the look-ahead queue, carry the two sums in registers (fp32 per tile, fp64 across tiles) and flush ONCE.
 // Keeps the hardware-like balance of the per-tile grid without a block reduction per tile: mid-size activations
 // (2^22..2^26 elements) no longer pay for the reduction epilogue.
-template <int V, int MASK_MODE, bool WANT_DZ, bool RELU>
+template <int V, int MASK_MODE, bool WANT_DZ, bool RELU, int GRID = kGridInt>
 __global__ void __launch_bounds__(kThreads, 3)  // <= 85 registers: three CTAs per SM (the RELU variants drifted to 95-110)
     lsq_bwd_pt_kernel(const float* __restrict__ x, const float* __restrict__ g, float* __restrict__ dx, Tiles tiles,
                       void* ws, LsqOut o) {
@@ -276,7 +372,7 @@ __global__ void __launch_bounds__(kThreads, 3)  // <= 85 registers: three CTAs p
     float* const out[1] = {dx};
     double* partials = ws_partials(ws);
     unsigned int* counter = (unsigned int*)ws + 1;
-    LsqBwdOp<MASK_MODE, WANT_DZ, RELU> op;
+    LsqBwdOp<MASK_MODE, WANT_DZ, RELU, GRID> op;
     op.p = load_qp(o.qpd, 0);
     double e_run = 0.0, b_run = 0.0;
     TileQueue tq;
@@ -297,7 +393,7 @@ __global__ void __launch_bounds__(kThreads, 3)  // <= 85 registers: three CTAs p
 }
 
 // Per-channel LSQ backward on [outer, C, inner] with the channel-item schedule (see PcGeom): one flush per CTA.
-template <int GROUP, int V, bool WANT_DZ, bool RELU>
+template <int GROUP, int V, bool WANT_DZ, bool RELU, int GRID = kGridInt>
 __global__ void __launch_bounds__(kThreads, 3)  // <= 85 registers: three CTAs per SM (the RELU variants drifted to 95-110)
     lsq_bwd_pc_kernel(const float* __restrict__ x, const float* __restrict__ g, float* __restrict__ dx, PcGeom geo,
                       void* ws, LsqOut o, int use_ticket) {
@@ -309,7 +405,7 @@ __global__ void __launch_bounds__(kThreads, 3)  // <= 85 registers: three CTAs p
     const int warp = threadIdx.x >> 5;
     const uint32_t C = (uint32_t)geo.channels;
     const uint32_t c = blockIdx.x % C, j = blockIdx.x / C;
-    LsqBwdOp<VSIQ_MASK_ROUNDED, WANT_DZ, RELU> op;
+    LsqBwdOp<VSIQ_MASK_ROUNDED, WANT_DZ, RELU, GRID> op;
     op.p = load_qp(o.qpd, c);
     double e_run = 0.0, b_run = 0.0;
     const uint32_t first = GROUP == 32 ? j + (uint32_t)warp * geo.k : j;
@@ -356,6 +452,51 @@ static uint32_t ctas_for_tiles(uint32_t n_tiles) {
         }                                               \
     } while (0)
 
+// The launch bodies shared by the integer entry points and their FP8 siblings (GRID: common.cuh)
+template <int GRID>
+static int fq_fwd_launch(const float* x, float* y, const vsiq_layout* layout, const QPDev& qpd, bool relu,
+                         cudaStream_t st) {
+    const bool warp_group = layout->inner < kWarpGroupMaxInner;
+    const bool vec8 = aligned32(x) && aligned32(y);
+    Tiles tiles;
+#define CALL(G, V)                                                                          \
+    {                                                                                       \
+        if (!make_tiles<G>(layout->outer, layout->channels, layout->inner, &tiles))         \
+            return VSIQ_ERR_INVALID_ARG;                                                    \
+        int grid = launch_grid(ctas_for_tiles<G>(tiles.n_tiles));                           \
+        if (grid < 0) return -grid;                                                         \
+        if (relu)                                                                           \
+            fq_fwd_kernel<G, V, true, GRID><<<grid, kThreads, 0, st>>>(x, y, tiles, qpd);   \
+        else                                                                                \
+            fq_fwd_kernel<G, V, false, GRID><<<grid, kThreads, 0, st>>>(x, y, tiles, qpd);  \
+    }
+    VSIQ_DISPATCH_GROUP_VEC(warp_group, vec8, CALL);
+#undef CALL
+    return (int)cudaGetLastError();
+}
+
+template <int GRID>
+static int fq_bwd_ste_launch(const float* x, const float* g, float* dx, const vsiq_layout* layout, const QPDev& qpd,
+                             bool relu, cudaStream_t st) {
+    const bool warp_group = layout->inner < kWarpGroupMaxInner;
+    const bool vec8 = aligned32(x) && aligned32(g) && aligned32(dx);
+    Tiles tiles;
+#define CALL(G, V)                                                                                  \
+    {                                                                                               \
+        if (!make_tiles<G>(layout->outer, layout->channels, layout->inner, &tiles))                 \
+            return VSIQ_ERR_INVALID_ARG;                                                            \
+        int grid = launch_grid(ctas_for_tiles<G>(tiles.n_tiles));                                   \
+        if (grid < 0) return -grid;                                                                 \
+        if (relu)                                                                                   \
+            fq_bwd_ste_kernel<G, V, true, GRID><<<grid, kThreads, 0, st>>>(x, g, dx, tiles, qpd);   \
+        else                                                                                        \
+            fq_bwd_ste_kernel<G, V, false, GRID><<<grid, kThreads, 0, st>>>(x, g, dx, tiles, qpd);  \
+    }
+    VSIQ_DISPATCH_GROUP_VEC(warp_group, vec8, CALL);
+#undef CALL
+    return (int)cudaGetLastError();
+}
+
 }  // namespace vsiq
 
 using namespace vsiq;
@@ -372,23 +513,7 @@ extern "C" int vsiq_fake_quant_fwd(const float* x, float* y, void* codes, const 
     if (qp->pre_op == VSIQ_PRE_SILU) return VSIQ_ERR_UNSUPPORTED;  // SiLU: channel-innermost entry points only
     if (codes)  // int8 (qmin < 0) / uint8 codes: the 8-bit form of vsiq_quantize_codes
         return vsiq_quantize_codes(x, y, codes, 8, layout, qp, stream);
-    const bool warp_group = layout->inner < kWarpGroupMaxInner;
-    const bool vec8 = aligned32(x) && aligned32(y);
-    Tiles tiles;
-#define CALL(G, V)                                                                          \
-    {                                                                                       \
-        if (!make_tiles<G>(layout->outer, layout->channels, layout->inner, &tiles))         \
-            return VSIQ_ERR_INVALID_ARG;                                                    \
-        int grid = launch_grid(ctas_for_tiles<G>(tiles.n_tiles));   \
-        if (grid < 0) return -grid;                                                         \
-        if (qp->pre_op == VSIQ_PRE_RELU)                                                    \
-            fq_fwd_kernel<G, V, true><<<grid, kThreads, 0, st>>>(x, y, tiles, qpd);         \
-        else                                                                                \
-            fq_fwd_kernel<G, V, false><<<grid, kThreads, 0, st>>>(x, y, tiles, qpd);        \
-    }
-    VSIQ_DISPATCH_GROUP_VEC(warp_group, vec8, CALL);
-#undef CALL
-    return (int)cudaGetLastError();
+    return fq_fwd_launch<kGridInt>(x, y, layout, qpd, qp->pre_op == VSIQ_PRE_RELU, st);
 }
 
 extern "C" int vsiq_quantize_codes(const float* x, float* y, void* codes, int code_bits, const vsiq_layout* layout,
@@ -433,24 +558,7 @@ extern "C" int vsiq_fake_quant_bwd_ste(const float* x, const float* g, float* dx
     if (qp->pre_op == VSIQ_PRE_SILU) return VSIQ_ERR_UNSUPPORTED;
     if (layout->outer * layout->channels * layout->inner == 0) return VSIQ_OK;
     if (!x || !g || !dx) return VSIQ_ERR_INVALID_ARG;
-    cudaStream_t st = (cudaStream_t)stream;
-    const bool warp_group = layout->inner < kWarpGroupMaxInner;
-    const bool vec8 = aligned32(x) && aligned32(g) && aligned32(dx);
-    Tiles tiles;
-#define CALL(G, V)                                                                            \
-    {                                                                                         \
-        if (!make_tiles<G>(layout->outer, layout->channels, layout->inner, &tiles))           \
-            return VSIQ_ERR_INVALID_ARG;                                                      \
-        int grid = launch_grid(ctas_for_tiles<G>(tiles.n_tiles)); \
-        if (grid < 0) return -grid;                                                           \
-        if (qp->pre_op == VSIQ_PRE_RELU)                                                      \
-            fq_bwd_ste_kernel<G, V, true><<<grid, kThreads, 0, st>>>(x, g, dx, tiles, qpd);   \
-        else                                                                                  \
-            fq_bwd_ste_kernel<G, V, false><<<grid, kThreads, 0, st>>>(x, g, dx, tiles, qpd);  \
-    }
-    VSIQ_DISPATCH_GROUP_VEC(warp_group, vec8, CALL);
-#undef CALL
-    return (int)cudaGetLastError();
+    return fq_bwd_ste_launch<kGridInt>(x, g, dx, layout, qpd, qp->pre_op == VSIQ_PRE_RELU, (cudaStream_t)stream);
 }
 
 extern "C" int vsiq_fake_quant_fwd_bwd(const float* x, const float* g, float* y, float* dx,
@@ -482,10 +590,15 @@ extern "C" size_t vsiq_lsq_bwd_workspace_bytes(const vsiq_layout* layout) {
     return reduce_workspace_bytes(layout, LsqRec::kSlot);
 }
 
-extern "C" int vsiq_lsq_bwd(const float* x, const float* g, float* dx, void* dscale, int dscale_dtype, void* dzp,
-                            int dzp_dtype, const vsiq_layout* layout, const vsiq_qparams* qp, double grad_scale_host,
-                            const float* grad_scale_dev, int mask_mode, void* workspace, size_t workspace_bytes,
-                            vsiq_stream_t stream) {
+// vsiq_lsq_bwd for the integer grid, vsiq_fp8_lsq_bwd for the FP8 ones (which has already refused FunLSQ and dzp: the
+// FunLSQ / dzp instantiations below collapse onto the rounded, dzp-free one for them and are never reached)
+template <int GRID>
+static int lsq_bwd_impl(const float* x, const float* g, float* dx, void* dscale, int dscale_dtype, void* dzp,
+                        int dzp_dtype, const vsiq_layout* layout, const vsiq_qparams* qp, double grad_scale_host,
+                        const float* grad_scale_dev, int mask_mode, void* workspace, size_t workspace_bytes,
+                        vsiq_stream_t stream) {
+    constexpr int kFunlsq = GRID == kGridInt ? VSIQ_MASK_FUNLSQ : VSIQ_MASK_ROUNDED;
+    constexpr bool kDz = GRID == kGridInt;
     if (!dscale) return VSIQ_ERR_INVALID_ARG;
     if (int e = check_layout(layout)) return e;
     if (mask_mode != VSIQ_MASK_ROUNDED && mask_mode != VSIQ_MASK_FUNLSQ) return VSIQ_ERR_INVALID_ARG;
@@ -493,7 +606,7 @@ extern "C" int vsiq_lsq_bwd(const float* x, const float* g, float* dx, void* dsc
     if ((dscale_dtype != VSIQ_F32 && dscale_dtype != VSIQ_F64) || (dzp && dzp_dtype != VSIQ_F32 && dzp_dtype != VSIQ_F64))
         return VSIQ_ERR_INVALID_ARG;
     LsqOut lo;
-    if (int e = fill_qp(qp, &lo.qpd)) return e;
+    if (int e = GRID == kGridInt ? fill_qp(qp, &lo.qpd) : fill_qp_fp8(qp, GRID, &lo.qpd)) return e;
     if (qp->pre_op == VSIQ_PRE_SILU) return VSIQ_ERR_UNSUPPORTED;
     if (!workspace || workspace_bytes < vsiq_lsq_bwd_workspace_bytes(layout)) return VSIQ_ERR_WORKSPACE;
     cudaStream_t st = (cudaStream_t)stream;
@@ -523,9 +636,9 @@ extern "C" int vsiq_lsq_bwd(const float* x, const float* g, float* dx, void* dsc
         const int grid = (int)(pc.channels * pc.k);
         // one partial wave: the last CTA combines; more: no ticket, no fence -- the combine kernel is a programmatic dependent
         const int use_ticket = grid <= dprops.sm_count * 4 ? 1 : 0;
-#define PC(G, V, Z, R) lsq_bwd_pc_kernel<G, V, Z, R><<<grid, kThreads, 0, st>>>(x, g, dx, pc, workspace, lo, use_ticket)
+#define PC(G, V, Z, R) lsq_bwd_pc_kernel<G, V, Z, R, GRID><<<grid, kThreads, 0, st>>>(x, g, dx, pc, workspace, lo, use_ticket)
 #define PC2(G, V, Z) { if (relu) PC(G, V, Z, true); else PC(G, V, Z, false); }
-#define PC1(G, V) { if (dzp) PC2(G, V, true) else PC2(G, V, false) }
+#define PC1(G, V) { if (dzp) PC2(G, V, kDz) else PC2(G, V, false) }
         if (warp_group) { if (vec8) PC1(32, 8) else PC1(32, 1) } else { if (vec8) PC1(kThreads, 8) else PC1(kThreads, 1) }
 #undef PC1
 #undef PC2
@@ -538,9 +651,9 @@ extern "C" int vsiq_lsq_bwd(const float* x, const float* g, float* dx, void* dsc
         if (!make_tiles<kThreads>(1, 1, layout->inner, &tiles)) return VSIQ_ERR_INVALID_ARG;
         const uint32_t cap = (uint32_t)dprops.sm_count * 3u;
         const int grid = (int)(tiles.n_tiles < cap ? tiles.n_tiles : cap);
-#define PT(V, M, Z, R) lsq_bwd_pt_kernel<V, M, Z, R><<<grid, kThreads, 0, st>>>(x, g, dx, tiles, workspace, lo)
+#define PT(V, M, Z, R) lsq_bwd_pt_kernel<V, M, Z, R, GRID><<<grid, kThreads, 0, st>>>(x, g, dx, tiles, workspace, lo)
 #define PT2(V, M, Z) { if (relu) PT(V, M, Z, true); else PT(V, M, Z, false); }
-#define PT1(V) { if (mask_mode == VSIQ_MASK_FUNLSQ) PT(V, VSIQ_MASK_FUNLSQ, false, false); else if (dzp) PT2(V, VSIQ_MASK_ROUNDED, true) else PT2(V, VSIQ_MASK_ROUNDED, false) }
+#define PT1(V) { if (mask_mode == VSIQ_MASK_FUNLSQ) PT(V, kFunlsq, false, false); else if (dzp) PT2(V, VSIQ_MASK_ROUNDED, kDz) else PT2(V, VSIQ_MASK_ROUNDED, false) }
         if (vec8) PT1(8) else PT1(1)
 #undef PT1
 #undef PT2
@@ -563,16 +676,16 @@ extern "C" int vsiq_lsq_bwd(const float* x, const float* g, float* dx, void* dsc
         int grid = launch_grid(ctas_for_tiles<G>(tiles.n_tiles));                                              \
         if (grid < 0) return -grid;                                                                            \
         const int use_ticket = (grid <= dprops.sm_count * 4 && tiles.n_tiles <= kTicketMaxRecords) ? 1 : 0;   \
-        lsq_bwd_kernel<G, V, M, Z, R><<<grid, kThreads, 0, st>>>(x, g, dx, tiles, workspace, lo, layout->outer, \
-                                                              use_ticket);                                     \
+        lsq_bwd_kernel<G, V, M, Z, R, GRID><<<grid, kThreads, 0, st>>>(x, g, dx, tiles, workspace, lo,        \
+                                                                    layout->outer, use_ticket);                                     \
         if (!use_ticket) launch_finalize<LsqRec>(tiles, layout->outer, true, workspace, lo, st);               \
     }
 #define CALL(G, V)                                   \
     {                                                \
         if (mask_mode == VSIQ_MASK_FUNLSQ) {         \
-            LAUNCH(G, V, VSIQ_MASK_FUNLSQ, false);   \
+            LAUNCH(G, V, kFunlsq, false);            \
         } else if (dzp) {                            \
-            LAUNCH(G, V, VSIQ_MASK_ROUNDED, true);   \
+            LAUNCH(G, V, VSIQ_MASK_ROUNDED, kDz);    \
         } else {                                     \
             LAUNCH(G, V, VSIQ_MASK_ROUNDED, false);  \
         }                                            \
@@ -581,6 +694,89 @@ extern "C" int vsiq_lsq_bwd(const float* x, const float* g, float* dx, void* dsc
 #undef CALL
 #undef LAUNCH
 #undef LAUNCH_R
+    return (int)cudaGetLastError();
+}
+
+extern "C" int vsiq_lsq_bwd(const float* x, const float* g, float* dx, void* dscale, int dscale_dtype, void* dzp,
+                            int dzp_dtype, const vsiq_layout* layout, const vsiq_qparams* qp, double grad_scale_host,
+                            const float* grad_scale_dev, int mask_mode, void* workspace, size_t workspace_bytes,
+                            vsiq_stream_t stream) {
+    return lsq_bwd_impl<kGridInt>(x, g, dx, dscale, dscale_dtype, dzp, dzp_dtype, layout, qp, grad_scale_host,
+                                  grad_scale_dev, mask_mode, workspace, workspace_bytes, stream);
+}
+
+// ------------------------------------------------------------------------------------ FP8 entry points
+extern "C" int vsiq_fp8_fake_quant_fwd(const float* x, float* y, void* codes, const vsiq_layout* layout,
+                                       const vsiq_qparams* qp, int fp8_format, vsiq_stream_t stream) {
+    if (int e = check_layout(layout)) return e;
+    QPDev qpd;
+    if (int e = fill_qp_fp8(qp, fp8_format, &qpd)) return e;
+    if (qp->pre_op == VSIQ_PRE_SILU) return VSIQ_ERR_UNSUPPORTED;
+    const int64_t n = layout->outer * layout->channels * layout->inner;
+    if (n == 0) return VSIQ_OK;
+    if (!x || (!y && !codes)) return VSIQ_ERR_INVALID_ARG;
+    cudaStream_t st = (cudaStream_t)stream;
+    if (!codes) {
+        const bool relu = qp->pre_op == VSIQ_PRE_RELU;
+        return fp8_format == VSIQ_FP8_E4M3 ? fq_fwd_launch<VSIQ_FP8_E4M3>(x, y, layout, qpd, relu, st)
+                                           : fq_fwd_launch<VSIQ_FP8_E5M2>(x, y, layout, qpd, relu, st);
+    }
+    if (qp->pre_op != VSIQ_PRE_NONE) return VSIQ_ERR_UNSUPPORTED;
+    const uintptr_t amask = reinterpret_cast<uintptr_t>(x) | (y ? reinterpret_cast<uintptr_t>(y) : 0);
+    if ((amask & 31u) || (reinterpret_cast<uintptr_t>(codes) & 15u)) return VSIQ_ERR_UNSUPPORTED;
+    Tiles tiles;
+    const int mult = reduce_tile_mult<kThreads>(layout->outer, layout->channels, layout->inner);
+    if (!make_tiles<kThreads>(layout->outer, layout->channels, layout->inner, &tiles, mult)) return VSIQ_ERR_INVALID_ARG;
+    const int grid = launch_grid(tiles.n_tiles);
+    if (grid < 0) return -grid;
+    uint8_t* c8 = (uint8_t*)codes;
+#define C(F)                                                                                       \
+    {                                                                                              \
+        if (y) fq_fp8_codes_kernel<F, true><<<grid, kThreads, 0, st>>>(x, y, c8, tiles, qpd);      \
+        else fq_fp8_codes_kernel<F, false><<<grid, kThreads, 0, st>>>(x, y, c8, tiles, qpd);       \
+    }
+    if (fp8_format == VSIQ_FP8_E4M3) C(VSIQ_FP8_E4M3) else C(VSIQ_FP8_E5M2)
+#undef C
+    return (int)cudaGetLastError();
+}
+
+extern "C" int vsiq_fp8_fake_quant_bwd_ste(const float* x, const float* g, float* dx, const vsiq_layout* layout,
+                                           const vsiq_qparams* qp, int fp8_format, vsiq_stream_t stream) {
+    if (int e = check_layout(layout)) return e;
+    QPDev qpd;
+    if (int e = fill_qp_fp8(qp, fp8_format, &qpd)) return e;
+    if (qp->pre_op == VSIQ_PRE_SILU) return VSIQ_ERR_UNSUPPORTED;
+    if (layout->outer * layout->channels * layout->inner == 0) return VSIQ_OK;
+    if (!x || !g || !dx) return VSIQ_ERR_INVALID_ARG;
+    const bool relu = qp->pre_op == VSIQ_PRE_RELU;
+    cudaStream_t st = (cudaStream_t)stream;
+    return fp8_format == VSIQ_FP8_E4M3 ? fq_bwd_ste_launch<VSIQ_FP8_E4M3>(x, g, dx, layout, qpd, relu, st)
+                                       : fq_bwd_ste_launch<VSIQ_FP8_E5M2>(x, g, dx, layout, qpd, relu, st);
+}
+
+extern "C" int vsiq_fp8_lsq_bwd(const float* x, const float* g, float* dx, void* dscale, int dscale_dtype, void* dzp,
+                                int dzp_dtype, const vsiq_layout* layout, const vsiq_qparams* qp, int fp8_format,
+                                double grad_scale_host, const float* grad_scale_dev, int mask_mode, void* workspace,
+                                size_t workspace_bytes, vsiq_stream_t stream) {
+    if (fp8_format != VSIQ_FP8_E4M3 && fp8_format != VSIQ_FP8_E5M2) return VSIQ_ERR_INVALID_ARG;
+    if (mask_mode != VSIQ_MASK_ROUNDED && mask_mode != VSIQ_MASK_FUNLSQ) return VSIQ_ERR_INVALID_ARG;
+    if (mask_mode != VSIQ_MASK_ROUNDED || dzp) return VSIQ_ERR_UNSUPPORTED;  // symmetric, autograd-mask semantics only
+    return fp8_format == VSIQ_FP8_E4M3
+               ? lsq_bwd_impl<VSIQ_FP8_E4M3>(x, g, dx, dscale, dscale_dtype, nullptr, dzp_dtype, layout, qp,
+                                             grad_scale_host, grad_scale_dev, mask_mode, workspace, workspace_bytes, stream)
+               : lsq_bwd_impl<VSIQ_FP8_E5M2>(x, g, dx, dscale, dscale_dtype, nullptr, dzp_dtype, layout, qp,
+                                             grad_scale_host, grad_scale_dev, mask_mode, workspace, workspace_bytes, stream);
+}
+
+extern "C" int vsiq_fp8_scale_from_range(const double* lo, const double* hi, int64_t stride, int64_t channels,
+                                         int fp8_format, double* scale, vsiq_stream_t stream) {
+    if (fp8_format != VSIQ_FP8_E4M3 && fp8_format != VSIQ_FP8_E5M2) return VSIQ_ERR_INVALID_ARG;
+    if (channels < 0 || stride < 1) return VSIQ_ERR_INVALID_ARG;
+    if (channels == 0) return VSIQ_OK;
+    if (!lo || !hi || !scale) return VSIQ_ERR_INVALID_ARG;
+    const int threads = 128;
+    fp8_scale_from_range_kernel<<<(unsigned)((channels + threads - 1) / threads), threads, 0, (cudaStream_t)stream>>>(
+        lo, hi, stride, channels, (double)fp8_max(fp8_format), scale);
     return (int)cudaGetLastError();
 }
 

@@ -21,30 +21,31 @@ struct QuantOpBase : OpBase {
 template <bool RELU>
 __device__ __forceinline__ float pre_act(float x) { return RELU ? max_nan(x, 0.0f) : x; }
 
-template <bool RELU>
+// GRID (common.cuh): kGridInt, or an FP8 grid (no zero-point; dequant's q - 0 is exact, -0.0 and NaN included)
+template <bool RELU, int GRID = kGridInt>
 struct FwdOp : QuantOpBase {
     __device__ __forceinline__ void apply(const float (&a)[1], float (&o)[1]) {
         const float x = pre_act<RELU>(a[0]);
         guard_note(guard, x);
-        o[0] = dequant(elem_fast(x, p).q, p);
+        o[0] = dequant(elem_fast<GRID>(x, p).q, p);
     }
     __device__ __forceinline__ void apply_slow(const float (&a)[1], float (&o)[1]) {
-        o[0] = dequant(elem_slow(pre_act<RELU>(a[0]), p).q, p);
+        o[0] = dequant(elem_slow<GRID>(pre_act<RELU>(a[0]), p).q, p);
     }
 };
 
-template <bool RELU>
+template <bool RELU, int GRID = kGridInt>
 struct SteBwdOp : QuantOpBase {
     __device__ __forceinline__ void apply(const float (&a)[2], float (&o)[1]) {
         const float x = pre_act<RELU>(a[0]);
         guard_note(guard, x);
         guard_note(guard, a[1]);
-        const Elem e = elem_fast(x, p);
+        const Elem e = elem_fast<GRID>(x, p);
         const float dx = dx_fast(a[1], e.m, p);
         o[0] = (!RELU || a[0] > 0.0f) ? dx : 0.0f;
     }
     __device__ __forceinline__ void apply_slow(const float (&a)[2], float (&o)[1]) {
-        const float dx = dx_slow(a[1], elem_slow(pre_act<RELU>(a[0]), p).m, p);
+        const float dx = dx_slow(a[1], elem_slow<GRID>(pre_act<RELU>(a[0]), p).m, p);
         o[0] = (!RELU || a[0] > 0.0f) ? dx : 0.0f;
     }
 };
@@ -64,7 +65,8 @@ struct FwdBwdOp : QuantOpBase {
     }
 };
 
-template <int MASK_MODE, bool WANT_DZ, bool RELU>
+// FP8 grids: MASK_MODE = VSIQ_MASK_ROUNDED and WANT_DZ = false only (z = 0, so the sum is g * (q - m * x/s))
+template <int MASK_MODE, bool WANT_DZ, bool RELU, int GRID = kGridInt>
 struct LsqBwdOp : QuantOpBase {
     float e_acc;  // sum g * ((q - z) - m * x/s)   over this thread's elements of the current tile
     float b_acc;  // sum g over clamped-out elements
@@ -100,13 +102,13 @@ struct LsqBwdOp : QuantOpBase {
         const float x = pre_act<RELU>(a[0]);
         guard_note(guard, x);
         guard_note(guard, a[1]);
-        const Elem e = elem_fast(x, p);
+        const Elem e = elem_fast<GRID>(x, p);
         if (MASK_MODE == VSIQ_MASK_ROUNDED) o[0] = dx_fast(a[1], e.m, p);
         accumulate(a[1], e, o);
         if (RELU) o[0] = a[0] > 0.0f ? o[0] : 0.0f;
     }
     __device__ __forceinline__ void apply_slow(const float (&a)[2], float (&o)[1]) {
-        const Elem e = elem_slow(pre_act<RELU>(a[0]), p);
+        const Elem e = elem_slow<GRID>(pre_act<RELU>(a[0]), p);
         if (MASK_MODE == VSIQ_MASK_ROUNDED) o[0] = dx_slow(a[1], e.m, p);
         accumulate(a[1], e, o);
         if (RELU) o[0] = a[0] > 0.0f ? o[0] : 0.0f;

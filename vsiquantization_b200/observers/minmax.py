@@ -198,6 +198,12 @@ class MinMaxObserver(BaseObserver):
         st = self._state
         return st[:, 2], st[:, 3]
 
+    def device_range(self):
+        """(lo, hi) views of the device state (fp64): the range this observer chose -- the running extrema here.  The
+        FP8 quantisers derive their scale from it (QuantizationManager)."""
+        st = self._state
+        return st[:, 0], st[:, 1]
+
     # -- data-parallel merge (parallel.sync_observers) ------------------------------------------------
     def sync_key(self) -> tuple:
         """Observers with equal keys are merged together: their states are concatenated into one merge_states arena."""

@@ -69,6 +69,11 @@ class HistogramObserver(MinMaxObserver):
     def recompute_clip(self) -> None:
         raise NotImplementedError
 
+    def device_range(self):
+        """(lo, hi) views of the device state (fp64): the clipped range (columns 8, 9)."""
+        st = self._state
+        return st[:, 8], st[:, 9]
+
     def sync_key(self) -> tuple:
         return ("percentile", self.n_bins)
 

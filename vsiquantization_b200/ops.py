@@ -169,11 +169,12 @@ class QSpec:
     mask_mode: int = _lib.MASK_ROUNDED
     pre_relu: bool = False  # quantise relu(x); the backward also applies relu's mask (one pass instead of two)
     pre_silu: bool = False  # quantise silu(x) (ATen-CUDA's op order); channels_last tensors only (ci_forward / ci_backward)
+    fp8_format: int = 0     # 0: the integer grid [qmin, qmax]; _lib.FP8_E4M3 / FP8_E5M2: that FP8 grid (qmin = qmax = 0)
 
 
 def _make_qparams(spec: QSpec, scale, zero_point, channels: int, device: torch.device, keep: list) -> QParams:
     qp = QParams()
-    qp.qmin, qp.qmax = int(spec.qmin), int(spec.qmax)
+    qp.qmin, qp.qmax = (0, 0) if spec.fp8_format else (int(spec.qmin), int(spec.qmax))
     qp.zp_learned = 1 if spec.zp_learned else 0
     qp.pre_op = _lib.PRE_SILU if spec.pre_silu else (_lib.PRE_RELU if spec.pre_relu else _lib.PRE_NONE)
     qp.scale_dtype = qp.zp_dtype = F32
@@ -207,7 +208,7 @@ def _make_qparams(spec: QSpec, scale, zero_point, channels: int, device: torch.d
     else:
         qp.zero_point = None
         qp.zp_host = float(zero_point)
-        if channels != 1 and isinstance(scale, torch.Tensor):
+        if channels != 1 and isinstance(scale, torch.Tensor) and not spec.fp8_format:
             # scalar zero-point with per-channel scales: broadcast it
             z = torch.full((channels,), float(zero_point), dtype=torch.float32, device=device)
             keep.append(z)
@@ -248,6 +249,8 @@ def quantize_codes(x: torch.Tensor, scale, zero_point, spec: QSpec, code_bits: O
     dimension, two codes per byte (element 2k in the low nibble, two's complement when qmin < 0)."""
     if spec.pre_relu or spec.pre_silu:
         raise ValueError("code export has no fused activation")
+    if spec.fp8_format:
+        return _fp8_codes(x, scale, spec, want_y, codes_out)
     x = _dense_for(x, "x", spec.ch_axis)
     if not x.is_contiguous():
         x = x.contiguous()  # codes are laid out in logical (row-major) order
@@ -281,6 +284,38 @@ def quantize_codes(x: torch.Tensor, scale, zero_point, spec: QSpec, code_bits: O
     return y, codes
 
 
+_FP8_DTYPES = {_lib.FP8_E4M3: torch.float8_e4m3fn, _lib.FP8_E5M2: torch.float8_e5m2}
+
+
+def _fp8_codes(x, scale, spec: QSpec, want_y: bool, codes_out: Optional[torch.Tensor]):
+    """(y or None, FP8 codes): codes is a float8_e4m3fn / float8_e5m2 tensor shaped like x holding
+    (x / s).clamp(-F, F) rounded to that format -- the deployable weights (vsiq_fp8_fake_quant_fwd with codes)."""
+    x = _dense_for(x, "x", spec.ch_axis)
+    if not x.is_contiguous():
+        x = x.contiguous()  # codes are laid out in logical (row-major) order
+    if x.data_ptr() % 32:
+        x = x.clone()
+    outer, C, inner = layout_of(x.shape, spec.ch_axis)
+    lay = Layout(outer, C, inner)
+    dt = _FP8_DTYPES[spec.fp8_format]
+    keep: list = []
+    with torch.cuda.device(x.device):
+        qp = _make_qparams(spec, scale, 0, max(C, 1), x.device, keep)
+        y = torch.empty_like(x) if want_y else None
+        if codes_out is not None:
+            if tuple(codes_out.shape) != tuple(x.shape) or codes_out.dtype != dt or codes_out.device != x.device \
+                    or not codes_out.is_contiguous():
+                raise ValueError(f"codes_out must be a contiguous {dt} tensor of shape {tuple(x.shape)} on {x.device}")
+            codes = codes_out
+        else:
+            codes = torch.empty(x.shape, dtype=dt, device=x.device)
+        check(lib.vsiq_fp8_fake_quant_fwd(x.data_ptr(), y.data_ptr() if want_y else None, codes.data_ptr(),
+                                          ctypes.byref(lay), ctypes.byref(qp), int(spec.fp8_format), _stream_ptr()),
+              "vsiq_fp8_fake_quant_fwd")
+        _count_launch()
+    return y, codes
+
+
 def fake_quant_forward(x: torch.Tensor, scale, zero_point, spec: QSpec, want_codes: bool = False,
                        out: Optional[torch.Tensor] = None):
     """y = (clamp(rint(x/s + z), qmin, qmax) - z) * s  [reference: quantizers/uniform.py:54-55,95].
@@ -299,8 +334,12 @@ def fake_quant_forward(x: torch.Tensor, scale, zero_point, spec: QSpec, want_cod
         qp = _make_qparams(spec, scale, zero_point, max(C, 1), x.device, keep)
         y = _out_like(x, out, "out")
         _note_alignment(x, y)
-        check(lib.vsiq_fake_quant_fwd(x.data_ptr(), y.data_ptr(), None, ctypes.byref(lay), ctypes.byref(qp), _stream_ptr()),
-              "vsiq_fake_quant_fwd")
+        if spec.fp8_format:
+            check(lib.vsiq_fp8_fake_quant_fwd(x.data_ptr(), y.data_ptr(), None, ctypes.byref(lay), ctypes.byref(qp),
+                                              int(spec.fp8_format), _stream_ptr()), "vsiq_fp8_fake_quant_fwd")
+        else:
+            check(lib.vsiq_fake_quant_fwd(x.data_ptr(), y.data_ptr(), None, ctypes.byref(lay), ctypes.byref(qp),
+                                          _stream_ptr()), "vsiq_fake_quant_fwd")
         _count_launch()
     return y
 
@@ -319,8 +358,13 @@ def fake_quant_backward_ste(x: torch.Tensor, g: torch.Tensor, scale, zero_point,
         qp = _make_qparams(spec, scale, zero_point, C, x.device, keep)
         dx = _out_like(x, out, "out")
         _note_alignment(x, g, dx)
-        check(lib.vsiq_fake_quant_bwd_ste(x.data_ptr(), g.data_ptr(), dx.data_ptr(), ctypes.byref(lay),
-                                          ctypes.byref(qp), _stream_ptr()), "vsiq_fake_quant_bwd_ste")
+        if spec.fp8_format:
+            check(lib.vsiq_fp8_fake_quant_bwd_ste(x.data_ptr(), g.data_ptr(), dx.data_ptr(), ctypes.byref(lay),
+                                                  ctypes.byref(qp), int(spec.fp8_format), _stream_ptr()),
+                  "vsiq_fp8_fake_quant_bwd_ste")
+        else:
+            check(lib.vsiq_fake_quant_bwd_ste(x.data_ptr(), g.data_ptr(), dx.data_ptr(), ctypes.byref(lay),
+                                              ctypes.byref(qp), _stream_ptr()), "vsiq_fake_quant_bwd_ste")
         _count_launch()
     return dx
 
@@ -372,11 +416,18 @@ def lsq_backward(x, g, scale, zero_point, spec: QSpec, grad_scale: float, grad_s
         if grad_scale_dev is not None:
             gsd = grad_scale_dev.detach().to(device=x.device, dtype=torch.float32).contiguous()
             keep.append(gsd)
-        check(lib.vsiq_lsq_bwd(x.data_ptr(), g.data_ptr(), dx.data_ptr(), ds.data_ptr(), _dtype_code(ds),
-                               dz.data_ptr() if dz is not None else None, _dtype_code(dz) if dz is not None else F32,
-                               ctypes.byref(lay), ctypes.byref(qp), float(grad_scale),
-                               gsd.data_ptr() if gsd is not None else None, int(spec.mask_mode), ws.data_ptr(),
-                               ws.numel(), _stream_ptr()), "vsiq_lsq_bwd")
+        if spec.fp8_format:
+            check(lib.vsiq_fp8_lsq_bwd(x.data_ptr(), g.data_ptr(), dx.data_ptr(), ds.data_ptr(), _dtype_code(ds),
+                                       dz.data_ptr() if dz is not None else None, _dtype_code(dz) if dz is not None else F32,
+                                       ctypes.byref(lay), ctypes.byref(qp), int(spec.fp8_format), float(grad_scale),
+                                       gsd.data_ptr() if gsd is not None else None, int(spec.mask_mode), ws.data_ptr(),
+                                       ws.numel(), _stream_ptr()), "vsiq_fp8_lsq_bwd")
+        else:
+            check(lib.vsiq_lsq_bwd(x.data_ptr(), g.data_ptr(), dx.data_ptr(), ds.data_ptr(), _dtype_code(ds),
+                                   dz.data_ptr() if dz is not None else None, _dtype_code(dz) if dz is not None else F32,
+                                   ctypes.byref(lay), ctypes.byref(qp), float(grad_scale),
+                                   gsd.data_ptr() if gsd is not None else None, int(spec.mask_mode), ws.data_ptr(),
+                                   ws.numel(), _stream_ptr()), "vsiq_lsq_bwd")
         _count_launch()
     return dx, ds, dz
 
@@ -417,6 +468,8 @@ def ci_forward(x: torch.Tensor, bias: Optional[torch.Tensor], scale, zero_point,
         ws = _workspace(lib.vsiq_ci_workspace_bytes(rows, C), x.device)
         if second is not None:
             s2, z2, spec2 = second
+            if spec.fp8_format or spec2.fp8_format:
+                raise ValueError("the two-output epilogue has integer grids only")
             if spec2.pre_relu or spec2.pre_silu:
                 raise ValueError("the second quantiser of a two-output pass has no activation of its own")
             qp2, qpc2 = _ci_qparams(spec2, s2, z2, C, x.device, keep)
@@ -426,9 +479,14 @@ def ci_forward(x: torch.Tensor, bias: Optional[torch.Tensor], scale, zero_point,
                                               ws.data_ptr(), ws.numel(), _stream_ptr()), "vsiq_ci_fake_quant_fwd2")
             _count_launch()
             return y, y2
-        check(lib.vsiq_ci_fake_quant_fwd(x.data_ptr(), b.data_ptr() if b is not None else None, y.data_ptr(), rows, C,
-                                         ctypes.byref(qp), qpc, ws.data_ptr(), ws.numel(), _stream_ptr()),
-              "vsiq_ci_fake_quant_fwd")
+        if spec.fp8_format:
+            check(lib.vsiq_ci_fp8_fake_quant_fwd(x.data_ptr(), b.data_ptr() if b is not None else None, y.data_ptr(), rows,
+                                                 C, ctypes.byref(qp), qpc, int(spec.fp8_format), ws.data_ptr(), ws.numel(),
+                                                 _stream_ptr()), "vsiq_ci_fp8_fake_quant_fwd")
+        else:
+            check(lib.vsiq_ci_fake_quant_fwd(x.data_ptr(), b.data_ptr() if b is not None else None, y.data_ptr(), rows,
+                                             C, ctypes.byref(qp), qpc, ws.data_ptr(), ws.numel(), _stream_ptr()),
+                  "vsiq_ci_fake_quant_fwd")
         _count_launch()
     return y
 
@@ -464,12 +522,16 @@ def ci_backward(x: torch.Tensor, bias: Optional[torch.Tensor], g: torch.Tensor, 
             gsd = grad_scale_dev.detach().to(device=x.device, dtype=torch.float32).contiguous()
             keep.append(gsd)
         ws = _workspace(lib.vsiq_ci_workspace_bytes(rows, C), x.device)
-        check(lib.vsiq_ci_lsq_bwd(x.data_ptr(), b.data_ptr() if b is not None else None, g.data_ptr(), dx.data_ptr(),
-                                  ds.data_ptr() if ds is not None else None, _dtype_code(ds) if ds is not None else F32,
-                                  dz.data_ptr() if dz is not None else None, _dtype_code(dz) if dz is not None else F32,
-                                  db.data_ptr() if db is not None else None, rows, C, ctypes.byref(qp), qpc,
-                                  float(grad_scale), gsd.data_ptr() if gsd is not None else None, pitch, ws.data_ptr(),
-                                  ws.numel(), _stream_ptr()), "vsiq_ci_lsq_bwd")
+        bwd_args = (x.data_ptr(), b.data_ptr() if b is not None else None, g.data_ptr(), dx.data_ptr(),
+                    ds.data_ptr() if ds is not None else None, _dtype_code(ds) if ds is not None else F32,
+                    dz.data_ptr() if dz is not None else None, _dtype_code(dz) if dz is not None else F32,
+                    db.data_ptr() if db is not None else None, rows, C, ctypes.byref(qp), qpc)
+        tail = (float(grad_scale), gsd.data_ptr() if gsd is not None else None, pitch, ws.data_ptr(), ws.numel(),
+                _stream_ptr())
+        if spec.fp8_format:
+            check(lib.vsiq_ci_fp8_lsq_bwd(*bwd_args, int(spec.fp8_format), *tail), "vsiq_ci_fp8_lsq_bwd")
+        else:
+            check(lib.vsiq_ci_lsq_bwd(*bwd_args, *tail), "vsiq_ci_lsq_bwd")
         _count_launch()
     return dx, ds, dz, db
 
@@ -714,6 +776,22 @@ def qparams_from_minmax(states: torch.Tensor, bits: torch.Tensor, symmetric: tor
         check(lib.vsiq_qparams_from_minmax(states.data_ptr(), n, bits.data_ptr(), symmetric.data_ptr(), float(eps),
                                            _stream_ptr()), "vsiq_qparams_from_minmax")
         _count_launch()
+
+
+def fp8_scale_from_range(lo: torch.Tensor, hi: torch.Tensor, fp8_format: int, out: torch.Tensor) -> torch.Tensor:
+    """out[c] = max(|lo[c]|, |hi[c]|) / F, or 1.0 where that is zero or not finite (vsiq_fp8_scale_from_range), written
+    IN PLACE: lo / hi are equally strided fp64 device views (an observer's device_range()), out a contiguous fp64 [C]."""
+    C = lo.numel()
+    if lo.dtype != torch.float64 or hi.dtype != torch.float64 or lo.dim() != 1 or hi.shape != lo.shape \
+            or lo.stride() != hi.stride() or not lo.is_cuda or hi.device != lo.device:
+        raise ValueError("lo / hi must be equally strided 1-D float64 CUDA views")
+    if out.dtype != torch.float64 or out.numel() != C or not out.is_contiguous() or out.device != lo.device:
+        raise ValueError(f"out must be a contiguous float64 tensor with {C} entries on {lo.device}")
+    with torch.cuda.device(lo.device):
+        check(lib.vsiq_fp8_scale_from_range(lo.data_ptr(), hi.data_ptr(), max(lo.stride(0), 1), C, int(fp8_format),
+                                            out.data_ptr(), _stream_ptr()), "vsiq_fp8_scale_from_range")
+        _count_launch()
+    return out
 
 
 def lsq_init_scale(state: torch.Tensor, bits: int, out: torch.Tensor) -> torch.Tensor:

@@ -38,6 +38,7 @@ from ..observers.minmax import MinMaxObserver  # noqa: F401
 from ..observers.moving_average import MovingAverageMinMaxObserver  # noqa: F401
 from ..observers.mse import MSEObserver  # noqa: F401
 from ..observers.percentile import PercentileObserver  # noqa: F401
+from ..quantizers.fp8 import FP8Quantizer  # noqa: F401
 from ..quantizers.uniform import UniformQuantizer  # noqa: F401
 from ..utils.registry import CLASS_REGISTRY
 
@@ -60,6 +61,12 @@ class QuantizationManager(nn.Module):
             self.quantizer.ch_axis = ch_axis
             self.observer.ch_axis = ch_axis
         self.ch_axis = ch_axis
+        # FP8 quantisers: scale = amax / F of the observer's range, kept in a persistent device buffer (_fp8_refresh)
+        self._fp8 = int(getattr(self.quantizer, "fp8_format", 0))
+        self._fp8_scale: Optional[torch.Tensor] = None
+        if self._fp8 and isinstance(self.observer, (MSEObserver, EntropyObserver)):
+            raise ValueError(f"{type(self.observer).__name__} searches the best integer grid; it cannot calibrate "
+                             f"{type(self.quantizer).__name__} (use MinMaxObserver or PercentileObserver)")
         if hasattr(self.observer, "_on_change"):
             self.observer._on_change = self._invalidate  # host code poking min_val / max_val drops the cached qparams
         self.bits_width = bits_width
@@ -77,14 +84,41 @@ class QuantizationManager(nn.Module):
     def __getattr__(self, name):
         # reached only when normal lookup fails: scale / zero_point were invalidated by a calibration call
         if name in _LAZY and "_calibrated" in self.__dict__ and self.__dict__["_calibrated"]:
-            s, z = self.observer.get_scale_zero_point()  # one D2H copy
+            if self.__dict__.get("_fp8"):
+                s = self.__dict__["_fp8_scale"].cpu()  # one D2H copy
+                s, z = (float(s[0]), 0) if s.numel() == 1 else (s.clone(), 0)
+            else:
+                s, z = self.observer.get_scale_zero_point()  # one D2H copy
             self.__dict__["scale"], self.__dict__["zero_point"] = s, z
             return self.__dict__[name]
         return super().__getattr__(name)
 
     def _invalidate(self) -> None:
+        """The observer state changed (calibration call, load_state, a host poke, sync_observers' merge)."""
         self.__dict__.pop("scale", None)
         self.__dict__.pop("zero_point", None)
+        self._fp8_refresh()
+
+    def _fp8_refresh(self) -> None:
+        """Rewrite the FP8 scale from the observer's range IN PLACE (no host sync): CUDA graphs captured with the fixed
+        qparams and cached pointers keep seeing the current value."""
+        st = getattr(self.observer, "state", None)
+        if not self.__dict__.get("_fp8") or not isinstance(st, torch.Tensor) or not st.is_cuda:
+            return
+        from .. import ops
+        buf = self._fp8_scale
+        if buf is None or buf.numel() != st.shape[0] or buf.device != st.device:
+            buf = self._fp8_scale = torch.empty(st.shape[0], dtype=torch.float64, device=st.device)
+        lo, hi = self.observer.device_range()
+        ops.fp8_scale_from_range(lo, hi, self._fp8, buf)
+
+    def _device_qparams(self):
+        """Calibrated fixed qparams on the device: the FP8 scale buffer and 0, or the observer's scale / zero-point."""
+        if self._fp8:
+            if self._fp8_scale is None:
+                self._fp8_refresh()
+            return self._fp8_scale, 0
+        return self.observer.device_qparams()
 
     def _stats_host(self):
         if not self._call_stats:
@@ -276,14 +310,15 @@ class QuantizationManager(nn.Module):
         if "scale" in self._parameters or "zero_point" in self._parameters or not self._calibrated \
                 or "scale" in self.__dict__:
             return self.scale, self.zero_point
-        return self.observer.device_qparams()
+        return self._device_qparams()
 
     def can_emit_second(self, act, x) -> bool:
         """True when quantize(x, pre_act=act, second=...) will run as the two-output channels_last epilogue."""
         from .. import ops
         q = self.quantizer
         return bool(act is not None and self.can_fuse_act(act, x) and ops.ci_supported(x) and hasattr(q, "kernel_args")
-                    and getattr(q, "mask_mode", "rounded") == "rounded" and self.__dict__.get("_banked") is None)
+                    and getattr(q, "mask_mode", "rounded") == "rounded" and self.__dict__.get("_banked") is None
+                    and not self._fp8)
 
     def prequant_plan(self, x):
         """(scale, zero_point, QSpec) for running THIS manager's quantise step as the second stage of another layer's
@@ -328,7 +363,7 @@ class QuantizationManager(nn.Module):
             if "scale" in self._parameters or "zero_point" in self._parameters or not self._calibrated \
                     or "scale" in self.__dict__:
                 return self.quantizer.quantize(x, self.scale, self.zero_point, self.is_learning_scale, **kw)
-            s, z = self.observer.device_qparams()
+            s, z = self._device_qparams()
             return self.quantizer.quantize(x, s, z, self.is_learning_scale, **kw)
         self.collect_qparameter(x)
         if not self.is_quantize:
@@ -338,17 +373,22 @@ class QuantizationManager(nn.Module):
             # learned Parameters, never-calibrated defaults, or values host code has set / read back
             return self.quantizer.quantize(x, self.scale, self.zero_point, self.is_learning_scale)
         # calibrated, fixed qparams: feed the kernels from the observer state on the device (no sync)
-        s, z = self.observer.device_qparams()
+        s, z = self._device_qparams()
         return self.quantizer.quantize(x, s, z, self.is_learning_scale)
 
     def init_scaling_factor_for_learning(self):
         """scale = 2*mean(mean|x|)/sqrt(2^(b-1)-1) (:105-114), computed on the device; becomes a 0-dim (per tensor)
-        or [C] tensor of ``param_dtype``.  Without calibration data the current scale is kept."""
+        or [C] tensor of ``param_dtype``.  FP8 quantisers start from the calibrated scale amax / F instead.  Without
+        calibration data the current scale is kept."""
         st = self.observer.state
         if st is None or not self._call_stats:
             return
-        out = torch.empty(st.shape[0], dtype=self.param_dtype, device=st.device)
-        self.observer.lsq_init_scale(self.bits_width, out)
+        if self._fp8:
+            self._fp8_refresh()
+            out = self._fp8_scale.to(self.param_dtype, copy=True)
+        else:
+            out = torch.empty(st.shape[0], dtype=self.param_dtype, device=st.device)
+            self.observer.lsq_init_scale(self.bits_width, out)
         self._calibrated = False
         if "scale" in self._parameters:
             # already learnable (a second activate_learning_qparam / deactivate_learning_qparam): re-initialise the
@@ -365,7 +405,7 @@ class QuantizationManager(nn.Module):
 
     def _current_zero_point(self):
         st = self.observer.state
-        if st is None:
+        if st is None or self._fp8:
             return 0
         z = st[:, 3]
         return z.reshape(()) if z.numel() == 1 else z.clone()

@@ -81,9 +81,14 @@ def link_quantize_inp(model, example_input=None, forward=None) -> int:
     finally:
         for h in handles:
             h.remove()
+    def fp8(m):
+        return bool(getattr(getattr(m.activation_quantizer, "quantizer", None), "fp8_format", 0))
+
     linked, seen = 0, set()
     for src, dst in pairs:
         if id(src) in seen:  # one second stage per producer: the first consumer found keeps the link
+            continue
+        if fp8(src) or fp8(dst):  # the two-output epilogue has integer grids only
             continue
         seen.add(id(src))
         src.feed_input_quantizer_of(dst)
